@@ -1,7 +1,7 @@
 """bench.py - headline benchmark of the ControlNet denoising hot path (BASELINE.json configs[1]).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config 2|3|4|5]
-                    [--scaling strong|weak] [--mode f16|fp32]
+                    [--scaling strong|weak] [--mode f16|fp32] [--dump-outputs DIR]
 
 Workload : MNIST DDPM ControlNet (config/mnist.yaml model_params), synthetic random-init weights, x_T ~ N(0,1),
            Canny-like hints (Bernoulli 0.1 in {0,1}, 3 identical channels), GLOBAL batch 1024 (BASELINE config 2).
@@ -17,6 +17,10 @@ shard H2D, all 1000 timesteps, all-gather, D2H of the gathered samples - all ins
 the box's host cores / on the same GPU through stock PyTorch) and `clocks` (nvidia-smi under load).
 `--impl reference` times the reference's own modules (baseline/_ref, installed by oracle/install_ref.py) on the CPU.
 `--config 3|4|5` run the other BASELINE configs (CelebHQ LDM + VAE decode; consistency students; CIFAR DM sweep).
+`--dump-outputs DIR` writes what the timed step computed in its last replay, the (x_{t-1}, x0) pair a caller of
+sampler.DDPMSampler.sample receives, as DIR/xt.npy and DIR/x0.npy (float32, the whole global batch, or a fixed seeded
+sample of its rows above 64 MB in all).  Weights, hints, x_T and the Philox noise are all seeded, so two builds run with
+the same arguments can be compared output for output.
 """
 import argparse
 import importlib
@@ -27,12 +31,14 @@ import sys
 import threading
 import time
 
+sys.dont_write_bytecode = True          # the tree may be read-only: nothing of this run is cached in it
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 METRIC = "controlnet_ddpm_samples_per_sec"
 UNIT = "samples/s"
 STEPS_PER_SAMPLE = 1000
 FLOP_PER_SAMPLE_STEP = 3.878e9          # BASELINE.md section 2 (MNIST ControlNet, 2*MAC convention)
+DUMP_LIMIT_BYTES = 63 * 10 ** 6          # --dump-outputs: under 64 MB in all, .npy headers included
 
 
 def _peaks():
@@ -487,6 +493,28 @@ def _timed_replay(smp, steps, warmup, world, dev):
     return float(ms.item()) / steps, w0, w1
 
 
+def dump_outputs(smp, total, world, rank, out_dir):
+    """Write the sampler's state after the last timed replay (x_{t-1} and the x0 prediction of that step, gathered over
+    the ranks) as float32 .npy files; above DUMP_LIMIT_BYTES a fixed seeded sample of the batch rows is kept."""
+    import numpy as np
+    import torch
+    S = importlib.import_module("controlnet-pytorch_b200.sampler")
+    outs = {"xt": smp.xt, "x0": smp.x0}
+    if world > 1:
+        outs = {k: S.gather_shards(v, total) for k, v in outs.items()}
+    if rank != 0:
+        return
+    row_bytes = sum(v[0].numel() * 4 for v in outs.values())
+    keep = None
+    if total * row_bytes > DUMP_LIMIT_BYTES:
+        g = torch.Generator().manual_seed(0)
+        keep = torch.randperm(total, generator=g)[: DUMP_LIMIT_BYTES // row_bytes].sort().values.to(smp.xt.device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in outs.items():
+        v = v if keep is None else v.index_select(0, keep)
+        np.save(os.path.join(out_dir, name + ".npy"), v.float().cpu().numpy())
+
+
 def run_b200(args):
     import torch
     import torch.distributed as dist
@@ -527,6 +555,8 @@ def run_b200(args):
     ms_per_step, w0, w1 = _timed_replay(smp, args.steps, args.warmup, world, dev)
     if rank == 0:
         clk.stop()
+    if args.dump_outputs:
+        dump_outputs(smp, total, world, rank, args.dump_outputs)
     value = total / (ms_per_step * 1e-3 * STEPS_PER_SAMPLE)
     launches = smp.launches_per_step * args.steps
 
@@ -700,7 +730,13 @@ def main():
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-other", action="store_true", help="skip the second (weak / strong) record at N > 1")
     ap.add_argument("--no-dropin", action="store_true", help="skip the reference-tool-loop measurement (e2e_dropin)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (config 2, --impl b200)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.config != 2 or args.impl != "b200"):
+        ap.error("--dump-outputs is implemented for the config 2 run of --impl b200")
     if args.mode == "tf32":
         args.mode = "f16"
     if args.config != 2:

@@ -13,7 +13,8 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import GOLDEN, ROOT, golden, syn
+import helpers as H
+from helpers import GOLDEN, REFERENCE, ROOT, golden, syn
 
 
 def _mod(name):
@@ -68,25 +69,13 @@ def test_state_dict_layout_matches_reference_manifest():
 
 
 def test_default_init_is_seed_identical_to_reference_when_present():
-    if not os.path.isdir("/root/reference/models"):
-        pytest.skip("reference tree only exists in the build container")
+    """torch.manual_seed(7) + ControlNet(TINY) gives the tensors the reference's class gives.  Without the reference
+    the comparison is with the regression pin of the parent's drop-ins (tests/helpers.py: expected)."""
     cn = _mod("models.controlnet")
     torch.manual_seed(7)
     mine = cn.ControlNet(syn.TINY_PARAMS).state_dict()
-    sys.path.insert(0, "/root/reference")
-    try:
-        for k in [k for k in sys.modules if k == "models" or k.startswith("models.")]:
-            del sys.modules[k]
-        from models.controlnet import ControlNet as Ref
-        torch.manual_seed(7)
-        ref = Ref(syn.TINY_PARAMS).state_dict()
-    finally:
-        sys.path.remove("/root/reference")
-        for k in [k for k in sys.modules if k == "models" or k.startswith("models.")]:
-            del sys.modules[k]
-    assert list(mine) == list(ref)
-    for k in ref:
-        assert torch.equal(mine[k], ref[k]), k
+    want, against = H.expected("init", H.init_digests)
+    assert H.digest(mine) == want["controlnet_tiny_seed7"], against
     # the zero convolutions really are zero at init (controlnet.py:7-10)
     assert float(mine["control_copy_unet_down_zero_convs.0.weight"].abs().sum()) == 0.0
 
@@ -206,7 +195,8 @@ def test_dropin_shim_serves_the_reference_import_lines(tmp_path):
     assert r.returncode == 0 and "dropin imports ok" in r.stdout, r.stdout + r.stderr
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/tools"), reason="needs the reference checkout")
+@pytest.mark.skipif(REFERENCE is None or not os.path.isdir(os.path.join(REFERENCE, "tools")),
+                    reason="needs a reference checkout (CNB_REFERENCE)")
 def test_reference_tools_import_the_dropins_and_keep_their_other_modules():
     """The unmodified tools/sample_*.py, run from the reference checkout, get the B200 models / scheduler while
     dataset.*, scheduler.consistency_scheduler and models.discriminator still come from the reference."""
@@ -222,50 +212,30 @@ def test_reference_tools_import_the_dropins_and_keep_their_other_modules():
         "assert l.ControlNet.__module__ == P + 'models.controlnet_ldm' and l.VAE.__module__ == P + 'models.vae'\n"
         "assert c.ConsistencyControlNetDistilled.__module__ == P + 'models.consistency_controlnet_distilled'\n"
         "assert d.DistributionMatchingControlNetDistilled.__module__ == P + 'models.distribution_matching_controlnet'\n"
-        "assert cs.__file__.startswith('/root/reference/') and md.__file__.startswith('/root/reference/')\n"
+        f"assert cs.__file__.startswith({REFERENCE + os.sep!r}) and md.__file__.startswith({REFERENCE + os.sep!r})\n"
         "assert t.MnistDataset.__module__ == 'dataset.mnist_dataset'\n"
         "print('tools ok')\n")
-    r = subprocess.run([sys.executable, "-c", code], env=_dropin_env(["/root/reference"]), cwd="/root/reference",
+    r = subprocess.run([sys.executable, "-c", code], env=_dropin_env([REFERENCE]), cwd=REFERENCE,
                        capture_output=True, text=True, timeout=300)
     assert r.returncode == 0 and "tools ok" in r.stdout, r.stdout + r.stderr
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/models"), reason="needs the reference checkout")
 def test_checkpoints_written_by_the_reference_load_the_way_the_tools_load_them(tmp_path):
     """The construction / checkpoint sequences of tools/sample_ddpm_controlnet.py:80-92,
     tools/sample_consistency_controlnet_distilled.py:30-49 and
     tools/sample_distribution_matching_controlnet_distilled.py:33-54, fed with files written by the REFERENCE classes:
-    every tensor of the resulting B200 module equals the reference module built the same way."""
+    every tensor of the resulting B200 module equals the reference module built the same way.  Without the reference
+    the drop-in classes write the files and both their modules and the loaded ones are compared with the regression
+    pins of the parent's drop-ins (tests/helpers.py: expected)."""
     cfg = syn.TINY_PARAMS
-    ddpm, ctrl = str(tmp_path / "ddpm_ckpt.pth"), str(tmp_path / "controlnet_ckpt.pth")
-    cons, dmck = str(tmp_path / "consistency.pth"), str(tmp_path / "dm.pth")
-    purge = lambda: [sys.modules.pop(k) for k in list(sys.modules)          # noqa: E731
-                     if k.split(".")[0] in ("models", "scheduler")]
-    sys.path.insert(0, "/root/reference")
-    try:
-        purge()
-        from models.unet_base import Unet as RefUnet
-        from models.controlnet import ControlNet as RefCN
-        from models.consistency_controlnet_distilled import ConsistencyControlNetDistilled as RefCons
-        from models.distribution_matching_controlnet import DistributionMatchingControlNetDistilled as RefDM
-        torch.manual_seed(11)
-        torch.save(RefUnet(cfg).state_dict(), ddpm)
-        torch.manual_seed(20)
-        ref_cn = RefCN(cfg, model_ckpt=ddpm, device=torch.device("cpu"))
-        ref_cn.load_state_dict(syn.det_state_dict(ref_cn.state_dict(), seed=5))
-        torch.save(ref_cn.state_dict(), ctrl)
-        torch.manual_seed(21)
-        ref_cons = RefCons(cfg, ddpm, device=torch.device("cpu"))
-        torch.save({"model_state_dict": syn.det_state_dict(ref_cons.student.state_dict(), seed=6)}, cons)
-        ref_cons.student.load_state_dict(torch.load(cons, weights_only=False)["model_state_dict"])
-        torch.manual_seed(22)
-        ref_dm = RefDM(cfg, ctrl, device=torch.device("cpu"))
-        torch.save({"model_state_dict": syn.det_state_dict(ref_dm.student.state_dict(), seed=7)}, dmck)
-        ref_dm.student.load_state_dict(torch.load(dmck, weights_only=False)["model_state_dict"])
-        want = {"cn": ref_cn.state_dict(), "cons": ref_cons.state_dict(), "dm": ref_dm.state_dict()}
-    finally:
-        sys.path.remove("/root/reference")
-        purge()
+    if REFERENCE is not None:
+        paths, want = H.on_reference(lambda get: H.write_tool_checkpoints(get, tmp_path))
+        against = "reference"
+    else:
+        paths, written = H.write_tool_checkpoints(_mod, tmp_path)
+        want, against = H.expected("tool_checkpoints", None)
+        assert written == want, against
+    ddpm, ctrl, cons, dmck = paths["ddpm"], paths["ctrl"], paths["cons"], paths["dm"]
     dev = torch.device("cpu")
     torch.manual_seed(20)
     cn = _mod("models.controlnet").ControlNet(cfg, model_ckpt=ddpm, device=dev).to(dev)
@@ -277,138 +247,53 @@ def test_checkpoints_written_by_the_reference_load_the_way_the_tools_load_them(t
     md = _mod("models.distribution_matching_controlnet").DistributionMatchingControlNetDistilled(cfg, ctrl, device=dev).to(dev)
     md.student.load_state_dict(torch.load(dmck, map_location=dev, weights_only=False)["model_state_dict"])
     for tag, mine in (("cn", cn.state_dict()), ("cons", mc.state_dict()), ("dm", md.state_dict())):
-        ref = want[tag]
-        assert list(mine) == list(ref), (tag, set(mine) ^ set(ref))
-        for k in ref:
-            assert torch.equal(mine[k], ref[k]), (tag, k)
+        assert H.digest(mine) == want[tag], (tag, against)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/models"), reason="needs the reference checkout")
 def test_every_dropin_class_initialises_seed_identically_to_the_reference():
     """torch.manual_seed(s) + constructor gives the same tensors under the same keys as the reference class, for every
-    module on the path (layers are created in the reference's order, so the default initialisers draw the same numbers)."""
-    specs = [("models.controlnet_ldm", "ControlNet", (4, syn.TINY_LDM_PARAMS), dict(down_sample_factor=8)),
-             ("models.vae", "VAE", (3, syn.TINY_VAE_PARAMS), {}),
-             ("models.unet_base", "Unet", (syn.TINY_PARAMS,), {}),
-             ("models.unet_cond_base", "Unet", (4, syn.TINY_LDM_PARAMS), {}),
-             ("models.consistency_controlnet_distilled", "ConsistencyControlNet", (syn.TINY_PARAMS,), {}),
-             ("models.consistency_controlnet_distilled", "ConsistencyControlNetDistilled", (syn.TINY_PARAMS,), {}),
-             ("models.distribution_matching_controlnet", "DistributionMatchingControlNet", (syn.TINY_PARAMS,), {}),
-             ("models.controlnet", "ControlNet", (syn.MNIST_PARAMS,), {})]
-    mine = []
-    for i, (mod, cls, a, k) in enumerate(specs):
-        torch.manual_seed(100 + i)
-        mine.append(getattr(_mod(mod), cls)(*a, **k).state_dict())
-    purge = lambda: [sys.modules.pop(k) for k in list(sys.modules)          # noqa: E731
-                     if k.split(".")[0] in ("models", "scheduler")]
-    sys.path.insert(0, "/root/reference")
-    try:
-        purge()
-        for i, (mod, cls, a, k) in enumerate(specs):
-            torch.manual_seed(100 + i)
-            ref = getattr(importlib.import_module(mod), cls)(*a, **k).state_dict()
-            assert list(mine[i]) == list(ref), (mod, cls)
-            for name in ref:
-                assert torch.equal(mine[i][name], ref[name]), (mod, cls, name)
-    finally:
-        sys.path.remove("/root/reference")
-        purge()
+    module on the path (layers are created in the reference's order, so the default initialisers draw the same numbers).
+    Without the reference: the regression pins of the parent's drop-ins (tests/helpers.py: expected)."""
+    want, against = H.expected("init", H.init_digests)
+    mine = H.init_digests(_mod)
+    for name in want:
+        assert mine[name] == want[name], (name, against)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/models"), reason="needs the reference checkout")
 def test_public_surface_matches_the_reference_signatures():
     """Every public class / function of the reference's hot-path modules exists in the drop-in module, and the
     inference-side methods take the reference's parameters (names, order, defaults); extra trailing keyword
-    parameters (`z=`, `step_index=`) are allowed."""
-    import inspect
-    mods = ["models.unet_base", "models.blocks", "models.unet_cond_base", "models.controlnet", "models.controlnet_ldm",
-            "models.consistency_controlnet_distilled", "models.distribution_matching_controlnet", "models.vae",
-            "scheduler.linear_noise_scheduler"]
-    methods = ("__init__", "forward", "encode", "decode", "generate", "sample_prev_timestep", "add_noise", "get_params",
-               "get_teacher_prediction", "get_ddpm_teacher_prediction", "sigma_to_timestep", "get_noise_schedule",
-               "c_skip", "c_out", "c_in", "c_noise")
-    ours = {m: _mod(m) for m in mods}
-    purge = lambda: [sys.modules.pop(k) for k in list(sys.modules)          # noqa: E731
-                     if k.split(".")[0] in ("models", "scheduler")]
-    params = lambda f: [(p.name, p.default) for p in inspect.signature(f).parameters.values()]   # noqa: E731
-    sys.path.insert(0, "/root/reference")
+    parameters (`z=`, `step_index=`) are allowed.  Without the reference the recorded surface is the parent's drop-in
+    surface (re-exported duplicates such as blocks.get_time_embedding included), so there the extras are pinned too."""
+    ref, against = H.expected("public_surface", H.public_surface)
     checked = 0
-    try:
-        purge()
-        for m in mods:
-            ref = importlib.import_module(m)
-            for name, obj in vars(ref).items():
-                if name.startswith("_") or getattr(obj, "__module__", None) != m:
-                    continue
-                mine = getattr(ours[m], name, None)
-                assert mine is not None, (m, name)
-                if inspect.isclass(obj):
-                    for meth in methods:
-                        if meth in vars(obj):
-                            want, got = params(getattr(obj, meth)), params(getattr(mine, meth))
-                            assert got[:len(want)] == want, (m, name, meth, want, got)
-                            checked += 1
-                elif inspect.isfunction(obj):
-                    want, got = params(obj), params(mine)
-                    assert got[:len(want)] == want, (m, name, want, got)
-                    checked += 1
-    finally:
-        sys.path.remove("/root/reference")
-        purge()
+    for m, entries in ref.items():
+        mod = _mod(m)
+        for name, want in entries.items():
+            mine = getattr(mod, name, None)
+            assert mine is not None, (m, name, against)
+            for meth, w in (want.items() if isinstance(want, dict) else [(None, want)]):
+                got = H.signature(mine if meth is None else getattr(mine, meth))
+                assert got[:len(w)] == w, (m, name, meth, w, got, against)
+                checked += 1
     assert checked >= 40
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/models"), reason="needs the reference checkout")
 def test_host_side_helpers_are_bit_identical_to_the_reference():
     """add_noise (linear_noise_scheduler.py:25-47), the EDM scalings (consistency_controlnet_distilled.py:45-74) and the
-    Karras schedule (:175-196) are plain host tensor expressions in both implementations: bit-identical on the CPU."""
-    s = _mod("scheduler.linear_noise_scheduler").LinearNoiseScheduler(**syn.MNIST_DIFFUSION)
-    g = torch.Generator().manual_seed(0)
-    x, n = torch.randn(4, 1, 8, 8, generator=g), torch.randn(4, 1, 8, 8, generator=g)
-    t, sig = torch.tensor([0, 5, 500, 999]), torch.tensor([0.002, 1.7, 80.0])
-    cc = _mod("models.consistency_controlnet_distilled")
-    cm, cd = cc.ConsistencyControlNet(syn.TINY_PARAMS), cc.ConsistencyControlNetDistilled(syn.TINY_PARAMS)
-    mine = [s.add_noise(x, n, t), cm.c_skip(sig), cm.c_out(sig), cm.c_in(sig), cm.c_noise(sig),
-            cd.get_noise_schedule(10, device=torch.device("cpu"))]
-    purge = lambda: [sys.modules.pop(k) for k in list(sys.modules)          # noqa: E731
-                     if k.split(".")[0] in ("models", "scheduler")]
-    sys.path.insert(0, "/root/reference")
-    try:
-        purge()
-        from scheduler.linear_noise_scheduler import LinearNoiseScheduler as RefS
-        from models.consistency_controlnet_distilled import ConsistencyControlNet as RC, \
-            ConsistencyControlNetDistilled as RCD
-        r, rc = RefS(**syn.MNIST_DIFFUSION), RC(syn.TINY_PARAMS)
-        ref = [r.add_noise(x, n, t), rc.c_skip(sig), rc.c_out(sig), rc.c_in(sig), rc.c_noise(sig),
-               RCD(syn.TINY_PARAMS).get_noise_schedule(10, device=torch.device("cpu"))]
-    finally:
-        sys.path.remove("/root/reference")
-        purge()
-    for i, (a, b) in enumerate(zip(mine, ref)):
-        assert torch.equal(a, b), i
+    Karras schedule (:175-196) are plain host tensor expressions in both implementations: bit-identical on the CPU.
+    Without the reference: the regression pins of the parent's drop-ins (tests/helpers.py: expected)."""
+    want, against = H.expected("host_helpers", H.host_helper_digests)
+    mine = H.host_helper_digests(_mod)
+    assert len(mine) == len(want)
+    for i, (a, b) in enumerate(zip(mine, want)):
+        assert a == b, (i, against)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/models"), reason="needs the reference checkout")
 @pytest.mark.parametrize("locked", [True, False])
 def test_model_locked_and_get_params_match_the_reference(locked):
     """`model_locked` freezes the same parameters and `get_params()` (controlnet.py:140-156, controlnet_ldm.py) returns
-    the same parameters in the same order as the reference."""
-    def describe(m):
-        names = {id(p): n for n, p in m.named_parameters()}
-        return {n: p.requires_grad for n, p in m.named_parameters()}, [names[id(p)] for p in m.get_params()]
-    mine = [describe(_mod("models.controlnet").ControlNet(syn.TINY_PARAMS, model_locked=locked)),
-            describe(_mod("models.controlnet_ldm").ControlNet(4, syn.TINY_LDM_PARAMS, model_locked=locked,
-                                                              down_sample_factor=8))]
-    purge = lambda: [sys.modules.pop(k) for k in list(sys.modules)          # noqa: E731
-                     if k.split(".")[0] in ("models", "scheduler")]
-    sys.path.insert(0, "/root/reference")
-    try:
-        purge()
-        from models.controlnet import ControlNet as RefCN
-        from models.controlnet_ldm import ControlNet as RefLDM
-        ref = [describe(RefCN(syn.TINY_PARAMS, model_locked=locked)),
-               describe(RefLDM(4, syn.TINY_LDM_PARAMS, model_locked=locked, down_sample_factor=8))]
-    finally:
-        sys.path.remove("/root/reference")
-        purge()
-    assert mine == ref
+    the same parameters in the same order as the reference.  Without the reference: the regression pins of the parent's
+    drop-ins (tests/helpers.py: expected)."""
+    want, against = H.expected("locked_params", lambda get: {str(lk): H.locked_params(get, lk) for lk in (True, False)})
+    assert H.locked_params(_mod, locked) == want[str(locked)], against

@@ -7,7 +7,7 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import det_sd_for, golden, inputs, max_abs, psnr, rel_l2, syn, ROOT
+from helpers import REFERENCE, det_sd_for, golden, inputs, max_abs, psnr, rel_l2, syn, ROOT
 
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 import cn_oracle as O  # noqa: E402
@@ -125,10 +125,10 @@ def test_scheduler_bit_exact_vs_golden(name, kw):
         assert np.array_equal(b.numpy(), g[f"x0_{t}"]), t
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/models"), reason="reference tree only exists in the build container")
+@pytest.mark.skipif(REFERENCE is None, reason="needs the reference's modules (CNB_REFERENCE or baseline/_ref)")
 def test_oracle_vs_live_reference_default_init():
     """Second pin: default torch init (zero-convs exactly zero) straight from the imported reference."""
-    sys.path.insert(0, "/root/reference")
+    sys.path.insert(0, REFERENCE)
     try:
         for k in [k for k in sys.modules if k == "models" or k.startswith("models.")]:
             del sys.modules[k]
@@ -141,7 +141,7 @@ def test_oracle_vs_live_reference_default_init():
             got = O.controlnet_ddpm_forward(m.state_dict(), syn.TINY_PARAMS, x, torch.as_tensor(77).unsqueeze(0), hint)
         assert rel_l2(got, want) < TOL
     finally:
-        sys.path.remove("/root/reference")
+        sys.path.remove(REFERENCE)
         for k in [k for k in sys.modules if k == "models" or k.startswith("models.")]:
             del sys.modules[k]
 
