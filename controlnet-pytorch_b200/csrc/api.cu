@@ -91,11 +91,6 @@ extern "C" int cnb_conv2d(const cnb_conv_params* p, cnb_stream_t stream) {
   CNB_REQUIRE(p->in_dtype == 0 || p->in_dtype == 1, "conv2d: in_dtype=%d", p->in_dtype);
   CNB_REQUIRE(p->out_dtype == 0 || p->out_dtype == 1, "conv2d: out_dtype=%d", p->out_dtype);
   CNB_REQUIRE(p->res_dtype == 0 || p->res_dtype == 1, "conv2d: res_dtype=%d", p->res_dtype);
-  static int small_on = -1;
-  if (small_on < 0) {
-    const char* e = getenv("CNB_CONV_SMALL");
-    small_on = e ? atoi(e) : 1;
-  }
   if (p->in2) {
     CNB_REQUIRE(p->Cin2 > 0 && p->ldi2 >= p->in2_coff + p->Cin2, "conv2d: bad second input");
     CNB_REQUIRE(p->mode != CNB_MODE_F32 && conv2d_tma_supported(p),
@@ -103,7 +98,7 @@ extern "C" int cnb_conv2d(const cnb_conv_params* p, cnb_stream_t stream) {
     return conv2d_tma(p, st);
   }
   // tiny-channel ends of the U-Net (Cin <= 4 or Cout <= 4): direct exact-fp32 kernels in every mode
-  if (small_on && (p->Cin <= 4 || p->Cout <= 4) && conv2d_small_supported(p)) return conv2d_small(p, st);
+  if ((p->Cin <= 4 || p->Cout <= 4) && conv2d_small_supported(p)) return conv2d_small(p, st);
   if (p->mode == CNB_MODE_F16) {
     if (conv2d_tma_supported(p)) return conv2d_tma(p, st);     // TMA-im2col fed persistent tcgen05 kernel
   } else if (p->mode != CNB_MODE_F32) {

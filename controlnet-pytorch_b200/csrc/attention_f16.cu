@@ -13,7 +13,6 @@
 //   * online softmax in the exp2 domain: p = ex2(fma(s, scale*log2e, -m*scale*log2e)), row max / sum reduced across
 //     the 4 lanes of a quad with shuffles, running (m, l) per row, O rescaled per tile.
 #include <cuda_fp16.h>
-#include <stdlib.h>
 
 #include <type_traits>
 
@@ -57,33 +56,14 @@ __device__ __forceinline__ uint32_t pack_h2(float lo, float hi) {
   return *reinterpret_cast<const uint32_t*>(&h);
 }
 
-__device__ __forceinline__ uint32_t ex2_h2(uint32_t x) {
-  uint32_t y;
-  asm("ex2.approx.f16x2 %0, %1;" : "=r"(y) : "r"(x));
-  return y;
-}
-
 // D: head dim (even; padded to a multiple of 16 for Q K^T); BK: keys per tile (multiple of 16); NW: warps per CTA
-// (BQ = 16 * NW);
-// H2: exponentials as ex2.approx.f16x2 on the packed pair that becomes the P operand anyway (one MUFU op per two
-//     scores; the argument fma(s, c, -m c) <= 0 is formed in fp32 and rounded to fp16 once).
+// (BQ = 16 * NW).
 // The softmax denominator is accumulated by the tensor core as one more output column tile whose B fragment is the
 // constant half2(1, 1): l = P . 1 in fp32, consistent with the fp16 P that multiplies V.
-// Key tiles processed per block barrier.  The narrow heads at 4 warps per CTA spent 14 % of their cycles at the one
-// barrier per 64-key tile (ncu: stall_barrier), so they take two tiles per barrier from a six-slot ring.
-#ifndef ATTN_SUB2
-#define ATTN_SUB2 0
-#endif
-__host__ __device__ constexpr int attn_sub(int D, int BK, int NW) { return (ATTN_SUB2 && D <= 16 && BK == 64 && NW == 4) ? 2 : 1; }
-
-#ifndef ATTN_MIN_BLOCKS
-#define ATTN_MIN_BLOCKS 7
-#endif
-template <int D, int BK, int NW, bool H2, int VAR>
-#ifndef ATTN_MIN_BLOCKS8
-#define ATTN_MIN_BLOCKS8 3   // 8-warp kernels: <= 85 registers (d = 24: 122 -> 80, L = 1024 launch 2.15 -> 1.97 ms)
-#endif
-__global__ void __launch_bounds__(NW * 32, (NW == 4 && D <= 16) ? ((VAR & 2) ? 8 : ATTN_MIN_BLOCKS) : (NW == 8 ? ((VAR & 2) ? 4 : ATTN_MIN_BLOCKS8) : 0))
+// Minimum resident CTAs per SM: 7 for the narrow 4-warp kernels; 3 for the 8-warp kernels, i.e. <= 85 registers
+// (d = 24: 122 -> 80, L = 1024 launch 2.15 -> 1.97 ms); the 64-register build (VAR bit 1) asks for 8 / 4.
+template <int D, int BK, int NW, int VAR>
+__global__ void __launch_bounds__(NW * 32, (NW == 4 && D <= 16) ? ((VAR & 2) ? 8 : 7) : (NW == 8 ? ((VAR & 2) ? 4 : 3) : 0))
 attention_f16_kernel(const __half* __restrict__ qkv, __half* __restrict__ out, int L, int E, float scale_log2) {
   constexpr int d = D;
   constexpr int DP = (D + 15) / 16 * 16;         // K extent of Q K^T
@@ -99,7 +79,7 @@ attention_f16_kernel(const __half* __restrict__ qkv, __half* __restrict__ out, i
   //      barrier that frees the other one; a group's compute time covers the L2 latency)
   constexpr bool HALVES = (VAR & 1) != 0;
   constexpr bool RING2 = (VAR & 4) != 0;
-  constexpr int SUB = RING2 ? 2 : attn_sub(D, BK, NW);   // key tiles per block barrier
+  constexpr int SUB = RING2 ? 2 : 1;                     // key tiles per block barrier
   constexpr int NSLOT = (RING2 ? 2 : 3) * SUB;           // smem ring: two / three groups of SUB tiles
   static_assert(BK % 16 == 0, "BK must be a multiple of 16");
   extern __shared__ __align__(16) __half smem[];   // [3 * SUB slots][K | V][BK][STRIDE]
@@ -285,13 +265,8 @@ attention_f16_kernel(const __half* __restrict__ qkv, __half* __restrict__ out, i
         const float* sv = s[2 * kk + j];
         const float x0 = fmaf(sv[0], scale_log2, -ms0), x1 = fmaf(sv[1], scale_log2, -ms0);
         const float x2 = fmaf(sv[2], scale_log2, -ms1), x3 = fmaf(sv[3], scale_log2, -ms1);
-        if (H2) {
-          pa[2 * j] = ex2_h2(pack_h2(x0, x1));
-          pa[2 * j + 1] = ex2_h2(pack_h2(x2, x3));
-        } else {
-          pa[2 * j] = pack_h2(ex2(x0), ex2(x1));
-          pa[2 * j + 1] = pack_h2(ex2(x2), ex2(x3));
-        }
+        pa[2 * j] = pack_h2(ex2(x0), ex2(x1));
+        pa[2 * j + 1] = pack_h2(ex2(x2), ex2(x3));
       }
       mma_f16(lsum, pa, ONES, ONES);
       const uint32_t vrow = sV + (uint32_t)(kk * 16 * STRIDE) * 2u;
@@ -379,20 +354,18 @@ attention_f16_kernel(const __half* __restrict__ qkv, __half* __restrict__ out, i
   }
 }
 
-static int g_h2 = -1;   // CNB_ATTN_EXP2H=1: ex2.approx.f16x2 exponentials (no faster on sm_100a: two MUFU ops per pair)
-
-template <int D, int BK, int NW, bool H2, int VAR>
+template <int D, int BK, int NW, int VAR>
 static int launch2(const void* qkv, void* out, int B, int L, int E, int heads, cudaStream_t st) {
   constexpr int DP = (D + 15) / 16 * 16;
-  constexpr size_t SMEM = (size_t)((VAR & 4) ? 4 : 3 * attn_sub(D, BK, NW)) * 2 * BK * (DP + 8) * sizeof(__half);
+  constexpr size_t SMEM = (size_t)((VAR & 4) ? 4 : 3) * 2 * BK * (DP + 8) * sizeof(__half);
   static DeviceOnce attr_once;
   if (attr_once.first()) {
-    CNB_CUDA(cudaFuncSetAttribute(attention_f16_kernel<D, BK, NW, H2, VAR>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    CNB_CUDA(cudaFuncSetAttribute(attention_f16_kernel<D, BK, NW, VAR>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                   (int)SMEM));
   }
   const float scale_log2 = 1.4426950408889634f / sqrtf((float)D);
   dim3 grid(ceil_div(L, 16 * NW), heads, B);
-  CNB_CUDA(launch_pdl((long long)B * L * E, attention_f16_kernel<D, BK, NW, H2, VAR>, grid, dim3(NW * 32), SMEM, st,
+  CNB_CUDA(launch_pdl((long long)B * L * E, attention_f16_kernel<D, BK, NW, VAR>, grid, dim3(NW * 32), SMEM, st,
                       reinterpret_cast<const __half*>(qkv), reinterpret_cast<__half*>(out), L, E, scale_log2));
   CNB_LAUNCH_CHECK();
   return CNB_OK;
@@ -400,25 +373,13 @@ static int launch2(const void* qkv, void* out, int B, int L, int E, int heads, c
 
 template <int D, int BK, int NW>
 static int launch(const void* qkv, void* out, int B, int L, int E, int heads, cudaStream_t st) {
-  if (g_h2 < 0) {
-    const char* e = getenv("CNB_ATTN_EXP2H");
-    g_h2 = e ? atoi(e) : 0;
-  }
-  static int halves = -1;                  // CNB_ATTN_HALVES=0: whole 64-key tiles (the round-1 kernel)
-  if (halves < 0) {
-    const char* e = getenv("CNB_ATTN_HALVES");
-    halves = e ? atoi(e) : 1;
-  }
-  if (D <= 32 && g_h2) return launch2<D, BK, NW, (D <= 32), 0>(qkv, out, B, L, E, heads, st);
   // measured (profiles/r02_attention_table.md): halves pay everywhere at head dims <= 16; with them the kernel also fits
   // 64 registers = 8 CTAs (4 warps) / 4 CTAs (8 warps) per SM, which wins or ties except at d = 16 with 4 warps (spills)
   constexpr bool NARROW = BK == 64 && D <= 16;
   // halves, + the 64-register build where it does not spill, + two tiles per barrier for the 8-warp CTAs (measured:
   // L = 1024 d = 16 1362 -> 1311 us, L = 196 d = 16 88 -> 82 us; the 4-warp CTAs lose: L = 784 d = 16 854 -> 877 us)
   constexpr int HV = NARROW ? (((D == 16 && NW == 4) ? 1 : 3) | (NW == 8 ? 4 : 0)) : 0;
-  if (NARROW && halves == 1) return launch2<D, BK, NW, false, HV>(qkv, out, B, L, E, heads, st);
-  if (NARROW && halves == 2) return launch2<D, BK, NW, false, NARROW ? (HV | 4) : 0>(qkv, out, B, L, E, heads, st);
-  return launch2<D, BK, NW, false, 0>(qkv, out, B, L, E, heads, st);
+  return launch2<D, BK, NW, HV>(qkv, out, B, L, E, heads, st);
 }
 
 static inline long long padded(int L, int bq, int bk) {
@@ -432,12 +393,7 @@ template <int D, int BK>
 static int launch_l(const void* qkv, void* out, int B, int L, int E, int heads, cudaStream_t st) {
   if (L <= 16) return launch<D, 16, 1>(qkv, out, B, L, E, heads, st);
   if (L <= 32) return launch<D, 32, 2>(qkv, out, B, L, E, heads, st);
-  static int tie4 = -1;                    // experiment: CNB_ATTN_NW4=1 prefers 4 warps when both paddings tie
-  if (tie4 < 0) {
-    const char* e = getenv("CNB_ATTN_NW4");
-    tie4 = e ? atoi(e) : 0;
-  }
-  if (D > 64 || padded(L, 64, BK) < padded(L, 128, BK) || (tie4 && padded(L, 64, BK) == padded(L, 128, BK)))
+  if (D > 64 || padded(L, 64, BK) < padded(L, 128, BK))
     return launch<D, BK, 4>(qkv, out, B, L, E, heads, st);
   return launch<D, BK, 8>(qkv, out, B, L, E, heads, st);
 }
@@ -454,23 +410,6 @@ int attention_f16(const void* qkv, void* out, int B, int L, int E, int heads, cu
   CNB_REQUIRE(B <= 65535 && heads <= 65535, "attention: grid too large (B=%d)", B);
   CNB_REQUIRE((((uintptr_t)qkv | (uintptr_t)out) & 15) == 0, "attention: qkv / out must be 16-byte aligned");
   const int d = E / heads;
-  static int bk_env = -1;                  // experiment: CNB_ATTN_BK=32 / 16 key tiles for the narrow heads
-  if (bk_env < 0) {
-    const char* e = getenv("CNB_ATTN_BK");
-    bk_env = e ? atoi(e) : 64;
-  }
-  if (bk_env == 32 && L > 64) {
-    if (d == 4) return af16::launch_l<4, 32>(qkv, out, B, L, E, heads, st);
-    if (d == 16) return af16::launch_l<16, 32>(qkv, out, B, L, E, heads, st);
-    if (d == 32) return af16::launch_l<32, 32>(qkv, out, B, L, E, heads, st);
-    if (d == 24) return af16::launch_l<24, 32>(qkv, out, B, L, E, heads, st);
-    if (d == 8) return af16::launch_l<8, 32>(qkv, out, B, L, E, heads, st);
-    if (d == 64) return af16::launch_l<64, 32>(qkv, out, B, L, E, heads, st);
-  }
-  if (bk_env == 16 && L > 64) {
-    if (d == 4) return af16::launch_l<4, 16>(qkv, out, B, L, E, heads, st);
-    if (d == 16) return af16::launch_l<16, 16>(qkv, out, B, L, E, heads, st);
-  }
   switch (d) {
     case 4: return af16::launch_l<4, 64>(qkv, out, B, L, E, heads, st);
     case 8: return af16::launch_l<8, 64>(qkv, out, B, L, E, heads, st);

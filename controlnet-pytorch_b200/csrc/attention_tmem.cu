@@ -122,33 +122,20 @@ __device__ __forceinline__ float fmax3(float a, float b, float c) {
   asm("max.f32 %0, %1, %2, %3;" : "=f"(y) : "f"(a), "f"(b), "f"(c));
   return y;
 }
-// 2^x on the FMA / ALU pipes: round-to-nearest split x = n + f, |f| <= 0.5, cubic minimax for 2^f (relative error
-// 7.5e-5: below the fp16 rounding of P), exponent added to the bit pattern.
-__device__ __forceinline__ float ex2_poly(float x) {
-  x = fmaxf(x, -60.f);
-  const float t = x + 12582912.f;                           // 1.5 * 2^23: low mantissa bits = round(x)
-  const float f = x - (t - 12582912.f);
-  float p = fmaf(f, 0.05517167f, 0.24261113f);
-  p = fmaf(p, f, 0.69326097f);
-  p = fmaf(p, f, 0.99992806f);
-  return __int_as_float(__float_as_int(p) + (__float_as_int(t) << 23));
-}
 __device__ __forceinline__ uint32_t pack2(float lo, float hi) {
   const __half2 h = __floats2half2_rn(lo, hi);
   return *reinterpret_cast<const uint32_t*>(&h);
 }
 
 // One chunk of W (16 or 32) scores of this thread's row: raw scores r[] -> packed P (W / 2 registers).
-//   c = scale * log2 e, mc = m * c.  `vk` = number of valid keys in the chunk (MASK only).  POLY of every 8 exponentials
-//   run on the FMA pipe.
-template <int W, bool MASK, int POLY>
+//   c = scale * log2 e, mc = m * c.  `vk` = number of valid keys in the chunk (MASK only).
+template <int W, bool MASK>
 __device__ __forceinline__ void exp_pack(const uint32_t* r, float c, float mc, int vk, uint32_t* pk) {
 #pragma unroll
   for (int i = 0; i < W; i += 2) {
     float x0 = fmaf(__uint_as_float(r[i]), c, -mc), x1 = fmaf(__uint_as_float(r[i + 1]), c, -mc);
-    const int s = (i >> 1) & 3;                              // position inside a group of 4 pairs = 8 scores
-    float e0 = (POLY > 0 && s == 1) || (POLY > 2 && s == 3) ? ex2_poly(x0) : ex2f(x0);
-    float e1 = (POLY > 1 && s == 2) || (POLY > 3 && s == 0) ? ex2_poly(x1) : ex2f(x1);
+    float e0 = ex2f(x0);
+    float e1 = ex2f(x1);
     if (MASK) {
       if (i >= vk) e0 = 0.f;
       if (i + 1 >= vk) e1 = 0.f;
@@ -220,7 +207,7 @@ __device__ __forceinline__ void rescale_rows(float& m, float tm, float lazy, flo
 
 // Softmax of one S tile for this thread's row.  LAST = false: every key valid, no masks (the steady state); LAST = true:
 // `vk_tile` valid keys, whole chunks beyond them are skipped (the PV MMA skips the same 16-key blocks).
-template <int BK, int NV, int POLY, bool LAST>
+template <int BK, int NV, bool LAST>
 __device__ __forceinline__ void softmax_tile(float& m, bool first_tile, int vk_tile, float c, float lazy, uint32_t t_s,
                                              uint32_t t_o, uint64_t* o_bar = nullptr, uint32_t o_par = 0,
                                              volatile int* abort_flag = nullptr) {
@@ -247,18 +234,18 @@ __device__ __forceinline__ void softmax_tile(float& m, bool first_tile, int vk_t
     const float mc = m * c;
     uint32_t pk[16];
     if (w16) {
-      if (full) exp_pack<16, false, POLY>(r, c, mc, 16, pk);
-      else exp_pack<16, true, 0>(r, c, mc, vk, pk);
+      if (full) exp_pack<16, false>(r, c, mc, 16, pk);
+      else exp_pack<16, true>(r, c, mc, vk, pk);
       tmem_st8(t_s + (uint32_t)(ch * 16), pk);
     } else {
-      if (full) exp_pack<32, false, POLY>(r, c, mc, 32, pk);
-      else exp_pack<32, true, 0>(r, c, mc, vk, pk);
+      if (full) exp_pack<32, false>(r, c, mc, 32, pk);
+      else exp_pack<32, true>(r, c, mc, vk, pk);
       tmem_st16(t_s + (uint32_t)(ch * 16), pk);
     }
   }
 }
 
-template <int DL, int D, int BK, int POLY>
+template <int DL, int D, int BK>
 __global__ void __launch_bounds__(NUM_THREADS, 2)
 attention_tmem_kernel(const __grid_constant__ Args a) {
   using C = Cfg<DL, D, BK>;
@@ -514,8 +501,8 @@ attention_tmem_kernel(const __grid_constant__ Args a) {
     for (int j = 0; !dead && j < NT; ++j) {
       if (!mbar_wait_parked(&s_full[g], (uint32_t)(j & 1), abort_flag)) { dead = true; break; }
       tc_fence_after();
-      if (j < NT - 1) softmax_tile<BK, NV, POLY, false>(m, j == 0, BK, c, lazy, t_s, t_o);
-      else softmax_tile<BK, NV, POLY, true>(m, j == 0, vlast, c, lazy, t_s, t_o);
+      if (j < NT - 1) softmax_tile<BK, NV, false>(m, j == 0, BK, c, lazy, t_s, t_o);
+      else softmax_tile<BK, NV, true>(m, j == 0, vlast, c, lazy, t_s, t_o);
       tmem_st_wait();
       tc_fence_before();
       __syncwarp();
@@ -571,7 +558,7 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 static EncodeTiledFn g_encode = nullptr;
 
-template <int DL, int D, int BK, int POLY>
+template <int DL, int D, int BK>
 static int launch(const void* qkv, void* out, int B, int L, int E, int heads, cudaStream_t st) {
   using C = Cfg<DL, D, BK>;
   if (!g_encode) {
@@ -586,7 +573,7 @@ static int launch(const void* qkv, void* out, int B, int L, int E, int heads, cu
   }
   static DeviceOnce attr_once;
   if (attr_once.first()) {
-    CNB_CUDA(cudaFuncSetAttribute(attention_tmem_kernel<DL, D, BK, POLY>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::TOTAL));
+    CNB_CUDA(cudaFuncSetAttribute(attention_tmem_kernel<DL, D, BK>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::TOTAL));
   }
   Args a;
   memset(&a, 0, sizeof(a));
@@ -622,7 +609,7 @@ static int launch(const void* qkv, void* out, int B, int L, int E, int heads, cu
   }
   a.safe = safe;
   dim3 grid(ceil_div(L, 2 * BQ), heads, B);
-  CNB_CUDA(launch_pdl((long long)B * L * E, attention_tmem_kernel<DL, D, BK, POLY>, grid, dim3(NUM_THREADS),
+  CNB_CUDA(launch_pdl((long long)B * L * E, attention_tmem_kernel<DL, D, BK>, grid, dim3(NUM_THREADS),
                       (size_t)C::TOTAL, st, a));
   CNB_LAUNCH_CHECK();
   return CNB_OK;
@@ -630,45 +617,21 @@ static int launch(const void* qkv, void* out, int B, int L, int E, int heads, cu
 
 // Key-tile size: S_A, S_B (BK columns each) and O_A, O_B (NV each) share the CTA's 256 TMEM columns, and two CTAs (Q
 // tiles, K ring, raw V, V^T stages) share one SM's shared memory.  The largest tile that fits, shrunk when a smaller
-// one pads the sequence less (784 = 7 x 112 = 8.2 x 96; 1024 = 10.7 x 96 = 12.8 x 80 = 16 x 64); CNB_ATTN_TMEM_BK overrides.
-template <int DL, int D, int POLY>
+// one pads the sequence less (784 = 7 x 112 = 8.2 x 96; 1024 = 10.7 x 96 = 12.8 x 80 = 16 x 64).
+template <int DL, int D>
 static int launch_bk(const void* qkv, void* out, int B, int L, int E, int heads, cudaStream_t st) {
   constexpr int NV = (D + 1 + 15) / 16 * 16;
   constexpr int BKMAX = DL == 64 ? 48 : ((256 - 2 * NV) / 2) / 16 * 16;   // 112 (NV 16), 96 (NV 32), 80 (NV 48); 48 for 64-channel rows
-  static int bk_env = -1;
-  if (bk_env < 0) {
-    const char* e = getenv("CNB_ATTN_TMEM_BK");
-    bk_env = e ? atoi(e) : 0;
-  }
   auto padded = [&](int bk) { return ceil_div(L, bk) * bk; };
   int bk = BKMAX;
-  if (bk_env) bk = bk_env < BKMAX ? bk_env : BKMAX;
-  else {
-    const int cands[4] = {96, 80, 64, 48};                  // a smaller tile only if it saves more than 6 % of the padded keys
-    for (int i = 0; i < 4; ++i)
-      if (cands[i] < bk && padded(cands[i]) * 100 < padded(bk) * 94) bk = cands[i];
-  }
-  if constexpr (BKMAX >= 112) if (bk >= 112) return launch<DL, D, 112, POLY>(qkv, out, B, L, E, heads, st);
-  if constexpr (BKMAX >= 96) if (bk >= 96) return launch<DL, D, 96, POLY>(qkv, out, B, L, E, heads, st);
-  if constexpr (BKMAX >= 80) if (bk >= 80) return launch<DL, D, 80, POLY>(qkv, out, B, L, E, heads, st);
-  if constexpr (BKMAX >= 64) if (bk >= 64) return launch<DL, D, 64, POLY>(qkv, out, B, L, E, heads, st);
-  return launch<DL, D, 48, POLY>(qkv, out, B, L, E, heads, st);
-}
-
-template <int POLY>
-static int launch_d(const void* qkv, void* out, int B, int L, int E, int heads, cudaStream_t st) {
-  switch (E / heads) {
-    case 4: return launch_bk<16, 4, POLY>(qkv, out, B, L, E, heads, st);
-    case 8: return launch_bk<16, 8, POLY>(qkv, out, B, L, E, heads, st);
-    case 16: return launch_bk<16, 16, POLY>(qkv, out, B, L, E, heads, st);
-    case 24: return launch_bk<32, 24, POLY>(qkv, out, B, L, E, heads, st);
-    case 32: return launch_bk<32, 32, POLY>(qkv, out, B, L, E, heads, st);
-    case 48: return launch_bk<64, 48, POLY>(qkv, out, B, L, E, heads, st);
-    case 64: return launch_bk<64, 64, POLY>(qkv, out, B, L, E, heads, st);
-    default:
-      set_error("attention_tmem: head dim %d not instantiated", E / heads);
-      return CNB_ERR_UNSUPPORTED;
-  }
+  const int cands[4] = {96, 80, 64, 48};                    // a smaller tile only if it saves more than 6 % of the padded keys
+  for (int i = 0; i < 4; ++i)
+    if (cands[i] < bk && padded(cands[i]) * 100 < padded(bk) * 94) bk = cands[i];
+  if constexpr (BKMAX >= 112) if (bk >= 112) return launch<DL, D, 112>(qkv, out, B, L, E, heads, st);
+  if constexpr (BKMAX >= 96) if (bk >= 96) return launch<DL, D, 96>(qkv, out, B, L, E, heads, st);
+  if constexpr (BKMAX >= 80) if (bk >= 80) return launch<DL, D, 80>(qkv, out, B, L, E, heads, st);
+  if constexpr (BKMAX >= 64) if (bk >= 64) return launch<DL, D, 64>(qkv, out, B, L, E, heads, st);
+  return launch<DL, D, 48>(qkv, out, B, L, E, heads, st);
 }
 
 }  // namespace atm
@@ -680,20 +643,8 @@ int attention_tmem_error_flag() { return tc_read_clear_error(); }
 // d = 64: 0.19 vs 0.49 ms; CelebHQ-latent 32x32 d = 24: 1.50 vs 1.95 ms, 16x16 d = 32: 0.139 vs 0.167 ms; MNIST 14x14
 // d = 32: 0.131 vs 0.135 ms); at head dims <= 16 the register-resident mma.sync kernel is still ahead (28x28 d = 16:
 // 0.90 vs 1.09 ms) and sequences of <= 64 tokens are one tile of either kernel (latency only).
-// CNB_ATTN_TMEM = 0 never, 1 measured rule (default), 2 every supported shape; CNB_ATTN_TMEM_MINL / _MIND move the rule.
-bool attention_tmem_default(int L, int d) {
-  static int on = -1, minl = 128, mind = 24;
-  if (on < 0) {
-    const char* e = getenv("CNB_ATTN_TMEM");
-    on = e ? atoi(e) : 1;
-    const char* m = getenv("CNB_ATTN_TMEM_MINL");
-    if (m) minl = atoi(m);
-    const char* dd = getenv("CNB_ATTN_TMEM_MIND");
-    if (dd) mind = atoi(dd);
-  }
-  if (on == 2) return true;
-  return on != 0 && L >= minl && d >= mind;
-}
+// runtime.attention_kernel_name mirrors this rule.
+bool attention_tmem_default(int L, int d) { return L >= 128 && d >= 24; }
 
 bool attention_tmem_supported(const void* qkv, const void* out, int B, int L, int E, int heads) {
   if (heads <= 0 || E % heads) return false;
@@ -705,15 +656,17 @@ bool attention_tmem_supported(const void* qkv, const void* out, int B, int L, in
 }
 
 int attention_tmem(const void* qkv, void* out, int B, int L, int E, int heads, cudaStream_t st) {
-  static int poly = -1;                                    // eighths of the exponentials evaluated on the FMA pipe
-  if (poly < 0) {
-    const char* e = getenv("CNB_ATTN_POLY");
-    poly = e ? atoi(e) : 0;
-  }
-  switch (poly) {
-    case 1: return atm::launch_d<1>(qkv, out, B, L, E, heads, st);
-    case 2: return atm::launch_d<2>(qkv, out, B, L, E, heads, st);
-    default: return atm::launch_d<0>(qkv, out, B, L, E, heads, st);
+  switch (E / heads) {
+    case 4: return atm::launch_bk<16, 4>(qkv, out, B, L, E, heads, st);
+    case 8: return atm::launch_bk<16, 8>(qkv, out, B, L, E, heads, st);
+    case 16: return atm::launch_bk<16, 16>(qkv, out, B, L, E, heads, st);
+    case 24: return atm::launch_bk<32, 24>(qkv, out, B, L, E, heads, st);
+    case 32: return atm::launch_bk<32, 32>(qkv, out, B, L, E, heads, st);
+    case 48: return atm::launch_bk<64, 48>(qkv, out, B, L, E, heads, st);
+    case 64: return atm::launch_bk<64, 64>(qkv, out, B, L, E, heads, st);
+    default:
+      set_error("attention_tmem: head dim %d not instantiated", E / heads);
+      return CNB_ERR_UNSUPPORTED;
   }
 }
 

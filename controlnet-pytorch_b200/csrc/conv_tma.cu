@@ -66,14 +66,8 @@ static int pick_rb(int cin, int elt) {
   return (cin * elt) % 16 == 0 ? 32 : 0;
 }
 
-static int g_tma_enabled = -1;
-
 bool conv2d_tma_supported(const cnb_conv_params* p) {
-  if (g_tma_enabled < 0) {
-    const char* e = getenv("CNB_CONV_TMA");
-    g_tma_enabled = e ? atoi(e) : 1;
-  }
-  if (!g_tma_enabled || p->mode == CNB_MODE_F32) return false;
+  if (p->mode == CNB_MODE_F32) return false;
   const bool half = p->in_dtype == 1;
   const int elt = half ? 2 : 4;
   if (half && !p->weight_lp) return false;
@@ -134,15 +128,10 @@ int conv2d_tma(const cnb_conv_params* p, cudaStream_t st) {
   bool halo = false;
   int Wp = p->W + 2, R = 0, halo_stage = 0;
   {
-    static int halo_on = -1;
-    if (halo_on < 0) {
-      const char* e = getenv("CNB_CONV_HALO");
-      halo_on = e ? atoi(e) : 1;
-    }
     bool std3 = p->ntaps == 9 && p->stride == 1 && p->OH == p->H && p->OW == p->W && p->oy_mul == 1 && p->ox_mul == 1 &&
                 p->oy_add == 0 && p->ox_add == 0 && p->OHf == p->OH && p->OWf == p->OW && p->Cout == bn_h;
     for (int t = 0; t < 9 && std3; ++t) std3 = p->dy[t] == t / 3 - 1 && p->dx[t] == t % 3 - 1;
-    if (halo_on && std3 && Wp <= 64 && p->W >= 12) {
+    if (std3 && Wp <= 64 && p->W >= 12) {
       R = BM / Wp;
       const int tiles_y = ceil_div(p->H, R);
       const double useful = (double)p->H * p->W / ((double)tiles_y * BM);
@@ -234,37 +223,16 @@ int conv2d_tma(const cnb_conv_params* p, cudaStream_t st) {
     // and its own A tile through one SM's L2 port (~64 B/clk: measured 24 us for 3x3 256+256->256 @7x7 at batch 128, 49
     // CTAs on 49 SMs, 2 MB each, against 10 us of tensor time).  Narrower N tiles spread the weights over more SMs - the K
     // order, hence the result, does not change.  Enter when the layer has fewer CTAs than SMs / ENTER, narrow until it has
-    // at least SMs / STOP (CNB_CONV_NSPLIT_ENTER / _STOP; measured defaults, profiles/r02_conv_nsplit.md).
-    static int ns_enter = -1, ns_stop = 2;
-    if (ns_enter < 0) {
-      const char* e = getenv("CNB_CONV_NSPLIT_ENTER");
-      ns_enter = e ? atoi(e) : 2;
-      const char* s2 = getenv("CNB_CONV_NSPLIT_STOP");
-      ns_stop = s2 ? atoi(s2) : 2;
-      if (ns_enter < 1) ns_enter = 1;
-      if (ns_stop < 1) ns_stop = 1;
-    }
+    // at least SMs / STOP (ENTER = STOP = 2, measured: profiles/r02_conv_nsplit.md).
+    constexpr int NS_ENTER = 2, NS_STOP = 2;
     const int tiles_m = ceil_div((long long)p->B * p->OH * p->OW, BM);
-    if (tiles_m * (p->Cout / bn) * ns_enter <= g_num_sms) {
+    if (tiles_m * (p->Cout / bn) * NS_ENTER <= g_num_sms) {
       static const int cand[] = {128, 96, 64, 48, 32};
       for (int c : cand) {
         if (c >= bn || p->Cout % c) continue;
         bn = c;
-        if (tiles_m * (p->Cout / bn) * ns_stop >= g_num_sms) break;
+        if (tiles_m * (p->Cout / bn) * NS_STOP >= g_num_sms) break;
       }
-    }
-  }
-  {
-    // experiment (CNB_CONV_2CTA=3): N tiles of at most 128 columns everywhere, so that every layer can run two CTAs per SM
-    static int two_env = -2;
-    if (two_env == -2) {
-      const char* e = getenv("CNB_CONV_2CTA");
-      two_env = e ? atoi(e) : 2;
-    }
-    if (two_env >= 3 && !halo && bn > 128) {
-      static const int cand[] = {128, 96, 64};
-      for (int c : cand)
-        if (p->Cout % c == 0) { bn = c; break; }
     }
   }
   {
@@ -285,16 +253,11 @@ int conv2d_tma(const cnb_conv_params* p, cudaStream_t st) {
   }
   // ---- dense fp16 output (+ fp16 residual): the epilogue stores / fetches 32-row x SLAB-column boxes by TMA (EPI 6)
   {
-    static int epi_tma = -1;
-    if (epi_tma < 0) {
-      const char* e = getenv("CNB_CONV_EPI_TMA");
-      epi_tma = e ? atoi(e) : 1;
-    }
     const bool dense = !halo && p->oy_mul == 1 && p->ox_mul == 1 && p->oy_add == 0 && p->ox_add == 0 &&
                        p->OHf * p->OWf == p->OH * p->OW;
     const bool simple = dense && p->act == 0 && !(p->temb && p->temb_per_sample);
     const bool res_ok = !p->residual || (p->res_dtype == 1 && p->ldr % 8 == 0 && p->res_coff % 8 == 0);
-    if (epi_tma && half && simple && p->out_dtype == 1 && p->ldo % 8 == 0 && p->out_coff % 8 == 0 && res_ok) {
+    if (half && simple && p->out_dtype == 1 && p->ldo % 8 == 0 && p->out_coff % 8 == 0 && res_ok) {
       const int slab = bn % 64 == 0 ? 32 : 16;
       const CUtensorMapSwizzle sw_o = slab == 32 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_32B;
       const cuuint64_t dims[2] = {(cuuint64_t)p->Cout, (cuuint64_t)p->B * p->OH * p->OW};

@@ -691,17 +691,6 @@ conv_tma_kernel(const __grid_constant__ TmaArgs a) {
   }
 }
 
-// Resident weights pay off when a CTA runs several tiles against the same [nkb][BN x RB] weight block and that block
-// leaves room for a >= 4-deep A ring: L2 -> smem traffic per tile drops from A + B to A.
-inline int g_bres_enabled() {
-  static int v = -1;
-  if (v < 0) {
-    const char* e = getenv("CNB_CONV_BRES");
-    v = e ? atoi(e) : 1;
-  }
-  return v;
-}
-
 template <int BN, bool HALF, int EPI, int RB>
 static int launch_epi(const TmaArgs& a_in, int num_sms, cudaStream_t st) {
   using C = Cfg<BN, RB>;
@@ -729,7 +718,9 @@ static int launch_epi(const TmaArgs& a_in, int num_sms, cudaStream_t st) {
       o.epi_off = o.ring_off + s_h * o.halo_stage_bytes;
       return s_h;
     }
-    if (g_bres_enabled() && o.tiles_n == 1 && ntiles >= 3 * ctas && s_res >= 4) {
+    // Resident weights pay off when a CTA runs several tiles against the same [nkb][BN x RB] weight block and that block
+    // leaves room for a >= 4-deep A ring: L2 -> smem traffic per tile drops from A + B to A.
+    if (o.tiles_n == 1 && ntiles >= 3 * ctas && s_res >= 4) {
       o.bres = 1;
       o.s_run = s_res;
       o.ring_off = b_res_bytes;
@@ -748,17 +739,13 @@ static int launch_epi(const TmaArgs& a_in, int num_sms, cudaStream_t st) {
   };
   // Two CTAs per SM (half the shared memory each, TMEM 2 x <= 256 columns): two independent load -> MMA -> epilogue
   // pipelines share an SM, which hides the per-tile latency chains of the short-K layers and lets the next kernel's
-  // prologue overlap this kernel's tail.  Needs BN <= 128 (TMEM) and a specialised epilogue (<= 102 registers).
-  static int two_env = -2;
-  if (two_env == -2) {
-    const char* e = getenv("CNB_CONV_2CTA");
-    two_env = e ? atoi(e) : 2;
-  }
+  // prologue overlap this kernel's tail.  Needs BN <= 128 (TMEM), a specialised epilogue (<= 102 registers) and a ring
+  // of depth >= 2 in 112 KB.
   int grid = ntiles < num_sms ? ntiles : num_sms;
   bool two = false;
-  if (two_env && BN <= 128 && EPI != 3 && ntiles >= 2 * num_sms) {
+  if (BN <= 128 && EPI != 3 && ntiles >= 2 * num_sms) {
     TmaArgs t = a_in;
-    if (plan(112 * 1024, 2 * num_sms, t) >= (two_env >= 2 ? 2 : 3)) {
+    if (plan(112 * 1024, 2 * num_sms, t) >= 2) {
       a = t;
       two = true;
       grid = ntiles < 2 * num_sms ? ntiles : 2 * num_sms;
@@ -776,28 +763,18 @@ static int launch_epi(const TmaArgs& a_in, int num_sms, cudaStream_t st) {
   if (EPI == 6) {
     // a third staging buffer per epilogue warp where shared memory is left over: the residual box of slab i+1 can then
     // be requested while the store of slab i-1 is still reading its buffer
-    static int nbuf_env = -1;
-    if (nbuf_env < 0) {
-      const char* e = getenv("CNB_CONV_EPI_NBUF");
-      nbuf_env = e ? atoi(e) : 0;
-    }
     const int budget = two ? 112 * 1024 : SMEM_BUDGET;
     const int e6_3 = EPI_WARPS * C::e6_warp_bytes(3);
     const bool fits3 = a.epi_off + e6_3 + C::BAR_BYTES + 1024 <= budget;
-    a.epi_nbuf = (nbuf_env == 2 || !fits3) ? 2 : 3;
+    a.epi_nbuf = fits3 ? 3 : 2;
     if (a.epi_nbuf == 3 && e6_3 > C::EPI_BYTES) a.bar_off = a.epi_off + e6_3;
   }
   {
     // alternate-tile epilogue when a tile's tensor work (~BN * K / 32 cycles) is shorter than its epilogue
-    static int alt_env = -2;
-    if (alt_env == -2) {
-      const char* e = getenv("CNB_CONV_EPI_ALT");
-      alt_env = e ? atoi(e) : -1;
-    }
     const long long ktot = (long long)nkb * (RB / (HALF ? 2 : 4));   // nkb counts every (tap, chunk) block
     // measured (B = 1024): halo 3x3 16->16 @28 54 -> 44 us, 64->64 @28 97 -> 91, 32->64 @28 89 -> 83; dense 1x1 layers
     // with several column slabs lose (256->768 @7 40 -> 44 us), so only the halo layers switch
-    a.epi_alt = alt_env >= 0 ? alt_env : ((a.halo && (long long)BN * ktot < 131072) ? 1 : 0);
+    a.epi_alt = (a.halo && (long long)BN * ktot < 131072) ? 1 : 0;
     if (EPI == 6) a.epi_alt = 0;
   }
   smem_bytes = (size_t)a.bar_off + C::BAR_BYTES + 1024;

@@ -5,8 +5,6 @@
 // Per-thread column ownership (thread <-> fixed 4 channels) makes the reduction a deterministic tree:
 // registers -> smem [rows][C] -> per-channel -> per-group.
 #include <cuda_fp16.h>
-#include <stdlib.h>
-#include <string.h>
 
 #include "common.cuh"
 
@@ -215,28 +213,15 @@ groupnorm_nhwc_kernel(const void* __restrict__ x, void* __restrict__ y, const fl
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// Register-resident variant: grid (SPLIT, B), a thread-block cluster of SPLIT CTAs per sample.  Every CTA loads its
-// slice of the [HW, C] slab ONCE into registers (up to KMAX float4 per thread, all loads in flight together),
-// statistics are reduced thread -> smem -> CTA -> cluster (distributed shared memory), and the normalised values are
-// stored from the same registers: exactly one global read and one global write per element, no L2 re-read.
-// Same two-pass numerics (mean, then centred second moment) as the kernel above.
+// Register-resident variant: one CTA per sample (grid (1, B)).  The CTA loads the [HW, C] slab ONCE into registers (up
+// to KMAX float4 per thread, all loads in flight together), statistics are reduced thread -> smem -> CTA, and the
+// normalised values are stored from the same registers: exactly one global read and one global write per element, no
+// L2 re-read.  Same two-pass numerics (mean, then centred second moment) as the kernel above.
 // ---------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ float ld_dsmem(const float* p, uint32_t cta_rank) {
-  const uint32_t a = (uint32_t)__cvta_generic_to_shared(p);
-  uint32_t r;
-  float v;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(a), "r"(cta_rank));
-  asm volatile("ld.shared::cluster.f32 %0, [%1];" : "=f"(v) : "r"(r) : "memory");
-  return v;
-}
-
 template <int KMAX, bool SILU, bool HALF, bool HIN>
 __global__ void __launch_bounds__(256)
 groupnorm_reg_kernel(const void* __restrict__ x, void* __restrict__ y, const float* __restrict__ gamma,
-                     const float* __restrict__ beta, int HW, int C, int G, float eps, int rows_per_cta) {
+                     const float* __restrict__ beta, int HW, int C, int G, float eps) {
   pdl_trigger();
   pdl_wait();
   extern __shared__ float sm[];
@@ -245,19 +230,14 @@ groupnorm_reg_kernel(const void* __restrict__ x, void* __restrict__ y, const flo
   const int R = NT / C4;            // pixel rows covered per sweep
   float* part = sm;                 // [R][C]
   float* chan = part + R * C;       // [C]
-  float* gpart1 = chan + C;         // [G] this CTA's group sums (pass 1), read by the whole cluster
-  float* gpart2 = gpart1 + G;       // [G] pass 2
-  float* g_mean = gpart2 + G;       // [G]
+  float* g_mean = chan + C;         // [G]
   float* g_rstd = g_mean + G;       // [G]
 
   const int tid = threadIdx.x;
   const int col = tid % C4;
   const int r0 = tid / C4;
   const int cg = C / G;
-  const int split = gridDim.x, rank = blockIdx.x;
-  const int row0 = rank * rows_per_cta;
-  const int nrows = min(rows_per_cta, HW - row0);
-  const size_t slab = ((size_t)blockIdx.y * HW + row0) * C4;
+  const size_t slab = (size_t)blockIdx.y * HW * C4;
   using IV = InVec<HIN>;
   const typename IV::type* xs = reinterpret_cast<const typename IV::type*>(x) + slab;
   using OV = OutVec<HALF>;
@@ -268,7 +248,7 @@ groupnorm_reg_kernel(const void* __restrict__ x, void* __restrict__ y, const flo
 #pragma unroll
   for (int k = 0; k < KMAX; ++k) {
     const int row = r0 + k * R;
-    v[k] = row < nrows ? IV::load_cs(xs + (size_t)row * C4 + col) : make_float4(0.f, 0.f, 0.f, 0.f);
+    v[k] = row < HW ? IV::load_cs(xs + (size_t)row * C4 + col) : make_float4(0.f, 0.f, 0.f, 0.f);
   }
 
   // ---- pass 1: sums -> group means
@@ -286,13 +266,6 @@ groupnorm_reg_kernel(const void* __restrict__ x, void* __restrict__ y, const flo
   for (int g = tid; g < G; g += NT) {
     float t = 0.f;
     for (int c = 0; c < cg; ++c) t += chan[g * cg + c];
-    gpart1[g] = t;
-  }
-  if (split > 1) cluster_sync_all(); else __syncthreads();
-  for (int g = tid; g < G; g += NT) {
-    float t = 0.f;
-    if (split > 1) { for (int q = 0; q < split; ++q) t += ld_dsmem(gpart1 + g, (uint32_t)q); }
-    else t = gpart1[g];
     g_mean[g] = t * inv_n;
   }
   __syncthreads();
@@ -304,7 +277,7 @@ groupnorm_reg_kernel(const void* __restrict__ x, void* __restrict__ y, const flo
   s = make_float4(0.f, 0.f, 0.f, 0.f);
 #pragma unroll
   for (int k = 0; k < KMAX; ++k) {
-    if (r0 + k * R < nrows) {
+    if (r0 + k * R < HW) {
       float d;
       d = v[k].x - m0; s.x = fmaf(d, d, s.x);
       d = v[k].y - m1; s.y = fmaf(d, d, s.y);
@@ -323,13 +296,6 @@ groupnorm_reg_kernel(const void* __restrict__ x, void* __restrict__ y, const flo
   for (int g = tid; g < G; g += NT) {
     float t = 0.f;
     for (int c = 0; c < cg; ++c) t += chan[g * cg + c];
-    gpart2[g] = t;
-  }
-  if (split > 1) cluster_sync_all(); else __syncthreads();
-  for (int g = tid; g < G; g += NT) {
-    float t = 0.f;
-    if (split > 1) { for (int q = 0; q < split; ++q) t += ld_dsmem(gpart2 + g, (uint32_t)q); }
-    else t = gpart2[g];
     g_rstd[g] = rsqrtf(t * inv_n + eps);
   }
   __syncthreads();
@@ -343,64 +309,38 @@ groupnorm_reg_kernel(const void* __restrict__ x, void* __restrict__ y, const flo
 #pragma unroll
   for (int k = 0; k < KMAX; ++k) {
     const int row = r0 + k * R;
-    if (row < nrows) {
+    if (row < HW) {
       float4 o;
       o.x = fmaf(v[k].x, a0, b0); o.y = fmaf(v[k].y, a1, b1); o.z = fmaf(v[k].z, a2, b2); o.w = fmaf(v[k].w, a3, b3);
       if (SILU) { o.x = silu_out<HALF>(o.x); o.y = silu_out<HALF>(o.y); o.z = silu_out<HALF>(o.z); o.w = silu_out<HALF>(o.w); }
       ys[(size_t)row * C4 + col] = OV::pack(o);
     }
   }
-  // a CTA may not exit while a peer can still read its shared memory
-  if (split > 1) cluster_sync_all();
 }
 
 template <int KMAX, bool SILU, bool HALF, bool HIN>
-static cudaError_t launch_reg_one(cudaLaunchConfig_t* cfg, const void* x, void* y, const float* gamma, const float* beta,
-                                  int HW, int C, int G, float eps, int rows_per_cta) {
-  return cudaLaunchKernelEx(cfg, groupnorm_reg_kernel<KMAX, SILU, HALF, HIN>, x, y, gamma, beta, HW, C, G, eps,
-                            rows_per_cta);
+static cudaError_t launch_reg_one(const void* x, void* y, const float* gamma, const float* beta, int B, int HW, int C,
+                                  int G, float eps, int NT, cudaStream_t st) {
+  const size_t smem = ((size_t)(NT / (C / 4)) * C + C + 2 * G) * sizeof(float);
+  return launch_pdl((long long)B * HW * C, groupnorm_reg_kernel<KMAX, SILU, HALF, HIN>, dim3(1, B), dim3(NT), smem, st,
+                    x, y, gamma, beta, HW, C, G, eps);
 }
 
 template <int KMAX>
 static int launch_reg(const void* x, void* y, const float* gamma, const float* beta, int B, int HW, int C, int G,
-                      float eps, int silu, int in_f16, int out_f16, int split, int rows_per_cta, int NT,
-                      cudaStream_t st) {
-  const int R = NT / (C / 4);
-  const size_t smem = ((size_t)R * C + C + 4 * G) * sizeof(float);
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3(split, B, 1);
-  cfg.blockDim = dim3(NT, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = split;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  if (split == 1) {      // single-CTA samples: plain (non-cluster) launch that may overlap its predecessor's tail
-    attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[0].val.programmaticStreamSerializationAllowed = pdl_enabled((long long)B * HW * C) ? 1 : 0;
-  }
-  cudaError_t e;
+                      float eps, int silu, int in_f16, int out_f16, int NT, cudaStream_t st) {
   const int sel = (silu ? 4 : 0) | (out_f16 ? 2 : 0) | (in_f16 ? 1 : 0);
   switch (sel) {
-    case 0: e = launch_reg_one<KMAX, false, false, false>(&cfg, x, y, gamma, beta, HW, C, G, eps, rows_per_cta); break;
-    case 1: e = launch_reg_one<KMAX, false, false, true>(&cfg, x, y, gamma, beta, HW, C, G, eps, rows_per_cta); break;
-    case 2: e = launch_reg_one<KMAX, false, true, false>(&cfg, x, y, gamma, beta, HW, C, G, eps, rows_per_cta); break;
-    case 3: e = launch_reg_one<KMAX, false, true, true>(&cfg, x, y, gamma, beta, HW, C, G, eps, rows_per_cta); break;
-    case 4: e = launch_reg_one<KMAX, true, false, false>(&cfg, x, y, gamma, beta, HW, C, G, eps, rows_per_cta); break;
-    case 5: e = launch_reg_one<KMAX, true, false, true>(&cfg, x, y, gamma, beta, HW, C, G, eps, rows_per_cta); break;
-    case 6: e = launch_reg_one<KMAX, true, true, false>(&cfg, x, y, gamma, beta, HW, C, G, eps, rows_per_cta); break;
-    default: e = launch_reg_one<KMAX, true, true, true>(&cfg, x, y, gamma, beta, HW, C, G, eps, rows_per_cta); break;
+    case 0: CNB_CUDA((launch_reg_one<KMAX, false, false, false>(x, y, gamma, beta, B, HW, C, G, eps, NT, st))); break;
+    case 1: CNB_CUDA((launch_reg_one<KMAX, false, false, true>(x, y, gamma, beta, B, HW, C, G, eps, NT, st))); break;
+    case 2: CNB_CUDA((launch_reg_one<KMAX, false, true, false>(x, y, gamma, beta, B, HW, C, G, eps, NT, st))); break;
+    case 3: CNB_CUDA((launch_reg_one<KMAX, false, true, true>(x, y, gamma, beta, B, HW, C, G, eps, NT, st))); break;
+    case 4: CNB_CUDA((launch_reg_one<KMAX, true, false, false>(x, y, gamma, beta, B, HW, C, G, eps, NT, st))); break;
+    case 5: CNB_CUDA((launch_reg_one<KMAX, true, false, true>(x, y, gamma, beta, B, HW, C, G, eps, NT, st))); break;
+    case 6: CNB_CUDA((launch_reg_one<KMAX, true, true, false>(x, y, gamma, beta, B, HW, C, G, eps, NT, st))); break;
+    default: CNB_CUDA((launch_reg_one<KMAX, true, true, true>(x, y, gamma, beta, B, HW, C, G, eps, NT, st))); break;
   }
-  if (e != cudaSuccess) {
-    set_error("groupnorm_reg launch failed: %s", cudaGetErrorString(e));
-    return CNB_ERR_CUDA;
-  }
-  count_launch();
+  CNB_LAUNCH_CHECK();
   return CNB_OK;
 }
 
@@ -492,21 +432,12 @@ static void launch_warp(const void* x, void* y, const float* gamma, const float*
   }
 }
 
-static int g_gn_reg = -1;
-static int g_gn_warp = -1;
-
-static int g_gn_stage = -1;
-
 template <bool SILU, bool HALF, bool HIN>
 static void launch_sweep(const void* x, void* y, const float* gamma, const float* beta, int B, int NT, size_t smem,
                          int HW, int C, int G, float eps, cudaStream_t st) {
-  if (g_gn_stage < 0) {
-    const char* e = getenv("CNB_GN_STAGE");
-    g_gn_stage = e ? atoi(e) : 1;
-  }
   const size_t slab = (size_t)HW * C * 2;                  // fp16 slab
   const size_t staged = (smem + 127) / 128 * 128 + slab;
-  if (HIN && g_gn_stage && slab % 16 == 0 && slab < (1u << 20) && staged <= 110 * 1024) {
+  if (HIN && slab % 16 == 0 && slab < (1u << 20) && staged <= 110 * 1024) {
     static DeviceOnce attr_once;
     if (attr_once.first()) {
       cudaFuncSetAttribute(groupnorm_nhwc_kernel<SILU, HALF, HIN, HIN>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -523,18 +454,10 @@ static void launch_sweep(const void* x, void* y, const float* gamma, const float
 int groupnorm(const void* x, void* y, const float* gamma, const float* beta, int B, int HW, int C, int G,
               float eps, int silu, int in_f16, int out_f16, cudaStream_t st) {
   CNB_REQUIRE(C % 4 == 0 && C % G == 0 && C / 4 <= 1024, "groupnorm: C=%d G=%d unsupported", C, G);
-  if (g_gn_reg < 0) {
-    const char* e = getenv("CNB_GN_REG");
-    g_gn_reg = e ? atoi(e) : 1;
-  }
   // Warp-per-group kernel: groups of 16 / 32 / 64 / 128 channels whose pixels fit 13 vectors per lane
-  if (g_gn_warp < 0) {
-    const char* e = getenv("CNB_GN_WARP");
-    g_gn_warp = e ? atoi(e) : 1;
-  }
   {
     const int cgq = (C / G) / 4;
-    if (g_gn_warp && (C / G) % 4 == 0 && (cgq == 4 || cgq == 8 || cgq == 16 || cgq == 32)) {
+    if ((C / G) % 4 == 0 && (cgq == 4 || cgq == 8 || cgq == 16 || cgq == 32)) {
       const int k = ceil_div(HW, 32 / cgq);
       if (k <= 13) {      // (25 vectors per lane was tried for 128 ch @ 14x14: register pressure makes it lose to the staged kernel)
         if (k <= 7) launch_warp<7>(x, y, gamma, beta, B, HW, C, G, eps, silu, in_f16, out_f16, st);
@@ -545,27 +468,16 @@ int groupnorm(const void* x, void* y, const float* gamma, const float* beta, int
     }
   }
   // Register-resident kernel when one CTA holds a whole sample (<= 256 threads x 16 float4): measured 1.2-1.6x faster
-  // than the three-sweep kernel on the 7x7 / 16-channel slabs.  Splitting a sample over a cluster (CNB_GN_SPLIT=8)
-  // works but loses to the three-sweep kernel on the large slabs (cluster barriers + co-scheduling), so it is off.
-  if (g_gn_reg && C / 4 <= 256 && B <= 65535) {
-    static int max_split = -1;
-    if (max_split < 0) {
-      const char* e = getenv("CNB_GN_SPLIT");
-      max_split = e ? atoi(e) : 1;
-    }
+  // than the three-sweep kernel on the 7x7 / 16-channel slabs.  (Splitting a sample over a thread-block cluster was
+  // measured too: it loses to the three-sweep kernel on the large slabs - cluster barriers + co-scheduling.)
+  if (C / 4 <= 256 && B <= 65535) {
     const int C4r = C / 4;
     const int NTr = (256 / C4r) * C4r;
-    const int Rr = NTr / C4r;
-    for (int split = 1; split <= max_split && split <= HW; split *= 2) {
-      const int rows = ceil_div(HW, split);
-      const int k = ceil_div(rows, Rr);
-      if (k <= 16) {
-        if (k <= 4) return launch_reg<4>(x, y, gamma, beta, B, HW, C, G, eps, silu, in_f16, out_f16, split, rows, NTr, st);
-        if (k <= 8) return launch_reg<8>(x, y, gamma, beta, B, HW, C, G, eps, silu, in_f16, out_f16, split, rows, NTr, st);
-        if (k <= 13) return launch_reg<13>(x, y, gamma, beta, B, HW, C, G, eps, silu, in_f16, out_f16, split, rows, NTr, st);
-        return launch_reg<16>(x, y, gamma, beta, B, HW, C, G, eps, silu, in_f16, out_f16, split, rows, NTr, st);
-      }
-    }
+    const int k = ceil_div(HW, NTr / C4r);
+    if (k <= 4) return launch_reg<4>(x, y, gamma, beta, B, HW, C, G, eps, silu, in_f16, out_f16, NTr, st);
+    if (k <= 8) return launch_reg<8>(x, y, gamma, beta, B, HW, C, G, eps, silu, in_f16, out_f16, NTr, st);
+    if (k <= 13) return launch_reg<13>(x, y, gamma, beta, B, HW, C, G, eps, silu, in_f16, out_f16, NTr, st);
+    if (k <= 16) return launch_reg<16>(x, y, gamma, beta, B, HW, C, G, eps, silu, in_f16, out_f16, NTr, st);
   }
   const int C4 = C / 4;
   int R = 512 / C4;

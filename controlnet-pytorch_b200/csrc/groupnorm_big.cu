@@ -15,7 +15,6 @@
 // Algorithmic bytes: 2 B read + 2 B written per element; the second read of a range follows its first within a few
 // hundred microseconds and is an L2 hit whenever B * slab stays under the 126 MB L2, else DRAM sees 2 reads + 1 write.
 #include <cuda_fp16.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 
@@ -231,12 +230,7 @@ static void plan(int B, int HW, int C, int* S_out, int* rows_out) {
 
 bool groupnorm_big_eligible(int B, int HW, int C, int G, int in_f16) {
   if (!in_f16 || C % 8 || C % G || C / 8 > gnb::NT || B > 65535) return false;
-  static long long min_bytes = -1;                        // CNB_GN_BIG_MIN_BYTES: experiment knob
-  if (min_bytes < 0) {
-    const char* e = getenv("CNB_GN_BIG_MIN_BYTES");
-    min_bytes = e ? atoll(e) : 110 * 1024;                // default: beyond the staged one-CTA-per-sample kernel
-  }
-  return (long long)HW * C * 2 > min_bytes;
+  return (long long)HW * C * 2 > 110 * 1024;              // beyond the staged one-CTA-per-sample kernel
 }
 
 size_t groupnorm_big_workspace(int B, int HW, int C, int G) {

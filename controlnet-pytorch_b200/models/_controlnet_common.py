@@ -20,12 +20,6 @@ def split_prefix(state, prefix, exclude=()):
             if k.startswith(prefix) and not any(k.startswith(e) for e in exclude)}
 
 
-def set_branch_parallel(value):
-    """Override CNB_BRANCH_PARALLEL for the calls that follow (None restores the default); used by the sampler when it
-    already runs batch parts on parallel streams."""
-    E._FORCE_PAR[0] = value
-
-
 _side_stream = E.side_stream
 
 
@@ -69,15 +63,10 @@ def controlnet_forward(trained, control, down_zero, mid_zero, hint_feat_fn, x, t
     # step at 128 samples 2.42 -> 2.24 ms, at 1024 samples 11.98 -> 11.80 ms; CelebHQ LDM at 256: 28.25 -> 27.7 ms; DESIGN.md 5);
     # the kernels of one branch fill the pipes the other leaves idle (MUFU-bound attention next to tensor- / HBM-bound
     # convolutions and GroupNorms).  Same kernels, same inputs, same order per tensor: results are bit-identical to the
-    # sequential schedule.  CNB_BRANCH_PARALLEL=0 turns it off; CNB_BRANCH_PARALLEL=2 is the round-1 layout (control
-    # encoder + all its mids on the side stream, everything else after the join).
+    # sequential schedule.
     # Only under graph capture: in eager mode the extra stream bookkeeping (event waits, record_stream on every
     # hand-over tensor) is host time, which is what a small-batch eager loop is bound by (CelebHQ B = 16: 6.9 -> 19.7 ms).
-    layout = E.capture_parallel()
-    parallel = layout != "0"
-    early_mid = layout == "1"
-
-    if not parallel:
+    if not E.capture_parallel():
         plan_t = E.temb_plan(trained, E.unet_time(trained, t, dev))
         plan_c = E.temb_plan(control, E.unet_time(control, t, dev), with_ups=False)
         a = E.conv_in(trained, xn, mode)
@@ -101,28 +90,23 @@ def controlnet_forward(trained, control, down_zero, mid_zero, hint_feat_fn, x, t
         cur = torch.cuda.current_stream(dev)
         side = _side_stream(dev, 0)
         skip = _side_stream(dev, 1)
+        aux = _side_stream(dev, 2)
         E.prewarm_conv_in(trained, xn, mode)       # the padded fp16 copy both conv_in layers read: before the fork
-        if early_mid:
-            # the two t-embedding chains (4 small launches each) leave the critical paths as well: they are only needed
-            # by the first resnet's conv1 epilogue, after conv_in and a GroupNorm
-            aux = _side_stream(dev, 2)
-            skip.wait_stream(cur)
-            aux.wait_stream(cur)
-            with torch.cuda.stream(skip):
-                plan_t = E.temb_plan(trained, E.unet_time(trained, t, dev))
-                ev_pt = skip.record_event()
-            with torch.cuda.stream(aux):
-                plan_c = E.temb_plan(control, E.unet_time(control, t, dev), with_ups=False)
-                ev_pc = aux.record_event()
+        # the two t-embedding chains (4 small launches each) leave the critical paths as well: they are only needed by
+        # the first resnet's conv1 epilogue, after conv_in and a GroupNorm
+        skip.wait_stream(cur)
+        aux.wait_stream(cur)
+        with torch.cuda.stream(skip):
+            plan_t = E.temb_plan(trained, E.unet_time(trained, t, dev))
+            ev_pt = skip.record_event()
+        with torch.cuda.stream(aux):
+            plan_c = E.temb_plan(control, E.unet_time(control, t, dev), with_ups=False)
+            ev_pc = aux.record_event()
         side.wait_stream(cur)
         with torch.cuda.stream(side):
-            if early_mid:
-                c = E.conv_in(control, xn, mode, residual=hf)
-                side.wait_event(ev_pc)
-                next(iter(plan_c.values())).table.record_stream(side)
-            else:
-                plan_c = E.temb_plan(control, E.unet_time(control, t, dev), with_ups=False)
-                c = E.conv_in(control, xn, mode, residual=hf)
+            c = E.conv_in(control, xn, mode, residual=hf)
+            side.wait_event(ev_pc)
+            next(iter(plan_c.values())).table.record_stream(side)
             cs, cms, ev_mid = [], [], []
             for d in control.downs:
                 cs.append(c)
@@ -132,41 +116,29 @@ def controlnet_forward(trained, control, down_zero, mid_zero, hint_feat_fn, x, t
                 c = E.run_mid(mblk, c, plan_c[mblk], mode)
                 cms.append(c)
                 ev_mid.append(side.record_event())
-        if early_mid:
-            a = E.conv_in(trained, xn, mode)
-            cur.wait_event(ev_pt)
-            next(iter(plan_t.values())).table.record_stream(cur)
-        else:
-            plan_t = E.temb_plan(trained, E.unet_time(trained, t, dev))
-            a = E.conv_in(trained, xn, mode)
+        a = E.conv_in(trained, xn, mode)
+        cur.wait_event(ev_pt)
+        next(iter(plan_t.values())).table.record_stream(cur)
         t_skips = []
         for d in trained.downs:
             t_skips.append(a)
             a = E.run_down(d, a, plan_t[d], mode)
-        if early_mid:
-            skip.wait_stream(cur)                  # trained skips
-            skip.wait_event(ev_enc)                # control skips
-            with torch.cuda.stream(skip):
-                for tns in cs + t_skips:
-                    tns.record_stream(skip)
-                cats = skip_sums(cs, t_skips)
-            for i in range(nmid):
-                a = E.run_mid(trained.mids[i], a, plan_t[trained.mids[i]], mode)
-                cur.wait_event(ev_mid[i])
-                cms[i].record_stream(cur)
-                a = inject(i, a, cms[i])
-            cur.wait_stream(side)
-            cur.wait_stream(skip)
-            cur.wait_stream(aux)
-            for tns in cats:
-                tns.record_stream(cur)
-        else:
-            cur.wait_stream(side)
-            for tns in cs + cms:
-                tns.record_stream(cur)
+        skip.wait_stream(cur)                      # trained skips
+        skip.wait_event(ev_enc)                    # control skips
+        with torch.cuda.stream(skip):
+            for tns in cs + t_skips:
+                tns.record_stream(skip)
             cats = skip_sums(cs, t_skips)
-            for i in range(nmid):
-                a = inject(i, E.run_mid(trained.mids[i], a, plan_t[trained.mids[i]], mode), cms[i])
+        for i in range(nmid):
+            a = E.run_mid(trained.mids[i], a, plan_t[trained.mids[i]], mode)
+            cur.wait_event(ev_mid[i])
+            cms[i].record_stream(cur)
+            a = inject(i, a, cms[i])
+        cur.wait_stream(side)
+        cur.wait_stream(skip)
+        cur.wait_stream(aux)
+        for tns in cats:
+            tns.record_stream(cur)
 
     for u in trained.ups:
         a = E.run_up(u, a, None, plan_t[u], mode, cat=cats.pop())

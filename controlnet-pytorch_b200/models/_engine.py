@@ -91,12 +91,9 @@ def conv16(x, param, kind, cout, mode, *, packed=None, packed_lp=None, out_f16=N
 ATTN_F16_DIMS = (4, 8, 16, 24, 32, 48, 64, 96, 128, 192)     # head dims attention_f16.cu instantiates
 
 
-_FUSE_RES = _os.environ.get("CNB_FUSE_RES", "1") != "0"
-
-
 def fuse_residual(mode, x, h, cout):
     """K-concatenation needs both operands fp16 and TMA-friendly channel counts."""
-    if not (_FUSE_RES and act16(mode) and x.dtype == torch.float16 and h.dtype == torch.float16):
+    if not (act16(mode) and x.dtype == torch.float16 and h.dtype == torch.float16):
         return False
     return h.shape[3] % 16 == 0 and x.shape[3] % 8 == 0 and cout % 16 == 0
 
@@ -298,16 +295,11 @@ def run_mid(block, x, temb, mode):
 # parallel graph branches (only under CUDA-graph capture: in eager mode the stream bookkeeping is host time)
 # ----------------------------------------------------------------------------------------------------------
 _SIDE = {}
-_FORCE_PAR = [None]      # sampler override: True / False / None (= environment default, CNB_BRANCH_PARALLEL)
 
 
 def capture_parallel():
-    """'0' (no forks), '1' (default: the four-stream ControlNet layout) or '2' (round-1 layout: only the two-encoder
-    fork) while the current stream is capturing; '0' otherwise."""
-    env = _os.environ.get("CNB_BRANCH_PARALLEL", "1")
-    if _FORCE_PAR[0] is not None:
-        env = env if (_FORCE_PAR[0] and env != "0") else ("1" if _FORCE_PAR[0] else "0")
-    return env if (env != "0" and torch.cuda.is_current_stream_capturing()) else "0"
+    """True while the current stream is capturing: the ControlNet forward then forks into its four-stream layout."""
+    return torch.cuda.is_current_stream_capturing()
 
 
 def side_stream(dev, which=0):
@@ -397,9 +389,6 @@ def unet_time(unet, t, device):
     return t_proj_mlp(unet.t_proj, sinusoid(t, unet.t_emb_dim, device))
 
 
-_WIDE_IN = _os.environ.get("CNB_CONV_IN_TC", "1") != "0"
-
-
 def pad16_f16(x_nhwc):
     """fp32 (B, H, W, C <= 8) -> fp16 (B, H, W, 16) zero-padded copy, memoised on the tensor object (the frozen and the
     control conv_in read the same x)."""
@@ -419,7 +408,7 @@ def conv3x3_narrow_in(conv, x_nhwc, mode, residual=None):
     channels zero-padded to 16 in fp16: 9 k FMAs per pixel on the FFMA pipe were 0.3 ms per launch at B = 256 (4 -> 256
     @32x32).  Narrow outputs (MNIST 1 -> 32) keep the exact direct kernel."""
     cin, cout = conv.in_channels, conv.out_channels
-    if (_WIDE_IN and mode != rt.MODE_F32 and _F16_ENABLED and cin <= 8 and cout >= 64 and cout % 16 == 0 and
+    if (mode != rt.MODE_F32 and _F16_ENABLED and cin <= 8 and cout >= 64 and cout % 16 == 0 and
             x_nhwc.dtype == torch.float32 and (residual is None or residual.dtype == torch.float16)):
         def build():
             w = torch.zeros((cout, 16) + tuple(conv.weight.shape[2:]), device=conv.weight.device, dtype=torch.float32)
@@ -442,7 +431,7 @@ def prewarm_conv_in(unet, x_nhwc, mode):
     and whichever branch created it first would otherwise hand it to the other stream without an ordering edge."""
     conv = unet.conv_in
     cin, cout = conv.in_channels, conv.out_channels
-    if (_WIDE_IN and mode != rt.MODE_F32 and _F16_ENABLED and cin <= 8 and cout >= 64 and cout % 16 == 0 and
+    if (mode != rt.MODE_F32 and _F16_ENABLED and cin <= 8 and cout >= 64 and cout % 16 == 0 and
             x_nhwc.dtype == torch.float32):
         pad16_f16(x_nhwc)
 
@@ -509,8 +498,8 @@ def hint_stack_ddpm(seq, hint_nhwc, mode):
 
 class HintCache:
     """hint_block(hint) depends on neither t nor x (controlnet.py:179): compute once per (hint storage, weights).
-    A few entries are kept (the split sampler runs batch halves of one hint tensor on parallel streams); every entry
-    holds a reference to its hint tensor, so the storage cannot be recycled under the cached key.
+    A few entries are kept; every entry holds a reference to its hint tensor, so the storage cannot be recycled under
+    the cached key.
 
     An entry is keyed by the hint's STORAGE (data_ptr, shape, strides), the mode and the hint-block weights; the hint's
     version counter is a stamp inside the entry.  When the same storage is overwritten in place (the way a captured

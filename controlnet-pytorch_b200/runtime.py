@@ -168,10 +168,7 @@ def mode_name(m=None):
 def attention_kernel_name(L=784, d=16):
     """Name of the kernel cnb_attention_f16 dispatches to for (sequence length L, head dim d): the measured routing rule of
     csrc/attention_tmem.cu::attention_tmem_default (bench.py's roofline label)."""
-    mode = os.environ.get("CNB_ATTN_TMEM", "1")
-    minl, mind = int(os.environ.get("CNB_ATTN_TMEM_MINL", "128")), int(os.environ.get("CNB_ATTN_TMEM_MIND", "24"))
-    tmem_ok = d in (4, 8, 16, 24, 32, 48, 64)
-    if tmem_ok and (mode == "2" or (mode != "0" and L >= minl and d >= mind)):
+    if d in (4, 8, 16, 24, 32, 48, 64) and L >= 128 and d >= 24:
         return "attention_tmem_kernel (tcgen05.mma SS + TS, S/P/O in TMEM, TMA)"
     return "attention_f16_kernel (mma.sync m16n8k16)"
 

@@ -8,7 +8,6 @@ tools/sample_ldm_controlnet.py:45-50 with the per-step host work removed.
   * data parallel: each rank owns a contiguous slice of the batch, no collective inside the loop, one all_gather of
     the final samples (NCCL over NVLink) at the end.
 """
-import os
 
 import torch
 
@@ -52,18 +51,13 @@ class DDPMSampler:
         and the graph (which baked the packed-weight caches derived from the old values) is rebuilt."""
         return tuple((p._version, p.data_ptr()) for p in self.model.parameters())
 
-    def _hint_parts(self):
-        return [self._hint[lo:hi] for lo, hi in self._bounds]
-
     def _refresh_hint(self):
         """The captured step reads the hint FEATURE tensors the warm-up cached (models/_engine.HintCache); after the
         static hint buffer has been overwritten they are recomputed in place, outside the graph, once per call."""
         fn = getattr(self.model, "_hint_feat", None)
         if fn is None:
             return
-        mode = rt.get_mode()
-        for part in self._hint_parts():
-            fn(part, mode)
+        fn(self._hint, rt.get_mode())
 
     def _capture(self, x_T, hint, steps, elem_offset):
         dev = x_T.device
@@ -80,64 +74,26 @@ class DDPMSampler:
         table = sch.coef_table(dev)
         L = rt.lib()
 
-        # Batch halves on parallel capture streams: every kernel is batch-invariant (DESIGN.md section 5), so the result
-        # is bit-identical to the unsplit step, while the GPU overlaps the MUFU-bound attention of one half with the
-        # tensor- / HBM-bound convolutions and GroupNorms of the other (measured at B = 1024: 13.08 -> 12.65 ms).
-        B = self.xt.shape[0]
-        per = self.xt[0].numel()
-        # Default: off.  The ControlNet forward's own fork of its branches (models/_controlnet_common.py) gives the overlap
-        # without halving the per-kernel batch: MNIST B = 1024 12.59 split vs 12.61 two branches vs 11.84 ms with the
-        # four-stream layout; CelebHQ (190 M parameters) B = 256: 31.2 unsplit, 31.1 two branches, 28.25 split, 27.79 ms
-        # four streams (gpu_jobs/r2_34_cfg3.sh).  CNB_SAMPLER_SPLIT=2 keeps the split available.  Never both.
-        nsplit = int(os.environ.get("CNB_SAMPLER_SPLIT", "1"))
-        nsplit = max(1, min(nsplit, B))
-        bounds = [shard_bounds(B, nsplit, k) for k in range(nsplit)]
-        self._bounds = bounds
-        self._split_streams = [torch.cuda.Stream(device=dev) for _ in range(nsplit)] if nsplit > 1 else []
-
-        def part(lo, hi):
-            xs = self.xt[lo:hi]
-            eps = self.model(xs, self.t_out, hint[lo:hi])
-            ops.sched_step(xs, eps, self.coef, z=None, seed=self.seed, step_dev=self.step_idx,
-                           elem_offset=elem_offset + lo * per, out=xs, x0_out=self.x0[lo:hi])
-
         def one_step():
             rt.check(L.cnb_sampler_prologue(self.step_idx.data_ptr(), self.t_seq.data_ptr(), self.t_out.data_ptr(),
                                             table.data_ptr(), self.coef.data_ptr(), rt.stream()))
-            if nsplit == 1:
-                part(0, B)
-            else:
-                cur = torch.cuda.current_stream()
-                for st, (lo, hi) in zip(self._split_streams, bounds):
-                    st.wait_stream(cur)
-                    with torch.cuda.stream(st):
-                        part(lo, hi)
-                for st in self._split_streams:
-                    cur.wait_stream(st)
+            eps = self.model(self.xt, self.t_out, hint)
+            ops.sched_step(self.xt, eps, self.coef, z=None, seed=self.seed, step_dev=self.step_idx,
+                           elem_offset=elem_offset, out=self.xt, x0_out=self.x0)
             rt.check(L.cnb_bump_index(self.step_idx.data_ptr(), 1, rt.stream()))
 
-        from .models import _controlnet_common as _cc
-        _cc.set_branch_parallel(False if (nsplit > 1 and os.environ.get("CNB_SPLIT_KEEP_BRANCH", "0") != "1") else None)
-        try:
-            if nsplit > 1:
-                # cold caches: ONE unsplit forward on a single stream packs every weight / builds the t-embedding table
-                # before the parts (which only read those caches) run concurrently on the split streams
-                self.model(self.xt, self.t_seq[:1], hint)
-                torch.cuda.synchronize(dev)
-            # warm-up on a side stream: builds weight / hint caches and sets kernel attributes outside the capture
-            s = torch.cuda.Stream(device=dev)
-            s.wait_stream(torch.cuda.current_stream())
-            with torch.cuda.stream(s):
-                one_step()
-            torch.cuda.current_stream().wait_stream(s)
-            torch.cuda.synchronize(dev)
-            c0 = rt.launch_count()
-            g = torch.cuda.CUDAGraph()
-            with torch.cuda.graph(g):
-                one_step()
-            self.launches_per_step = rt.launch_count() - c0
-        finally:
-            _cc.set_branch_parallel(None)
+        # warm-up on a side stream: builds weight / hint caches and sets kernel attributes outside the capture
+        s = torch.cuda.Stream(device=dev)
+        s.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(s):
+            one_step()
+        torch.cuda.current_stream().wait_stream(s)
+        torch.cuda.synchronize(dev)
+        c0 = rt.launch_count()
+        g = torch.cuda.CUDAGraph()
+        with torch.cuda.graph(g):
+            one_step()
+        self.launches_per_step = rt.launch_count() - c0
         self._graph = g
         self._nsteps, self._pos = steps, 0
         # keep every tensor the graph reads alive for as long as the graph: the hint features (HintCache may evict)

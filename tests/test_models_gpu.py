@@ -375,38 +375,12 @@ def test_graphed_students_match_eager(rt):
     assert rt.lib().cnb_tc_error_flag() == 0
 
 
-def test_split_stream_sampler_is_bit_identical(rt, monkeypatch):
-    """The graph-replayed step run as two (or three, ragged) batch parts on parallel capture streams must equal the
-    unsplit graph and the eager loop bit for bit (batch-invariant kernels, Philox keyed by global element index)."""
-    rt.set_mode("f16" if rt.lib().cnb_has_tcgen05() else "fp32")
-    cfg = syn.MNIST_PARAMS
-    m = _fill(_mod("models.controlnet").ControlNet(cfg))
-    sched = _mod("scheduler.linear_noise_scheduler").LinearNoiseScheduler(**syn.MNIST_DIFFUSION)
-    S = _mod("sampler")
-    B, steps = 70, 4
-    x, hint = inputs("split", B, 1, 28)
-    xc, hc = x.cuda(), hint.cuda()
-    outs = {}
-    for split in ("1", "2", "3"):
-        monkeypatch.setenv("CNB_SAMPLER_SPLIT", split)
-        smp = S.DDPMSampler(m, sched, seed=9, use_graph=True)
-        outs[split] = smp.sample(xc, hc, steps=steps, elem_offset=1000)
-        if split != "1":
-            assert smp.launches_per_step > 1.8 * base_launches
-        else:
-            base_launches = smp.launches_per_step
-    eager = S.DDPMSampler(m, sched, seed=9, use_graph=False).sample(xc, hc, steps=steps, elem_offset=1000)
-    for split in ("1", "2", "3"):
-        assert torch.equal(outs[split][0], eager[0]) and torch.equal(outs[split][1], eager[1]), split
-    assert rt.lib().cnb_tc_error_flag() == 0
-
-
-def test_branch_layouts_of_the_step_graph_are_bit_identical(rt, monkeypatch):
+def test_branch_layouts_of_the_step_graph_are_bit_identical(rt):
     """models/_controlnet_common.py lays the ControlNet forward out on four capture streams (trained mids ahead of the
-    control join, skip sums and t-embedding rows off the critical path).  Every layout - sequential (0), four streams
-    (1, default), the round-1 two-stream fork (2) - runs the same kernels on the same inputs, so the replayed samples
-    must equal the eager loop bit for bit: MNIST DDPM ControlNet, the tiny LDM ControlNet (image-pyramid hints), and a
-    CIFAR-width ControlNet whose conv_in layers share the padded fp16 copy of x (built before the fork)."""
+    control join, skip sums and t-embedding rows off the critical path); the eager loop runs it on one stream.  Both
+    run the same kernels on the same inputs, so the replayed samples must equal the eager loop bit for bit: MNIST DDPM
+    ControlNet, the tiny LDM ControlNet (image-pyramid hints), and a CIFAR-width ControlNet whose conv_in layers share
+    the padded fp16 copy of x (built before the fork)."""
     rt.set_mode("f16" if rt.lib().cnb_has_tcgen05() else "fp32")
     S = _mod("sampler")
     L = _mod("scheduler.linear_noise_scheduler").LinearNoiseScheduler
@@ -421,11 +395,9 @@ def test_branch_layouts_of_the_step_graph_are_bit_identical(rt, monkeypatch):
     for name, m, sched, (x, hint) in cases:
         xc, hc = x.cuda(), hint.cuda()
         eager = S.DDPMSampler(m, sched, seed=11, use_graph=False).sample(xc, hc, steps=3, elem_offset=64)
-        for layout in ("0", "1", "2"):
-            monkeypatch.setenv("CNB_BRANCH_PARALLEL", layout)
-            got = S.DDPMSampler(m, sched, seed=11, use_graph=True).sample(xc, hc, steps=3, elem_offset=64)
-            assert torch.equal(got[0], eager[0]) and torch.equal(got[1], eager[1]), (name, layout)
-            assert torch.isfinite(got[0]).all()
+        got = S.DDPMSampler(m, sched, seed=11, use_graph=True).sample(xc, hc, steps=3, elem_offset=64)
+        assert torch.equal(got[0], eager[0]) and torch.equal(got[1], eager[1]), name
+        assert torch.isfinite(got[0]).all()
     assert rt.lib().cnb_tc_error_flag() == 0
 
 
@@ -472,21 +444,20 @@ def test_sampler_graph_follows_hint_and_weight_updates(rt):
     assert torch.equal(d, e.sample(xT, hint2, steps=4)[0]) and not torch.equal(c, d)
 
 
-def test_cold_cache_split_stream_sampler(rt, monkeypatch):
-    """ADVICE r1: with batch parts on parallel capture streams the FIRST warm-up runs on cold weight caches; the parts
-    must not read packed weights another stream is still building.  A fresh model goes straight into the split path."""
+def test_cold_cache_graph_sampler(rt):
+    """ADVICE r1: the graph sampler's FIRST warm-up runs on cold weight caches, and the captured four-stream step must
+    not read packed weights that were still being built.  A fresh model goes straight into the graph sampler and must
+    equal the eager loop on a warm copy."""
     cfg = syn.TINY_PARAMS
     sched = _mod("scheduler.linear_noise_scheduler").LinearNoiseScheduler(**syn.MNIST_DIFFUSION)
     S = _mod("sampler")
     rt.set_mode("f16" if rt.lib().cnb_has_tcgen05() else "fp32")
     B = 8
     hint = syn.det_hint(B, 16).cuda()
-    monkeypatch.setenv("CNB_SAMPLER_SPLIT", "2")
     cold = _fill(_mod("models.controlnet").ControlNet(cfg))            # no forward has run on this module yet
     g = S.DDPMSampler(cold, sched, seed=2, use_graph=True)
     xT = g.draw_xT((B, 1, 16, 16), "cuda")
     a, _ = g.sample(xT, hint, steps=3)
-    monkeypatch.setenv("CNB_SAMPLER_SPLIT", "1")
     warm = _fill(_mod("models.controlnet").ControlNet(cfg))
     b, _ = S.DDPMSampler(warm, sched, seed=2, use_graph=False).sample(xT, hint, steps=3)
     assert torch.equal(a, b)
