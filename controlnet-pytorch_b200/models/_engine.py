@@ -33,9 +33,11 @@ def zero_(module):
 # ----------------------------------------------------------------------------------------------------------
 # derived weight cache
 # ----------------------------------------------------------------------------------------------------------
-def _cached(param, key, builder):
-    store = param.__dict__.setdefault("_cnb_pack", {})
-    stamp = (param._version, param.data_ptr())
+def _cached(params, key, builder):
+    """builder()'s result, kept on params[0] under `key` and rebuilt when any of `params` is changed in place (version
+    counter) or replaced (data_ptr)."""
+    store = params[0].__dict__.setdefault("_cnb_pack", {})
+    stamp = tuple((p._version, p.data_ptr()) for p in params)
     ent = store.get(key)
     if ent is None or ent[0] != stamp:
         with torch.no_grad():
@@ -51,31 +53,28 @@ def _tc_shape(o, i):
 
 def packed_conv(param, mode):
     r = mode != rt.MODE_F32 and _tc_shape(param.shape[0], param.shape[1])
-    return _cached(param, ("conv", r), lambda: ops.pack_conv_weight(param, r))
+    return _cached((param,), ("conv", r), lambda: ops.pack_conv_weight(param, r))
 
 
-def packed_conv_f16(param, mode):
+def packed_conv_f16(param):
     """fp16 copy of the packed (unrounded) weights: B operand of the kind::f16 convolution."""
-    return _cached(param, ("conv_f16",), lambda: ops.cast_f16(ops.pack_conv_weight(param, False)))
+    return _cached((param,), ("conv_f16",), lambda: ops.cast_f16(ops.pack_conv_weight(param, False)))
 
 
 def use_f16(mode, cin, cout):
     """GroupNorm -> conv pairs run with fp16 operands in the tensor-core mode (same 10-bit mantissa as tf32, half the
-    bytes, twice the MMA rate) when the layer is tensor-core eligible.  CNB_F16=0 keeps everything tf32."""
-    return mode != rt.MODE_F32 and _F16_ENABLED and cin % 8 == 0 and cout % 16 == 0
+    bytes, twice the MMA rate) when the layer is tensor-core eligible."""
+    return mode != rt.MODE_F32 and cin % 8 == 0 and cout % 16 == 0
 
 
-import os as _os
-_F16_ENABLED = _os.environ.get("CNB_F16", "1") != "0"
-ATTN_F16 = _os.environ.get("CNB_ATTN_F16", "1") != "0"
-_ACT16_ENABLED = _os.environ.get("CNB_ACT16", "1") != "0"
+_F16_ENABLED = True      # the tensor-core mode computes with fp16 operands; bench.py reads this to label its dtype
 
 
 def act16(mode):
     """Tensor-core modes keep the whole activation stream (block inputs / outputs, skips, concat buffers) in fp16:
     half the bytes of every HBM-bound kernel, every convolution runs kind::f16.  Statistics, accumulators, biases,
-    time-embedding rows and the softmax stay fp32.  CNB_ACT16=0 keeps the fp32 residual stream."""
-    return mode != rt.MODE_F32 and _F16_ENABLED and _ACT16_ENABLED
+    time-embedding rows and the softmax stay fp32."""
+    return mode != rt.MODE_F32
 
 
 def conv16(x, param, kind, cout, mode, *, packed=None, packed_lp=None, out_f16=None, **kw):
@@ -84,7 +83,7 @@ def conv16(x, param, kind, cout, mode, *, packed=None, packed_lp=None, out_f16=N
     w = packed_conv(param, mode) if packed is None else packed
     lp = None
     if x.dtype == torch.float16:
-        lp = packed_conv_f16(param, mode) if packed_lp is None else packed_lp
+        lp = packed_conv_f16(param) if packed_lp is None else packed_lp
     if out_f16 is None:
         out_f16 = act16(mode) and cout % 16 == 0
     return ops.conv(x, w, kind, cout, mode=mode, weight_lp=lp, out_f16=out_f16, **kw)
@@ -105,18 +104,11 @@ def packed_cat_f16(param3x3, param1x1):
         b = ops.pack_conv_weight(param1x1, False)
         o = a.shape[0]
         return ops.cast_f16(torch.cat([a.reshape(o, -1), b.reshape(o, -1)], dim=1).contiguous())
-    store = param3x3.__dict__.setdefault("_cnb_pack", {})
-    stamp = (param3x3._version, param3x3.data_ptr(), param1x1._version, param1x1.data_ptr())
-    ent = store.get(("cat_f16",))
-    if ent is None or ent[0] != stamp:
-        with torch.no_grad():
-            ent = (stamp, build())
-        store[("cat_f16",)] = ent
-    return ent[1]
+    return _cached((param3x3, param1x1), ("cat_f16",), build)
 
 
-def packed_convT_f16(param, mode):
-    return _cached(param, ("convT_f16",), lambda: ops.cast_f16(ops.pack_convT_weight(param, False)))
+def packed_convT_f16(param):
+    return _cached((param,), ("convT_f16",), lambda: ops.cast_f16(ops.pack_convT_weight(param, False)))
 
 
 def cast_like(x, ref):
@@ -130,7 +122,7 @@ def cast_like(x, ref):
 
 def packed_convT(param, mode):
     r = mode != rt.MODE_F32 and _tc_shape(param.shape[1], param.shape[0])
-    return _cached(param, ("convT", r), lambda: ops.pack_convT_weight(param, r))
+    return _cached((param,), ("convT", r), lambda: ops.pack_convT_weight(param, r))
 
 
 def raw(param):
@@ -263,7 +255,7 @@ class ResAttnStack(nn.Module):
         h16 = use_f16(mode, E, 3 * E)
         a = ops.groupnorm(x, raw(norm.weight), raw(norm.bias), self._groups, silu=False, out_f16=h16)
         # tensor-core modes: q|k|v and the attention output stay fp16 between the three kernels
-        f16_core = h16 and ATTN_F16 and (E // att.num_heads) in ATTN_F16_DIMS
+        f16_core = h16 and (E // att.num_heads) in ATTN_F16_DIMS
         qkv = conv16(a, att.in_proj_weight, "1x1", 3 * E, mode, bias=raw(att.in_proj_bias), out_f16=f16_core)
         o = ops.attention(qkv, att.num_heads, mode=mode)
         return conv16(o, att.out_proj.weight, "1x1", E, mode, bias=raw(att.out_proj.bias), residual=x)
@@ -291,24 +283,6 @@ def run_mid(block, x, temb, mode):
     return x
 
 
-# ----------------------------------------------------------------------------------------------------------
-# parallel graph branches (only under CUDA-graph capture: in eager mode the stream bookkeeping is host time)
-# ----------------------------------------------------------------------------------------------------------
-_SIDE = {}
-
-
-def capture_parallel():
-    """True while the current stream is capturing: the ControlNet forward then forks into its four-stream layout."""
-    return torch.cuda.is_current_stream_capturing()
-
-
-def side_stream(dev, which=0):
-    key = (str(dev), torch.cuda.current_stream(dev).cuda_stream, which)
-    if key not in _SIDE:
-        _SIDE[key] = torch.cuda.Stream(device=dev)
-    return _SIDE[key]
-
-
 def run_up(block, x, skip, temb, mode, cat=None):
     """ConvTranspose (4 parity phases) or identity into the first half of the concat buffer, skip in the second
     half (unet_base.py:267-269).  `cat` may arrive with its second half already written by the producer of the
@@ -329,7 +303,7 @@ def run_up(block, x, skip, temb, mode, cat=None):
             ops.copy_channels(cast_like(skip, cat), cat, d_coff=cu)
     if block.up_sample:
         wp = packed_convT(up.weight, mode)
-        wl = packed_convT_f16(up.weight, mode) if x.dtype == torch.float16 else None
+        wl = packed_convT_f16(up.weight) if x.dtype == torch.float16 else None
         for ph in range(4):
             ops.conv(x, wp[ph], None, cu, bias=raw(up.bias), out=cat, out_coff=0, mode=mode, phase=(ph >> 1, ph & 1),
                      weight_lp=None if wl is None else wl[ph])
@@ -357,23 +331,14 @@ def temb_plan(unet, temb_vec, with_ups=True):
     """One launch for all t_emb_layers of a U-Net: rows = SiLU(temb) @ Wcat^T + bcat, Wcat = concat over blocks.
     Returns {block: Temb}."""
     blocks = unet_blocks(unet, with_ups)
-    key_params = [seq[1].weight for b in blocks for seq in b.t_emb_layers]
-    holder = key_params[0]
+    lins = [seq[1] for b in blocks for seq in b.t_emb_layers]
 
     def build():
-        w = torch.cat([raw(seq[1].weight) for b in blocks for seq in b.t_emb_layers], dim=0).contiguous()
-        bias = torch.cat([raw(seq[1].bias) for b in blocks for seq in b.t_emb_layers], dim=0).contiguous()
+        w = torch.cat([raw(lin.weight) for lin in lins], dim=0).contiguous()
+        bias = torch.cat([raw(lin.bias) for lin in lins], dim=0).contiguous()
         return w, bias
 
-    store = holder.__dict__.setdefault("_cnb_pack", {})
-    stamp = tuple((p._version, p.data_ptr()) for p in key_params) + tuple(
-        (seq[1].bias._version, seq[1].bias.data_ptr()) for b in blocks for seq in b.t_emb_layers)
-    ent = store.get(("tcat", with_ups))
-    if ent is None or ent[0] != stamp:
-        with torch.no_grad():
-            ent = (stamp, build())
-        store[("tcat", with_ups)] = ent
-    wcat, bcat = ent[1]
+    wcat, bcat = _cached([lin.weight for lin in lins] + [lin.bias for lin in lins], ("tcat", with_ups), build)
     table = ops.linear_small(temb_vec, wcat, bcat, silu_in=True)
     plan, off = {}, 0
     for b in blocks:
@@ -402,20 +367,26 @@ def pad16_f16(x_nhwc):
     return buf
 
 
+def narrow_in_tc(conv, x_nhwc, mode, residual=None):
+    """True when conv3x3_narrow_in runs `conv` on the tensor core from the zero-padded fp16 copy of x."""
+    cin, cout = conv.in_channels, conv.out_channels
+    return (mode != rt.MODE_F32 and cin <= 8 and cout >= 64 and cout % 16 == 0 and x_nhwc.dtype == torch.float32 and
+            (residual is None or residual.dtype == torch.float16))
+
+
 def conv3x3_narrow_in(conv, x_nhwc, mode, residual=None):
     """3x3 conv from a handful of input channels (conv_in of the U-Nets, VAE decoder_conv_in / encoder_conv_in).
     Wide outputs (>= 64 channels: CelebHQ 4 -> 256, VAE 4 -> 384, CIFAR 3 -> 64) run on the tensor core with the input
     channels zero-padded to 16 in fp16: 9 k FMAs per pixel on the FFMA pipe were 0.3 ms per launch at B = 256 (4 -> 256
     @32x32).  Narrow outputs (MNIST 1 -> 32) keep the exact direct kernel."""
     cin, cout = conv.in_channels, conv.out_channels
-    if (mode != rt.MODE_F32 and _F16_ENABLED and cin <= 8 and cout >= 64 and cout % 16 == 0 and
-            x_nhwc.dtype == torch.float32 and (residual is None or residual.dtype == torch.float16)):
+    if narrow_in_tc(conv, x_nhwc, mode, residual):
         def build():
             w = torch.zeros((cout, 16) + tuple(conv.weight.shape[2:]), device=conv.weight.device, dtype=torch.float32)
             w[:, :cin] = conv.weight.detach()
             packed = ops.pack_conv_weight(w, False)
             return packed, ops.cast_f16(packed)
-        packed, packed16 = _cached(conv.weight, ("cin_pad16",), build)
+        packed, packed16 = _cached((conv.weight,), ("cin_pad16",), build)
         return ops.conv(pad16_f16(x_nhwc), packed, "3x3", cout, bias=raw(conv.bias), mode=mode, weight_lp=packed16,
                         out_f16=True, residual=residual)
     return conv16(x_nhwc, conv.weight, "3x3", cout, mode, bias=raw(conv.bias), residual=residual)
@@ -426,13 +397,11 @@ def conv_in(unet, x_nhwc, mode, residual=None):
 
 
 def prewarm_conv_in(unet, x_nhwc, mode):
-    """Build the memoised padded fp16 copy of x (pad16_f16) on the CURRENT stream when conv_in will take the tensor-core
-    route.  The ControlNet forward calls this before it forks its branches: both conv_in layers read that one buffer,
-    and whichever branch created it first would otherwise hand it to the other stream without an ordering edge."""
-    conv = unet.conv_in
-    cin, cout = conv.in_channels, conv.out_channels
-    if (mode != rt.MODE_F32 and _F16_ENABLED and cin <= 8 and cout >= 64 and cout % 16 == 0 and
-            x_nhwc.dtype == torch.float32):
+    """Under CUDA-graph capture, build the memoised padded fp16 copy of x (pad16_f16) on the CURRENT stream when conv_in
+    will take the tensor-core route.  The ControlNet forward calls this before it forks its branches: both conv_in
+    layers read that one buffer, and whichever branch created it first would otherwise hand it to the other stream
+    without an ordering edge.  Outside capture both run on one stream and the first of them builds it."""
+    if torch.cuda.is_current_stream_capturing() and narrow_in_tc(unet.conv_in, x_nhwc, mode):
         pad16_f16(x_nhwc)
 
 
@@ -443,7 +412,7 @@ def gn_silu_conv_tail(norm, conv, h, mode):
     (CelebHQ U-Net 128 -> 4, VAE decoder 128 -> 3 at 128x128: 3.5 k MACs per pixel) run on the tensor core with Cout
     zero-padded to 16: 4-5x wasted MMA work is still ~10x faster than FFMA."""
     cout, cin = conv.out_channels, conv.in_channels
-    lowp = mode != rt.MODE_F32 and _F16_ENABLED and cout <= 4
+    lowp = mode != rt.MODE_F32 and cout <= 4
     tc = lowp and cin % 16 == 0 and cin >= 64
     h16 = lowp and cin % 4 == 0
     h = ops.groupnorm(h, raw(norm.weight), raw(norm.bias), norm.num_groups, silu=True, out_f16=h16)
@@ -457,14 +426,7 @@ def gn_silu_conv_tail(norm, conv, h, mode):
         b[:cout] = conv.bias.detach()
         packed = ops.pack_conv_weight(w, False)
         return packed, ops.cast_f16(packed), b
-    store = conv.weight.__dict__.setdefault("_cnb_pack", {})
-    stamp = (conv.weight._version, conv.weight.data_ptr(), conv.bias._version, conv.bias.data_ptr())
-    ent = store.get(("pad16",))
-    if ent is None or ent[0] != stamp:
-        with torch.no_grad():
-            ent = (stamp, build())
-        store[("pad16",)] = ent
-    packed, packed16, bias = ent[1]
+    packed, packed16, bias = _cached((conv.weight, conv.bias), ("pad16",), build)
     return ops.conv(h, packed, "3x3", 16, bias=bias, mode=mode, weight_lp=packed16, out_f16=True)[..., :cout]
 
 

@@ -444,6 +444,45 @@ def test_sampler_graph_follows_hint_and_weight_updates(rt):
     assert torch.equal(d, e.sample(xT, hint2, steps=4)[0]) and not torch.equal(c, d)
 
 
+@pytest.mark.parametrize("cache", ["cat_f16", "tcat", "pad16"])
+def test_graph_sampler_follows_the_second_parameter_of_a_cached_weight(rt, cache):
+    """Three derived weights are kept on one parameter but built from several: the second 3x3 fused with the residual
+    1x1 (`cat_f16`), the concatenated t-embedding rows (`tcat`) and conv_out padded to 16 outputs (`pad16`, taken when
+    conv_out reads >= 64 channels, hence the wider LDM).  Changing only the secondary parameter (the 1x1 weight, one
+    t-embedding bias, conv_out's bias) in place after capture must rebuild that cache: the re-captured step equals an
+    eager step on a fresh copy of the changed model."""
+    if not rt.lib().cnb_has_tcgen05():
+        pytest.skip("these caches serve the tensor-core mode")
+    rt.set_mode("f16")
+    S = _mod("sampler")
+    L = _mod("scheduler.linear_noise_scheduler").LinearNoiseScheduler
+    if cache == "pad16":
+        make = lambda: _mod("models.controlnet_ldm").ControlNet(4, dict(syn.TINY_LDM_PARAMS, conv_out_channels=64),
+                                                                down_sample_factor=8)
+        sched, (x, hint) = L(ldm_scheduler=True, **syn.CELEBHQ_DIFFUSION), inputs("cache_ldm", 2, 4, 8, hint_size=64)
+    else:
+        make = lambda: _mod("models.controlnet").ControlNet(syn.TINY_PARAMS)
+        sched, (x, hint) = L(**syn.MNIST_DIFFUSION), inputs("cache_tiny", 2, 1, 16)
+    m = _fill(make())
+    tu = m.trained_unet
+    holder, key, prm = {
+        "cat_f16": (tu.downs[0].resnet_conv_second[0][2].weight, ("cat_f16",), tu.downs[0].residual_input_conv[0].weight),
+        "tcat": (tu.downs[0].t_emb_layers[0][1].weight, ("tcat", True), tu.mids[0].t_emb_layers[0][1].bias),
+        "pad16": (tu.conv_out.weight, ("pad16",), tu.conv_out.bias)}[cache]
+    xc, hc = x.cuda(), hint.cuda()
+    g = S.DDPMSampler(m, sched, seed=11, use_graph=True)
+    before = g.sample(xc, hc, steps=2)
+    assert key in holder._cnb_pack                                      # the step took the cached route
+    with torch.no_grad():
+        prm.add_(0.25)
+    got = g.sample(xc, hc, steps=2)
+    fresh = _fill(make())
+    fresh.load_state_dict(m.state_dict())
+    want = S.DDPMSampler(fresh, sched, seed=11, use_graph=False).sample(xc, hc, steps=2)
+    assert torch.equal(got[0], want[0]) and torch.equal(got[1], want[1])
+    assert not torch.equal(got[0], before[0])
+
+
 def test_cold_cache_graph_sampler(rt):
     """ADVICE r1: the graph sampler's FIRST warm-up runs on cold weight caches, and the captured four-stream step must
     not read packed weights that were still being built.  A fresh model goes straight into the graph sampler and must
