@@ -1,5 +1,5 @@
 // Small / memory-bound kernels of the path: time embedding, t-embedding MLP rows, scheduler step (bit-exact fp32
-// restatement of scheduler/linear_noise_scheduler.py:58-77 with optional fused Philox noise), EDM scalings,
+// restatement of scheduler/linear_noise_scheduler.py:58-77 with optional fused Philox noise), DDIM step, EDM scalings,
 // NCHW <-> channels-last plumbing and one-time weight packers.
 #include <cuda_fp16.h>
 
@@ -106,6 +106,28 @@ __global__ void philox_normal_kernel(float* __restrict__ out, long long n, uint6
   }
 }
 
+// The noise of the fused scheduler updates: z[4i .. 4i+3] (or z[i]) when the caller supplies it, otherwise the Philox
+// normals of global elements elem_offset + 4i .. (or elem_offset + i), whatever the alignment of elem_offset.
+__device__ __forceinline__ float4 step_noise4(const float* __restrict__ z, long long i, uint64_t seed, uint64_t step,
+                                              uint64_t elem_offset, bool aligned4) {
+  if (z) return reinterpret_cast<const float4*>(z)[i];
+  if (aligned4) return philox_normal4(seed, step, (elem_offset >> 2) + (uint64_t)i);
+  const uint64_t g = elem_offset + 4ull * (uint64_t)i;
+  float4 zz;
+  zz.x = philox_pick(philox_normal4(seed, step, (g + 0) >> 2), (int)((g + 0) & 3));
+  zz.y = philox_pick(philox_normal4(seed, step, (g + 1) >> 2), (int)((g + 1) & 3));
+  zz.z = philox_pick(philox_normal4(seed, step, (g + 2) >> 2), (int)((g + 2) & 3));
+  zz.w = philox_pick(philox_normal4(seed, step, (g + 3) >> 2), (int)((g + 3) & 3));
+  return zz;
+}
+
+__device__ __forceinline__ float step_noise1(const float* __restrict__ z, long long i, uint64_t seed, uint64_t step,
+                                             uint64_t elem_offset) {
+  if (z) return z[i];
+  const uint64_t g = elem_offset + (uint64_t)i;
+  return philox_pick(philox_normal4(seed, step, g >> 2), (int)(g & 3));
+}
+
 // ------------------------------------------------------------------------------------------------
 // sample_prev_timestep: separate IEEE ops in the reference's order (the *_rn intrinsics are never contracted)
 // ------------------------------------------------------------------------------------------------
@@ -131,20 +153,7 @@ __global__ void sched_step_kernel(const float* __restrict__ xt, const float* __r
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
     float4 a = reinterpret_cast<const float4*>(xt)[i];
     float4 e = reinterpret_cast<const float4*>(eps)[i];
-    float4 zz = make_float4(0.f, 0.f, 0.f, 0.f);
-    if (noisy) {
-      if (z) {
-        zz = reinterpret_cast<const float4*>(z)[i];
-      } else if (aligned4) {
-        zz = philox_normal4(seed, step, (elem_offset >> 2) + (uint64_t)i);
-      } else {
-        uint64_t g = elem_offset + 4ull * (uint64_t)i;
-        zz.x = philox_pick(philox_normal4(seed, step, (g + 0) >> 2), (int)((g + 0) & 3));
-        zz.y = philox_pick(philox_normal4(seed, step, (g + 1) >> 2), (int)((g + 1) & 3));
-        zz.z = philox_pick(philox_normal4(seed, step, (g + 2) >> 2), (int)((g + 2) & 3));
-        zz.w = philox_pick(philox_normal4(seed, step, (g + 3) >> 2), (int)((g + 3) & 3));
-      }
-    }
+    const float4 zz = noisy ? step_noise4(z, i, seed, step, elem_offset, aligned4) : make_float4(0.f, 0.f, 0.f, 0.f);
     float4 p, o;
     sched_one(a.x, e.x, zz.x, s1, sq_acp, beta, sq_alpha, sigma, noisy, p.x, o.x);
     sched_one(a.y, e.y, zz.y, s1, sq_acp, beta, sq_alpha, sigma, noisy, p.y, o.y);
@@ -156,16 +165,55 @@ __global__ void sched_step_kernel(const float* __restrict__ xt, const float* __r
   // tail (n % 4 elements)
   if (blockIdx.x == 0 && threadIdx.x < (n & 3)) {
     long long i = (n4 << 2) + threadIdx.x;
-    float zv = 0.f;
-    if (noisy) {
-      if (z) zv = z[i];
-      else {
-        uint64_t g = elem_offset + (uint64_t)i;
-        zv = philox_pick(philox_normal4(seed, step, g >> 2), (int)(g & 3));
-      }
-    }
+    const float zv = noisy ? step_noise1(z, i, seed, step, elem_offset) : 0.f;
     float p, o;
     sched_one(xt[i], eps[i], zv, s1, sq_acp, beta, sq_alpha, sigma, noisy, p, o);
+    prev[i] = p;
+    if (x0) x0[i] = o;
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
+// DDIM update (scheduler/ddim_scheduler.py): x0 exactly as sched_one computes it, then
+// x_prev = c2 * x0' + c3 * eps (+ c4 * z), x0' = clamp(x0) with clip_sample, else x0; separate IEEE ops
+// ------------------------------------------------------------------------------------------------
+__device__ __forceinline__ void ddim_one(float xt, float e, float zv, const float c0, const float c1, const float c2,
+                                         const float c3, const float c4, const bool noisy, const bool clip,
+                                         float& prev, float& x0) {
+  const float v = __fdiv_rn(__fsub_rn(xt, __fmul_rn(c0, e)), c1);
+  x0 = fminf(fmaxf(v, -1.0f), 1.0f);
+  const float p = __fadd_rn(__fmul_rn(c2, clip ? x0 : v), __fmul_rn(c3, e));
+  prev = noisy ? __fadd_rn(p, __fmul_rn(c4, zv)) : p;
+}
+
+__global__ void ddim_step_kernel(const float* __restrict__ xt, const float* __restrict__ eps,
+                                 const float* __restrict__ z, float* __restrict__ prev, float* __restrict__ x0,
+                                 long long n, const float* __restrict__ coef, int clip_sample, uint64_t seed,
+                                 uint64_t step, const int32_t* __restrict__ step_dev, uint64_t elem_offset) {
+  if (step_dev) step = (uint64_t)step_dev[0];
+  const float c0 = coef[0], c1 = coef[1], c2 = coef[2], c3 = coef[3], c4 = coef[4];
+  const bool noisy = coef[5] != 0.0f, clip = clip_sample != 0;
+  const long long n4 = n >> 2;
+  const bool aligned4 = ((elem_offset & 3) == 0);
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
+    float4 a = reinterpret_cast<const float4*>(xt)[i];
+    float4 e = reinterpret_cast<const float4*>(eps)[i];
+    const float4 zz = noisy ? step_noise4(z, i, seed, step, elem_offset, aligned4) : make_float4(0.f, 0.f, 0.f, 0.f);
+    float4 p, o;
+    ddim_one(a.x, e.x, zz.x, c0, c1, c2, c3, c4, noisy, clip, p.x, o.x);
+    ddim_one(a.y, e.y, zz.y, c0, c1, c2, c3, c4, noisy, clip, p.y, o.y);
+    ddim_one(a.z, e.z, zz.z, c0, c1, c2, c3, c4, noisy, clip, p.z, o.z);
+    ddim_one(a.w, e.w, zz.w, c0, c1, c2, c3, c4, noisy, clip, p.w, o.w);
+    reinterpret_cast<float4*>(prev)[i] = p;
+    if (x0) reinterpret_cast<float4*>(x0)[i] = o;
+  }
+  // tail (n % 4 elements)
+  if (blockIdx.x == 0 && threadIdx.x < (n & 3)) {
+    long long i = (n4 << 2) + threadIdx.x;
+    const float zv = noisy ? step_noise1(z, i, seed, step, elem_offset) : 0.f;
+    float p, o;
+    ddim_one(xt[i], eps[i], zv, c0, c1, c2, c3, c4, noisy, clip, p, o);
     prev[i] = p;
     if (x0) x0[i] = o;
   }
@@ -395,6 +443,22 @@ extern "C" int cnb_sched_step(const float* xt, const float* eps, const float* z,
   if (blocks > 148 * 16) blocks = 148 * 16;
   sched_step_kernel<<<blocks, 256, 0, (cudaStream_t)s>>>(xt, eps, z, xt_prev, x0, n, coef, seed, step, step_dev,
                                                          elem_offset);
+  CNB_LAUNCH_CHECK();
+  return CNB_OK;
+}
+
+extern "C" int cnb_ddim_step(const float* xt, const float* eps, const float* z, float* xt_prev, float* x0, long long n,
+                             const float* coef, int clip_sample, uint64_t seed, uint64_t step, const int32_t* step_dev,
+                             uint64_t elem_offset, cnb_stream_t s) {
+  CNB_REQUIRE(n > 0 && xt && eps && xt_prev && coef, "ddim_step: null pointer or n=%lld", n);
+  CNB_REQUIRE((((uintptr_t)xt | (uintptr_t)eps | (uintptr_t)xt_prev | (uintptr_t)z | (uintptr_t)x0) & 15) == 0,
+              "ddim_step: pointers must be 16-byte aligned");
+  long long n4 = n >> 2;
+  unsigned blocks = (unsigned)((n4 + 255) / 256);
+  if (blocks < 1) blocks = 1;
+  if (blocks > 148 * 16) blocks = 148 * 16;
+  ddim_step_kernel<<<blocks, 256, 0, (cudaStream_t)s>>>(xt, eps, z, xt_prev, x0, n, coef, clip_sample, seed, step,
+                                                        step_dev, elem_offset);
   CNB_LAUNCH_CHECK();
   return CNB_OK;
 }

@@ -243,6 +243,18 @@ def sched_step(xt, eps, coef, z=None, want_x0=True, seed=0, step=0, step_dev=Non
     return prev, x0
 
 
+def ddim_step(xt, eps, coef, z=None, want_x0=True, clip_sample=False, seed=0, step=0, step_dev=None, elem_offset=0,
+              out=None, x0_out=None):
+    """One DDIM update (cnb_ddim_step); coef is a row of DDIMScheduler.coef_table.  Same conventions as sched_step."""
+    rt.require_cuda(xt, eps, coef, z, step_dev, out, x0_out)
+    prev = torch.empty_like(xt) if out is None else out
+    x0 = x0_out if x0_out is not None else (torch.empty_like(xt) if want_x0 else None)
+    rt.check(rt.lib().cnb_ddim_step(xt.data_ptr(), eps.data_ptr(), rt.ptr(z), prev.data_ptr(), rt.ptr(x0), xt.numel(),
+                                    coef.data_ptr(), 1 if clip_sample else 0, seed, step, rt.ptr(step_dev),
+                                    elem_offset, rt.stream()))
+    return prev, x0
+
+
 def philox_normal(shape, device, seed, step, elem_offset=0):
     out = torch.empty(shape, device=device, dtype=torch.float32)
     rt.require_cuda(out)

@@ -7,6 +7,11 @@ tools/sample_ldm_controlnet.py:45-50 with the per-step host work removed.
   * noise is Philox keyed by the GLOBAL element index, so the result is independent of how the batch is sharded;
   * data parallel: each rank owns a contiguous slice of the batch, no collective inside the loop, one all_gather of
     the final samples (NCCL over NVLink) at the end.
+
+The algorithm is the scheduler's: a LinearNoiseScheduler (DDPM, t = steps-1 .. 0) or a DDIMScheduler (a strided
+schedule) answers the same questions - `timesteps(steps)`, the [T, 6] `coef_table(device, steps)` the sampler prologue
+reads at row t, the fused `update` launch, and the `graph_key(steps)` of what a captured step depends on.  With
+steps=None the schedule is the scheduler's own (all T timesteps for DDPM, num_inference_steps for DDIM).
 """
 
 import torch
@@ -31,16 +36,17 @@ class DDPMSampler:
     @torch.no_grad()
     def sample_eager(self, x_T, hint, steps=None, zs=None, elem_offset=0, callback=None):
         sch = self.scheduler
-        steps = sch.num_timesteps if steps is None else steps
-        table = sch.coef_table(x_T.device)
+        ts = sch.timesteps(steps)
+        table = sch.coef_table(x_T.device, steps)
         xt, x0 = x_T.contiguous(), None
         t_dev = torch.empty((1,), device=x_T.device, dtype=torch.int64)
-        for k, t in enumerate(reversed(range(steps))):
+        for k, t in enumerate(ts):
             t_dev.fill_(t)
             eps = self.model(xt, t_dev, hint)
-            z = zs[k].to(xt.device) if (zs is not None and t > 0) else None
-            xt, x0 = ops.sched_step(xt, eps, table[t], z=z, want_x0=True, seed=self.seed, step=k,
-                                    elem_offset=elem_offset)
+            # the last step adds no noise in either scheduler, so zs may stop one short of the schedule
+            z = zs[k].to(xt.device) if (zs is not None and k < len(ts) - 1) else None
+            xt, x0 = sch.update(xt, eps, table[t], z=z, want_x0=True, seed=self.seed, step=k,
+                                elem_offset=elem_offset)
             if callback is not None:
                 callback(t, xt, x0)
         return xt, x0
@@ -67,19 +73,21 @@ class DDPMSampler:
         self._hint = hint.clone().contiguous()
         hint = self._hint
         self.x0 = torch.empty_like(self.xt)
-        self.t_seq = torch.arange(steps - 1, -1, -1, device=dev, dtype=torch.int64)
+        ts = sch.timesteps(steps)
+        self.t_seq = torch.tensor(ts, dtype=torch.int64).to(dev)
         self.step_idx = torch.zeros((1,), device=dev, dtype=torch.int32)
         self.t_out = torch.zeros((1,), device=dev, dtype=torch.int64)
         self.coef = torch.zeros((6,), device=dev, dtype=torch.float32)
-        table = sch.coef_table(dev)
+        table = sch.coef_table(dev, steps)
+        self._table = table          # the graph reads it: kept alive, so no other table can take its address
         L = rt.lib()
 
         def one_step():
             rt.check(L.cnb_sampler_prologue(self.step_idx.data_ptr(), self.t_seq.data_ptr(), self.t_out.data_ptr(),
                                             table.data_ptr(), self.coef.data_ptr(), rt.stream()))
             eps = self.model(self.xt, self.t_out, hint)
-            ops.sched_step(self.xt, eps, self.coef, z=None, seed=self.seed, step_dev=self.step_idx,
-                           elem_offset=elem_offset, out=self.xt, x0_out=self.x0)
+            sch.update(self.xt, eps, self.coef, z=None, seed=self.seed, step_dev=self.step_idx,
+                       elem_offset=elem_offset, out=self.xt, x0_out=self.x0)
             rt.check(L.cnb_bump_index(self.step_idx.data_ptr(), 1, rt.stream()))
 
         # warm-up on a side stream: builds weight / hint caches and sets kernel attributes outside the capture
@@ -95,22 +103,24 @@ class DDPMSampler:
             one_step()
         self.launches_per_step = rt.launch_count() - c0
         self._graph = g
-        self._nsteps, self._pos = steps, 0
+        self._nsteps, self._pos = len(ts), 0
         # keep every tensor the graph reads alive for as long as the graph: the hint features (HintCache may evict)
         cache = getattr(self.model, "_hint_cache", None)
         self._baked = cache.pinned() if cache is not None else []
 
     @torch.no_grad()
     def sample(self, x_T, hint, steps=None, elem_offset=0):
-        """Run t = steps-1 .. 0 (SURVEY.md 3.5 semantics) with fused on-device noise; returns (x_{-1 mean}, x0)."""
+        """Run the scheduler's timesteps (DDPM: t = steps-1 .. 0, SURVEY.md 3.5 semantics) with fused on-device noise;
+        returns (x after the last step, x0)."""
         rt.require_cuda(x_T, hint)
-        steps = self.scheduler.num_timesteps if steps is None else steps
+        sch = self.scheduler
         if not self.use_graph:
             return self.sample_eager(x_T, hint, steps, None, elem_offset)
         if hint.shape[0] != x_T.shape[0]:
             raise rt.CnbError("sample: x_T and hint must have the same batch size")
-        key = (tuple(x_T.shape), tuple(hint.shape), steps, elem_offset, rt.get_mode(), str(x_T.device),
-               self._param_stamp())
+        # the table's address tells apart schedulers with equal graph keys but other beta schedules
+        key = (tuple(x_T.shape), tuple(hint.shape), sch.graph_key(steps), sch.coef_table(x_T.device, steps).data_ptr(),
+               elem_offset, rt.get_mode(), str(x_T.device), self._param_stamp())
         if self._graph is None or key != self._key:
             self._capture(x_T, hint, steps, elem_offset)
             self._key = key
@@ -118,7 +128,7 @@ class DDPMSampler:
             self._hint.copy_(hint)
             self._refresh_hint()
         self.xt.copy_(x_T)
-        self.replay_steps(steps, reset=True)
+        self.replay_steps(self._nsteps, reset=True)
         out = self.xt.clone(), self.x0.clone()
         check_device_errors()
         return out

@@ -165,7 +165,22 @@ int cnb_time_embedding(const int64_t* t, const float* factor, float* out, int n,
 int cnb_sched_step(const float* xt, const float* eps, const float* z, float* xt_prev, float* x0, long long n,
                    const float* coef, uint64_t seed, uint64_t step, const int32_t* step_dev, uint64_t elem_offset,
                    cnb_stream_t stream);
-/* Fill out[i] with the same N(0,1) stream as above (used for x_T and by tests). */
+/*
+ * One DDIM update (scheduler/ddim_scheduler.py; no counterpart in the reference).  For step k of the timesteps
+ * tau_0 > ... > tau_{S-1}, with a_t = alpha_cum_prod[tau_k] and a_p = alpha_cum_prod[tau_{k+1}] (1.0 at the last step),
+ * coef (device, 6 floats) holds
+ *   [0] sqrt_one_minus_alpha_cum_prod[tau_k]  [1] sqrt_alpha_cum_prod[tau_k]  [2] sqrt(a_p)
+ *   [3] sqrt(max(1 - a_p - sigma^2, 0))  [4] sigma  [5] 1.0 if sigma > 0 (noise is added) else 0.0
+ * where sigma = eta * sqrt((1 - a_p) / (1 - a_t)) * sqrt(1 - a_t / a_p).  Per element, fp32, no FMA contraction:
+ *   x0 = (xt - c0 * eps) / c1   (the operations of cnb_sched_step's x0, so that x0 is bit-identical to it)
+ *   x_prev = c2 * (clip_sample ? clamp(x0, -1, 1) : x0) + c3 * eps  (+ c4 * z when c5 != 0)
+ * and the x0 output is clamp(x0, -1, 1).  z, x0, seed, step, step_dev and elem_offset behave as in cnb_sched_step:
+ * z == NULL draws the same Philox stream, keyed by (seed, step, elem_offset + i); x0 may be NULL; xt_prev may alias xt.
+ */
+int cnb_ddim_step(const float* xt, const float* eps, const float* z, float* xt_prev, float* x0, long long n,
+                  const float* coef, int clip_sample, uint64_t seed, uint64_t step, const int32_t* step_dev,
+                  uint64_t elem_offset, cnb_stream_t stream);
+/* Fill out[i] with the same N(0,1) stream as cnb_sched_step (used for x_T and by tests). */
 int cnb_philox_normal(float* out, long long n, uint64_t seed, uint64_t step, uint64_t elem_offset,
                       cnb_stream_t stream);
 /* dst[0..ncols) = table[row_index[0] * ncols ..]; row_index lives on the device so a captured graph can be
