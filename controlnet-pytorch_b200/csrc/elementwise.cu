@@ -1,6 +1,6 @@
 // Small / memory-bound kernels of the path: time embedding, t-embedding MLP rows, scheduler step (bit-exact fp32
-// restatement of scheduler/linear_noise_scheduler.py:58-77 with optional fused Philox noise), DDIM step, EDM scalings,
-// NCHW <-> channels-last plumbing and one-time weight packers.
+// restatement of scheduler/linear_noise_scheduler.py:58-77 with optional fused Philox noise), DDIM and DPM-Solver++
+// steps, EDM scalings, NCHW <-> channels-last plumbing and one-time weight packers.
 #include <cuda_fp16.h>
 
 #include "common.cuh"
@@ -215,6 +215,61 @@ __global__ void ddim_step_kernel(const float* __restrict__ xt, const float* __re
     float p, o;
     ddim_one(xt[i], eps[i], zv, c0, c1, c2, c3, c4, noisy, clip, p, o);
     prev[i] = p;
+    if (x0) x0[i] = o;
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
+// DPM-Solver++ multistep update (scheduler/dpm_solver_scheduler.py): D = x0 as sched_one computes it (clamped with
+// clip_sample), x_prev = A * xt + B0 * D (+ B1 * hist) (+ C * z), hist = D; separate IEEE ops.  hist is read only
+// when B1 != 0, so a first-order row never touches the previous step's (possibly uninitialised) buffer.
+// ------------------------------------------------------------------------------------------------
+__device__ __forceinline__ void dpm_one(float xt, float e, float zv, float hv, const float c0, const float c1,
+                                        const float A, const float B0, const float B1, const float C,
+                                        const bool second, const bool noisy, const bool clip, float& prev,
+                                        float& d, float& x0) {
+  const float v = __fdiv_rn(__fsub_rn(xt, __fmul_rn(c0, e)), c1);
+  x0 = fminf(fmaxf(v, -1.0f), 1.0f);
+  d = clip ? x0 : v;
+  float p = __fadd_rn(__fmul_rn(A, xt), __fmul_rn(B0, d));
+  if (second) p = __fadd_rn(p, __fmul_rn(B1, hv));
+  prev = noisy ? __fadd_rn(p, __fmul_rn(C, zv)) : p;
+}
+
+__global__ void dpm_solver_step_kernel(const float* __restrict__ xt, const float* __restrict__ eps,
+                                       const float* __restrict__ z, float* __restrict__ hist,
+                                       float* __restrict__ prev, float* __restrict__ x0, long long n,
+                                       const float* __restrict__ coef, int clip_sample, uint64_t seed, uint64_t step,
+                                       const int32_t* __restrict__ step_dev, uint64_t elem_offset) {
+  if (step_dev) step = (uint64_t)step_dev[0];
+  const float c0 = coef[0], c1 = coef[1], A = coef[2], B0 = coef[3], B1 = coef[4], C = coef[5];
+  const bool second = B1 != 0.0f, noisy = C != 0.0f, clip = clip_sample != 0;
+  const long long n4 = n >> 2;
+  const bool aligned4 = ((elem_offset & 3) == 0);
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
+    float4 a = reinterpret_cast<const float4*>(xt)[i];
+    float4 e = reinterpret_cast<const float4*>(eps)[i];
+    const float4 zz = noisy ? step_noise4(z, i, seed, step, elem_offset, aligned4) : make_float4(0.f, 0.f, 0.f, 0.f);
+    const float4 h = second ? reinterpret_cast<const float4*>(hist)[i] : make_float4(0.f, 0.f, 0.f, 0.f);
+    float4 p, d, o;
+    dpm_one(a.x, e.x, zz.x, h.x, c0, c1, A, B0, B1, C, second, noisy, clip, p.x, d.x, o.x);
+    dpm_one(a.y, e.y, zz.y, h.y, c0, c1, A, B0, B1, C, second, noisy, clip, p.y, d.y, o.y);
+    dpm_one(a.z, e.z, zz.z, h.z, c0, c1, A, B0, B1, C, second, noisy, clip, p.z, d.z, o.z);
+    dpm_one(a.w, e.w, zz.w, h.w, c0, c1, A, B0, B1, C, second, noisy, clip, p.w, d.w, o.w);
+    reinterpret_cast<float4*>(prev)[i] = p;
+    reinterpret_cast<float4*>(hist)[i] = d;
+    if (x0) reinterpret_cast<float4*>(x0)[i] = o;
+  }
+  // tail (n % 4 elements)
+  if (blockIdx.x == 0 && threadIdx.x < (n & 3)) {
+    long long i = (n4 << 2) + threadIdx.x;
+    const float zv = noisy ? step_noise1(z, i, seed, step, elem_offset) : 0.f;
+    const float hv = second ? hist[i] : 0.f;
+    float p, d, o;
+    dpm_one(xt[i], eps[i], zv, hv, c0, c1, A, B0, B1, C, second, noisy, clip, p, d, o);
+    prev[i] = p;
+    hist[i] = d;
     if (x0) x0[i] = o;
   }
 }
@@ -459,6 +514,29 @@ extern "C" int cnb_ddim_step(const float* xt, const float* eps, const float* z, 
   if (blocks > 148 * 16) blocks = 148 * 16;
   ddim_step_kernel<<<blocks, 256, 0, (cudaStream_t)s>>>(xt, eps, z, xt_prev, x0, n, coef, clip_sample, seed, step,
                                                         step_dev, elem_offset);
+  CNB_LAUNCH_CHECK();
+  return CNB_OK;
+}
+
+static bool cnb_overlaps(const float* a, const float* b, long long n) {
+  return a && b && a < b + n && b < a + n;
+}
+
+extern "C" int cnb_dpm_solver_step(const float* xt, const float* eps, const float* z, float* hist, float* xt_prev,
+                                   float* x0, long long n, const float* coef, int clip_sample, uint64_t seed,
+                                   uint64_t step, const int32_t* step_dev, uint64_t elem_offset, cnb_stream_t s) {
+  CNB_REQUIRE(n > 0 && xt && eps && hist && xt_prev && coef, "dpm_solver_step: null pointer or n=%lld", n);
+  CNB_REQUIRE(!cnb_overlaps(hist, xt, n) && !cnb_overlaps(hist, xt_prev, n) && !cnb_overlaps(hist, x0, n),
+              "dpm_solver_step: hist must not overlap xt, xt_prev or x0");
+  CNB_REQUIRE((((uintptr_t)xt | (uintptr_t)eps | (uintptr_t)xt_prev | (uintptr_t)z | (uintptr_t)x0 |
+                (uintptr_t)hist) & 15) == 0,
+              "dpm_solver_step: pointers must be 16-byte aligned");
+  long long n4 = n >> 2;
+  unsigned blocks = (unsigned)((n4 + 255) / 256);
+  if (blocks < 1) blocks = 1;
+  if (blocks > 148 * 16) blocks = 148 * 16;
+  dpm_solver_step_kernel<<<blocks, 256, 0, (cudaStream_t)s>>>(xt, eps, z, hist, xt_prev, x0, n, coef, clip_sample,
+                                                              seed, step, step_dev, elem_offset);
   CNB_LAUNCH_CHECK();
   return CNB_OK;
 }

@@ -255,6 +255,22 @@ def ddim_step(xt, eps, coef, z=None, want_x0=True, clip_sample=False, seed=0, st
     return prev, x0
 
 
+def dpm_solver_step(xt, eps, coef, z=None, want_x0=True, clip_sample=False, seed=0, step=0, step_dev=None,
+                    elem_offset=0, out=None, x0_out=None, *, hist):
+    """One DPM-Solver++ update (cnb_dpm_solver_step); coef is a row of DPMSolverMultistepScheduler.coef_table.  hist
+    (fp32, xt's size) holds the previous step's data prediction and receives this step's.  Same conventions as
+    sched_step."""
+    rt.require_cuda(xt, eps, coef, z, step_dev, out, x0_out, hist)
+    if hist.dtype != torch.float32 or hist.numel() != xt.numel() or not hist.is_contiguous():
+        raise rt.CnbError("dpm_solver_step: hist must be a contiguous fp32 tensor with xt's number of elements")
+    prev = torch.empty_like(xt) if out is None else out
+    x0 = x0_out if x0_out is not None else (torch.empty_like(xt) if want_x0 else None)
+    rt.check(rt.lib().cnb_dpm_solver_step(xt.data_ptr(), eps.data_ptr(), rt.ptr(z), hist.data_ptr(), prev.data_ptr(),
+                                          rt.ptr(x0), xt.numel(), coef.data_ptr(), 1 if clip_sample else 0, seed,
+                                          step, rt.ptr(step_dev), elem_offset, rt.stream()))
+    return prev, x0
+
+
 def philox_normal(shape, device, seed, step, elem_offset=0):
     out = torch.empty(shape, device=device, dtype=torch.float32)
     rt.require_cuda(out)

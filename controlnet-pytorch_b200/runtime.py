@@ -62,6 +62,8 @@ _SIGS = {
                                c_void_p, c_u64, c_void_p]),
     "cnb_ddim_step": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_ll, c_void_p, c_int, c_u64, c_u64,
                               c_void_p, c_u64, c_void_p]),
+    "cnb_dpm_solver_step": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_ll, c_void_p, c_int,
+                                    c_u64, c_u64, c_void_p, c_u64, c_void_p]),
     "cnb_philox_normal": (c_int, [c_void_p, c_ll, c_u64, c_u64, c_u64, c_void_p]),
     "cnb_gather_row": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
     "cnb_sampler_prologue": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),

@@ -8,10 +8,13 @@ tools/sample_ldm_controlnet.py:45-50 with the per-step host work removed.
   * data parallel: each rank owns a contiguous slice of the batch, no collective inside the loop, one all_gather of
     the final samples (NCCL over NVLink) at the end.
 
-The algorithm is the scheduler's: a LinearNoiseScheduler (DDPM, t = steps-1 .. 0) or a DDIMScheduler (a strided
-schedule) answers the same questions - `timesteps(steps)`, the [T, 6] `coef_table(device, steps)` the sampler prologue
-reads at row t, the fused `update` launch, and the `graph_key(steps)` of what a captured step depends on.  With
-steps=None the schedule is the scheduler's own (all T timesteps for DDPM, num_inference_steps for DDIM).
+The algorithm is the scheduler's: a LinearNoiseScheduler (DDPM, t = steps-1 .. 0), a DDIMScheduler or a
+DPMSolverMultistepScheduler (strided schedules) answers the same questions - `timesteps(steps)`, the [T, 6]
+`coef_table(device, steps)` the sampler prologue reads at row t, the fused `update` launch, the `graph_key(steps)` of
+what a captured step depends on, and `new_state(x)`, the dict of per-run device buffers carried from one step to the
+next (DPM-Solver++'s previous data prediction; empty for DDPM and DDIM) that the sampler allocates once per run, or
+once per captured graph, and passes to every `update`.  With steps=None the schedule is the scheduler's own (all T
+timesteps for DDPM, num_inference_steps for the strided schedulers).
 """
 
 import torch
@@ -39,14 +42,15 @@ class DDPMSampler:
         ts = sch.timesteps(steps)
         table = sch.coef_table(x_T.device, steps)
         xt, x0 = x_T.contiguous(), None
+        state = sch.new_state(xt)
         t_dev = torch.empty((1,), device=x_T.device, dtype=torch.int64)
         for k, t in enumerate(ts):
             t_dev.fill_(t)
             eps = self.model(xt, t_dev, hint)
-            # the last step adds no noise in either scheduler, so zs may stop one short of the schedule
+            # the last step adds no noise in any scheduler, so zs may stop one short of the schedule
             z = zs[k].to(xt.device) if (zs is not None and k < len(ts) - 1) else None
             xt, x0 = sch.update(xt, eps, table[t], z=z, want_x0=True, seed=self.seed, step=k,
-                                elem_offset=elem_offset)
+                                elem_offset=elem_offset, **state)
             if callback is not None:
                 callback(t, xt, x0)
         return xt, x0
@@ -80,6 +84,8 @@ class DDPMSampler:
         self.coef = torch.zeros((6,), device=dev, dtype=torch.float32)
         table = sch.coef_table(dev, steps)
         self._table = table          # the graph reads it: kept alive, so no other table can take its address
+        self._state = sch.new_state(self.xt)   # carried across replays: owned by the sampler, as long as the graph
+        state = self._state
         L = rt.lib()
 
         def one_step():
@@ -87,7 +93,7 @@ class DDPMSampler:
                                             table.data_ptr(), self.coef.data_ptr(), rt.stream()))
             eps = self.model(self.xt, self.t_out, hint)
             sch.update(self.xt, eps, self.coef, z=None, seed=self.seed, step_dev=self.step_idx,
-                       elem_offset=elem_offset, out=self.xt, x0_out=self.x0)
+                       elem_offset=elem_offset, out=self.xt, x0_out=self.x0, **state)
             rt.check(L.cnb_bump_index(self.step_idx.data_ptr(), 1, rt.stream()))
 
         # warm-up on a side stream: builds weight / hint caches and sets kernel attributes outside the capture

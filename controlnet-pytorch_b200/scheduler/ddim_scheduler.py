@@ -14,15 +14,12 @@ columns 3 and 4 are evaluated in float64 from the fp32 alpha_cum_prod and rounde
 kernel (cnb_ddim_step).  eta = 0 is deterministic DDIM; eta = 1 with S = T is the DDPM posterior step.
 """
 import math
-import numbers
-from fractions import Fraction
 
 import torch
 
 from .. import ops
 from .. import runtime as rt
-
-SPACINGS = ("trailing", "leading")
+from .schedule import strided_timesteps
 
 
 class DDIMScheduler:
@@ -51,22 +48,8 @@ class DDIMScheduler:
 
     def timesteps(self, steps=None):
         """tau_0 > ... > tau_{S-1} as a tuple of ints; `steps` overrides num_inference_steps."""
-        T = self.num_timesteps
-        if self.explicit_timesteps is not None:
-            ts = self.explicit_timesteps
-            if steps is not None and int(steps) != len(ts):
-                raise rt.CnbError(f"DDIMScheduler: steps={steps} disagrees with the {len(ts)} explicit timesteps")
-            if not ts or any(not 0 <= t < T for t in ts) or any(a <= b for a, b in zip(ts, ts[1:])):
-                raise rt.CnbError(f"DDIMScheduler: timesteps must be strictly decreasing and inside [0, {T})")
-            return ts
-        S = self.num_inference_steps if steps is None else steps
-        if isinstance(S, bool) or not isinstance(S, numbers.Integral) or not 1 <= S <= T:
-            raise rt.CnbError(f"DDIMScheduler: the number of steps must be an int in [1, {T}] (got {S!r})")
-        if self.spacing == "trailing":
-            return tuple(round(Fraction(T) - Fraction(k * T, S)) - 1 for k in range(S))   # round(): half to even
-        if self.spacing == "leading":
-            return tuple((S - 1 - k) * (T // S) for k in range(S))
-        raise rt.CnbError(f"DDIMScheduler: spacing must be one of {SPACINGS} (got {self.spacing!r})")
+        return strided_timesteps("DDIMScheduler", self.num_timesteps, self.num_inference_steps, self.spacing,
+                                 self.explicit_timesteps, steps)
 
     def coef_table_host(self, steps=None):
         """fp32 [T, 6]: row tau_k is row_k of the module docstring; rows off the schedule are NaN, so that reading one
@@ -96,6 +79,10 @@ class DDIMScheduler:
     def graph_key(self, steps=None):
         """Everything a captured sampling step depends on besides the model and the coefficient table."""
         return ("ddim", self.timesteps(steps), self._eta(), bool(self.clip_sample))
+
+    def new_state(self, x):
+        """DDIM carries nothing from one step to the next."""
+        return {}
 
     def update(self, xt, eps, coef, **kw):
         """The fused update for one row of coef_table (ops.ddim_step and its keyword arguments)."""

@@ -46,7 +46,8 @@ class LinearNoiseScheduler:
             self._coef[key] = self.coef_table_host().to(device)
         return self._coef[key]
 
-    # ---- what sampler.DDPMSampler asks a scheduler for (scheduler/ddim_scheduler.py answers the same questions)
+    # ---- what sampler.DDPMSampler asks a scheduler for (ddim_scheduler.py and dpm_solver_scheduler.py answer the
+    # same questions)
     def timesteps(self, steps=None):
         """t = steps-1 .. 0: the whole chain, or the reference's truncated chain for steps < T (SURVEY.md 3.5)."""
         steps = self.num_timesteps if steps is None else int(steps)
@@ -55,6 +56,10 @@ class LinearNoiseScheduler:
     def graph_key(self, steps=None):
         """Everything a captured sampling step depends on besides the model and the coefficient table."""
         return ("ddpm", self.timesteps(steps))
+
+    def new_state(self, x):
+        """The per-run device buffers `update` takes besides its row: the DDPM step carries none."""
+        return {}
 
     def update(self, xt, eps, coef, **kw):
         """The fused update for one row of coef_table (ops.sched_step and its keyword arguments)."""

@@ -180,6 +180,29 @@ int cnb_sched_step(const float* xt, const float* eps, const float* z, float* xt_
 int cnb_ddim_step(const float* xt, const float* eps, const float* z, float* xt_prev, float* x0, long long n,
                   const float* coef, int clip_sample, uint64_t seed, uint64_t step, const int32_t* step_dev,
                   uint64_t elem_offset, cnb_stream_t stream);
+/*
+ * One DPM-Solver++ multistep update (scheduler/dpm_solver_scheduler.py; no counterpart in the reference).  Step k of
+ * the timesteps tau_0 > ... > tau_{S-1} goes from s = tau_k to t = tau_{k+1} (to alpha_cum_prod = 1 after the last
+ * step), with alpha = sqrt(alpha_cum_prod), sigma = sqrt(1 - alpha_cum_prod), lambda = log(alpha / sigma),
+ * h_k = lambda_t - lambda_s, r_k = h_{k-1} / h_k and e^{-h} = (sigma_t alpha_s) / (alpha_t sigma_s).  coef (device,
+ * 6 floats) holds
+ *   [0] sqrt_one_minus_alpha_cum_prod[tau_k]  [1] sqrt_alpha_cum_prod[tau_k]  [2] A  [3] B0  [4] B1  [5] C
+ * where, with F = alpha_t (1 - e^{-h}) for variant "ode" and F = alpha_t (1 - e^{-2h}) for "sde",
+ *   A = sigma_t / sigma_s ("ode") or (sigma_t / sigma_s) e^{-h} ("sde");  C = 0 ("ode") or sigma_t sqrt(1 - e^{-2h})
+ *   first order (the first step, the last step, order 1):  B0 = F, B1 = 0
+ *   second order (2M, midpoint):  B0 = F (1 + 1 / (2 r_k)),  B1 = -F / (2 r_k).
+ * Per element, fp32, no FMA contraction:
+ *   v = (xt - c0 * eps) / c1   (the operations of cnb_sched_step's x0, so that x0 is bit-identical to it)
+ *   D = clip_sample ? clamp(v, -1, 1) : v
+ *   x_prev = A * xt + B0 * D  (+ B1 * hist when B1 != 0)  (+ C * z when C != 0);  hist = D
+ * and the x0 output is clamp(v, -1, 1).  hist (n floats, not overlapping xt, xt_prev or x0) carries the data
+ * prediction D from one step to the next; it is read only when B1 != 0, so the first step may pass an uninitialised
+ * buffer.  z, x0, seed, step, step_dev and elem_offset behave as in cnb_sched_step: z == NULL draws the same Philox
+ * stream; x0 may be NULL; xt_prev may alias xt.
+ */
+int cnb_dpm_solver_step(const float* xt, const float* eps, const float* z, float* hist, float* xt_prev, float* x0,
+                        long long n, const float* coef, int clip_sample, uint64_t seed, uint64_t step,
+                        const int32_t* step_dev, uint64_t elem_offset, cnb_stream_t stream);
 /* Fill out[i] with the same N(0,1) stream as cnb_sched_step (used for x_T and by tests). */
 int cnb_philox_normal(float* out, long long n, uint64_t seed, uint64_t step, uint64_t elem_offset,
                       cnb_stream_t stream);
