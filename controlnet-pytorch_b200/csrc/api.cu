@@ -36,7 +36,7 @@ bool pdl_enabled(long long work) {
 int conv2d_f32(const cnb_conv_params* p, cudaStream_t st);
 int conv2d_small(const cnb_conv_params* p, cudaStream_t st);
 bool conv2d_small_supported(const cnb_conv_params* p);
-int conv2d_tma(const cnb_conv_params* p, cudaStream_t st);
+int conv2d_tma(const cnb_conv_params* p, cudaStream_t st, int32_t* route);
 bool conv2d_tma_supported(const cnb_conv_params* p);
 bool groupnorm_big_eligible(int B, int HW, int C, int G, int in_f16);
 size_t groupnorm_big_workspace(int B, int HW, int C, int G);
@@ -75,7 +75,9 @@ extern "C" long long cnb_launch_count(void) { return g_launches.load(); }
 extern "C" void cnb_reset_launch_count(void) { g_launches.store(0); }
 extern "C" int cnb_has_tcgen05(void) { return query_tc(); }
 
-extern "C" int cnb_conv2d(const cnb_conv_params* p, cnb_stream_t stream) {
+// One decision for cnb_conv2d and cnb_conv2d_route: with `route` set, every branch fills it in and returns where it
+// would launch.
+static int conv2d_dispatch(const cnb_conv_params* p, cudaStream_t st, int32_t* route) {
   CNB_REQUIRE(p != nullptr, "conv2d: null params");
   CNB_REQUIRE(p->in && p->weight && p->out, "conv2d: null tensor pointer");
   CNB_REQUIRE(p->B > 0 && p->H > 0 && p->W > 0 && p->Cin > 0 && p->Cout > 0 && p->OH > 0 && p->OW > 0,
@@ -87,7 +89,6 @@ extern "C" int cnb_conv2d(const cnb_conv_params* p, cnb_stream_t stream) {
   CNB_REQUIRE((long long)p->B * p->OH * p->OW < (1ll << 31), "conv2d: M overflows int32");
   CNB_REQUIRE((p->OH - 1) * p->oy_mul + p->oy_add < p->OHf && (p->OW - 1) * p->ox_mul + p->ox_add < p->OWf,
               "conv2d: output mapping exceeds the output tensor");
-  cudaStream_t st = (cudaStream_t)stream;
   CNB_REQUIRE(p->in_dtype == 0 || p->in_dtype == 1, "conv2d: in_dtype=%d", p->in_dtype);
   CNB_REQUIRE(p->out_dtype == 0 || p->out_dtype == 1, "conv2d: out_dtype=%d", p->out_dtype);
   CNB_REQUIRE(p->res_dtype == 0 || p->res_dtype == 1, "conv2d: res_dtype=%d", p->res_dtype);
@@ -95,12 +96,18 @@ extern "C" int cnb_conv2d(const cnb_conv_params* p, cnb_stream_t stream) {
     CNB_REQUIRE(p->Cin2 > 0 && p->ldi2 >= p->in2_coff + p->Cin2, "conv2d: bad second input");
     CNB_REQUIRE(p->mode != CNB_MODE_F32 && conv2d_tma_supported(p),
                 "conv2d: a second input (K-concatenated 1x1 tap) needs the TMA tensor-core path");
-    return conv2d_tma(p, st);
+    return conv2d_tma(p, st, route);
   }
   // tiny-channel ends of the U-Net (Cin <= 4 or Cout <= 4): direct exact-fp32 kernels in every mode
-  if ((p->Cin <= 4 || p->Cout <= 4) && conv2d_small_supported(p)) return conv2d_small(p, st);
+  if ((p->Cin <= 4 || p->Cout <= 4) && conv2d_small_supported(p)) {
+    if (route) {
+      route[CNB_ROUTE_PATH] = CNB_PATH_SMALL;
+      return CNB_OK;
+    }
+    return conv2d_small(p, st);
+  }
   if (p->mode == CNB_MODE_F16) {
-    if (conv2d_tma_supported(p)) return conv2d_tma(p, st);     // TMA-im2col fed persistent tcgen05 kernel
+    if (conv2d_tma_supported(p)) return conv2d_tma(p, st, route);     // TMA-im2col fed persistent tcgen05 kernel
   } else if (p->mode != CNB_MODE_F32) {
     set_error("conv2d: unknown mode %d", p->mode);
     return CNB_ERR_BAD_ARG;
@@ -108,7 +115,21 @@ extern "C" int cnb_conv2d(const cnb_conv_params* p, cnb_stream_t stream) {
   // fp32 mode, and tiny-channel layers (Cin % 4 != 0 or Cout < 16) which are HBM-bound CUDA-core work
   CNB_REQUIRE(p->out_dtype == 0 && p->res_dtype == 0, "conv2d: fp16 output / residual needs a tensor-core eligible layer");
   CNB_REQUIRE(p->in_dtype == 0, "conv2d: fp16 activations need a tensor-core eligible layer (Cin %% 8 == 0, Cout %% 16 == 0)");
+  if (route) {
+    route[CNB_ROUTE_PATH] = CNB_PATH_F32;
+    return CNB_OK;
+  }
   return conv2d_f32(p, st);
+}
+
+extern "C" int cnb_conv2d(const cnb_conv_params* p, cnb_stream_t stream) {
+  return conv2d_dispatch(p, (cudaStream_t)stream, nullptr);
+}
+
+extern "C" int cnb_conv2d_route(const cnb_conv_params* p, int32_t* route) {
+  CNB_REQUIRE(route != nullptr, "conv2d_route: null route");
+  memset(route, 0, CNB_ROUTE_LEN * sizeof(int32_t));
+  return conv2d_dispatch(p, nullptr, route);
 }
 
 extern "C" size_t cnb_groupnorm_workspace_bytes(int B, int HW, int C, int G, int in_f16) {

@@ -40,8 +40,8 @@ static int resolve_driver() {
 
 }  // namespace tma
 
-int conv_tma_launch_f16(int rb, int bn, const tma::TmaArgs& a, int num_sms, cudaStream_t st);
-int conv_tma_launch_tf32(int rb, int bn, const tma::TmaArgs& a, int num_sms, cudaStream_t st);
+int conv_tma_launch_f16(int rb, int bn, const tma::TmaArgs& a, int num_sms, cudaStream_t st, int32_t* route);
+int conv_tma_launch_tf32(int rb, int bn, const tma::TmaArgs& a, int num_sms, cudaStream_t st, int32_t* route);
 int conv_tma_error_flag_f16();
 int conv_tma_error_flag_tf32();
 
@@ -100,7 +100,8 @@ bool conv2d_tma_supported(const cnb_conv_params* p) {
   return true;
 }
 
-int conv2d_tma(const cnb_conv_params* p, cudaStream_t st) {
+// route != nullptr: fill in the route (cnb_conv2d_route) instead of launching
+int conv2d_tma(const cnb_conv_params* p, cudaStream_t st, int32_t* route) {
   using namespace tma;
   int rc = resolve_driver();
   if (rc != CNB_OK) return rc;
@@ -287,7 +288,17 @@ int conv2d_tma(const cnb_conv_params* p, cudaStream_t st) {
   a.Cin = p->Cin; a.ntaps = p->ntaps; a.kchunks = ceil_div(p->Cin, kc);
   a.stride = p->stride; a.lower_w = dxmin; a.lower_h = dymin;
   a.tiles_m = halo ? p->B * a.tiles_y : ceil_div(a.M, BM); a.tiles_n = p->Cout / bn;
-  return half ? conv_tma_launch_f16(rb, bn, a, g_num_sms, st) : conv_tma_launch_tf32(rb, bn, a, g_num_sms, st);
+  if (route) {
+    route[CNB_ROUTE_PATH] = CNB_PATH_TMA;
+    route[CNB_ROUTE_RB] = rb;
+    route[CNB_ROUTE_BN] = bn;
+    route[CNB_ROUTE_HALO] = halo ? 1 : 0;
+    route[CNB_ROUTE_TILES_N] = a.tiles_n;
+    route[CNB_ROUTE_HALO_R] = halo ? a.R : 0;
+    route[CNB_ROUTE_TILES_Y] = halo ? a.tiles_y : 0;
+  }
+  return half ? conv_tma_launch_f16(rb, bn, a, g_num_sms, st, route)
+              : conv_tma_launch_tf32(rb, bn, a, g_num_sms, st, route);
 }
 
 }  // namespace cnb

@@ -692,7 +692,7 @@ conv_tma_kernel(const __grid_constant__ TmaArgs a) {
 }
 
 template <int BN, bool HALF, int EPI, int RB>
-static int launch_epi(const TmaArgs& a_in, int num_sms, cudaStream_t st) {
+static int launch_epi(const TmaArgs& a_in, int num_sms, cudaStream_t st, int32_t* route) {
   using C = Cfg<BN, RB>;
   static DeviceOnce attr_once;
   if (attr_once.first()) {
@@ -778,50 +778,60 @@ static int launch_epi(const TmaArgs& a_in, int num_sms, cudaStream_t st) {
     if (EPI == 6) a.epi_alt = 0;
   }
   smem_bytes = (size_t)a.bar_off + C::BAR_BYTES + 1024;
+  if (route) {        // cnb_conv2d_route: everything above is the launch's own decision
+    route[CNB_ROUTE_EPI] = EPI;
+    route[CNB_ROUTE_BRES] = a.bres;
+    route[CNB_ROUTE_CTAS_PER_SM] = two ? 2 : 1;
+    route[CNB_ROUTE_EPI_ALT] = a.epi_alt;
+    route[CNB_ROUTE_EPI_NBUF] = EPI == 6 ? a.epi_nbuf : 0;
+    route[CNB_ROUTE_GRID] = grid;
+    route[CNB_ROUTE_NTILES] = ntiles;
+    return CNB_OK;
+  }
   CNB_CUDA(launch_pdl((long long)ntiles * 128 * BN, conv_tma_kernel<BN, HALF, EPI, RB>, dim3(grid), dim3(NUM_THREADS), smem_bytes, st, a));
   CNB_LAUNCH_CHECK();
   return CNB_OK;
 }
 
 template <int BN, bool HALF, int RB>
-static int launch(const TmaArgs& a, int num_sms, cudaStream_t st) {
+static int launch(const TmaArgs& a, int num_sms, cudaStream_t st, int32_t* route) {
   const bool dense = !a.halo && a.oy_mul == 1 && a.ox_mul == 1 && a.oy_add == 0 && a.ox_add == 0 &&
                      a.OHf * a.OWf == a.OHW;
   const bool simple = dense && a.act == 0 && !(a.temb && a.temb_per_sample);
   if (a.halo && a.act == 0 && !(a.temb && a.temb_per_sample) && a.out_f16 && (!a.residual || a.res_f16))
-    return launch_epi<BN, HALF, 5, RB>(a, num_sms, st);
-  if (simple && !a.out_f16 && !a.residual) return launch_epi<BN, HALF, 0, RB>(a, num_sms, st);
-  if (simple && !a.out_f16 && a.residual && !a.res_f16) return launch_epi<BN, HALF, 1, RB>(a, num_sms, st);
+    return launch_epi<BN, HALF, 5, RB>(a, num_sms, st, route);
+  if (simple && !a.out_f16 && !a.residual) return launch_epi<BN, HALF, 0, RB>(a, num_sms, st, route);
+  if (simple && !a.out_f16 && a.residual && !a.res_f16) return launch_epi<BN, HALF, 1, RB>(a, num_sms, st, route);
   if constexpr (HALF) {
-    if (simple && a.out_f16 && a.tma_epi && (!a.residual || a.res_f16)) return launch_epi<BN, HALF, 6, RB>(a, num_sms, st);
+    if (simple && a.out_f16 && a.tma_epi && (!a.residual || a.res_f16)) return launch_epi<BN, HALF, 6, RB>(a, num_sms, st, route);
   }
-  if (simple && a.out_f16 && !a.residual) return launch_epi<BN, HALF, 2, RB>(a, num_sms, st);
-  if (simple && a.out_f16 && a.residual && a.res_f16) return launch_epi<BN, HALF, 4, RB>(a, num_sms, st);
-  return launch_epi<BN, HALF, 3, RB>(a, num_sms, st);
+  if (simple && a.out_f16 && !a.residual) return launch_epi<BN, HALF, 2, RB>(a, num_sms, st, route);
+  if (simple && a.out_f16 && a.residual && a.res_f16) return launch_epi<BN, HALF, 4, RB>(a, num_sms, st, route);
+  return launch_epi<BN, HALF, 3, RB>(a, num_sms, st, route);
 }
 
 template <bool HALF, int RB>
-static int dispatch_bn(int bn, const TmaArgs& a, int num_sms, cudaStream_t st) {
+static int dispatch_bn(int bn, const TmaArgs& a, int num_sms, cudaStream_t st, int32_t* route) {
   switch (bn) {
-    case 256: return launch<256, HALF, RB>(a, num_sms, st);
-    case 192: return launch<192, HALF, RB>(a, num_sms, st);
-    case 128: return launch<128, HALF, RB>(a, num_sms, st);
-    case 96: return launch<96, HALF, RB>(a, num_sms, st);
-    case 64: return launch<64, HALF, RB>(a, num_sms, st);
-    case 48: return launch<48, HALF, RB>(a, num_sms, st);
-    case 32: return launch<32, HALF, RB>(a, num_sms, st);
-    case 16: return launch<16, HALF, RB>(a, num_sms, st);
+    case 256: return launch<256, HALF, RB>(a, num_sms, st, route);
+    case 192: return launch<192, HALF, RB>(a, num_sms, st, route);
+    case 128: return launch<128, HALF, RB>(a, num_sms, st, route);
+    case 96: return launch<96, HALF, RB>(a, num_sms, st, route);
+    case 64: return launch<64, HALF, RB>(a, num_sms, st, route);
+    case 48: return launch<48, HALF, RB>(a, num_sms, st, route);
+    case 32: return launch<32, HALF, RB>(a, num_sms, st, route);
+    case 16: return launch<16, HALF, RB>(a, num_sms, st, route);
   }
   set_error("conv_tma: no tile for Cout");
   return CNB_ERR_UNSUPPORTED;
 }
 
 template <bool HALF>
-static int dispatch_rb(int rb, int bn, const TmaArgs& a, int num_sms, cudaStream_t st) {
+static int dispatch_rb(int rb, int bn, const TmaArgs& a, int num_sms, cudaStream_t st, int32_t* route) {
   switch (rb) {
-    case 128: return dispatch_bn<HALF, 128>(bn, a, num_sms, st);
-    case 64: return dispatch_bn<HALF, 64>(bn, a, num_sms, st);
-    case 32: return dispatch_bn<HALF, 32>(bn, a, num_sms, st);
+    case 128: return dispatch_bn<HALF, 128>(bn, a, num_sms, st, route);
+    case 64: return dispatch_bn<HALF, 64>(bn, a, num_sms, st, route);
+    case 32: return dispatch_bn<HALF, 32>(bn, a, num_sms, st, route);
   }
   set_error("conv_tma: row bytes %d", rb);
   return CNB_ERR_UNSUPPORTED;

@@ -46,12 +46,10 @@ def empty(*shape, device, dtype=torch.float32):
     return torch.empty(shape, device=device, dtype=dtype)
 
 
-def conv(x, weight, kind, cout, *, bias=None, temb=None, temb_ld=0, temb_per_sample=False, residual=None,
-         res_coff=0, act=0, out=None, out_coff=0, in_coff=0, cin=None, mode=None, phase=None, weight_lp=None,
-         out_f16=False, x2=None, x2_coff=0, cin2=None):
-    """Launch cnb_conv2d.  `x` is (B, H, W, ldi); `weight` is the packed [cout][ntaps][cin] tensor.
-    kind in {"1x1","3x3","3x3s2","4x4s2"} or phase=(py,px) for a ConvTranspose2d phase (then `out` is required
-    and has spatial size (2H, 2W))."""
+def _conv_params(x, weight, kind, cout, *, bias=None, temb=None, temb_ld=0, temb_per_sample=False, residual=None,
+                 res_coff=0, act=0, out=None, out_coff=0, in_coff=0, cin=None, mode=None, phase=None, weight_lp=None,
+                 out_f16=False, x2=None, x2_coff=0, cin2=None):
+    """(ConvParams, out) for conv / conv_route; allocates `out` when it is None."""
     rt.require_cuda(x, weight, bias, temb, residual, out, weight_lp, x2)
     half = x.dtype == torch.float16
     if half and weight_lp is None and cout > 4:
@@ -94,8 +92,30 @@ def conv(x, weight, kind, cout, *, bias=None, temb=None, temb_ld=0, temb_per_sam
     p.temb_ld, p.temb_per_sample = temb_ld, 1 if temb_per_sample else 0
     p.act = act
     p.mode = rt.get_mode() if mode is None else mode
+    return p, out
+
+
+def conv(x, weight, kind, cout, **kw):
+    """Launch cnb_conv2d.  `x` is (B, H, W, ldi); `weight` is the packed [cout][ntaps][cin] tensor.
+    kind in {"1x1","3x3","3x3s2","4x4s2"} or phase=(py,px) for a ConvTranspose2d phase (then `out` is required
+    and has spatial size (2H, 2W))."""
+    p, out = _conv_params(x, weight, kind, cout, **kw)
     rt.check(rt.lib().cnb_conv2d(ctypes.byref(p), rt.stream()))
     return out
+
+
+ROUTE_FIELDS = ("path", "rb", "bn", "epi", "halo", "bres", "ctas_per_sm", "epi_alt", "epi_nbuf", "grid", "ntiles",
+                "tiles_n", "halo_r", "tiles_y")      # CNB_ROUTE_* order (include/cnb200.h)
+PATH_NAMES = ("f32", "small", "tma")                  # CNB_PATH_*
+
+
+def conv_route(x, weight, kind, cout, **kw):
+    """The kernel route conv(...) with the same arguments would take (cnb_conv2d_route), as {ROUTE_FIELDS: int};
+    nothing is launched.  Raises what conv would raise before its launch."""
+    p, _ = _conv_params(x, weight, kind, cout, **kw)
+    r = (ctypes.c_int32 * rt.ROUTE_LEN)()
+    rt.check(rt.lib().cnb_conv2d_route(ctypes.byref(p), r))
+    return dict(zip(ROUTE_FIELDS, r))
 
 
 def groupnorm(x, gamma, beta, groups, silu, eps=1e-5, out_f16=False):

@@ -12,6 +12,7 @@ _LIB_PATH = os.path.join(_HERE, "libcnb200.so")
 
 MODE_F32, MODE_F16 = 0, 1
 MAX_TAPS = 16
+ROUTE_LEN = 16      # CNB_ROUTE_LEN
 
 c_void_p, c_int, c_ll, c_float, c_u64 = ctypes.c_void_p, ctypes.c_int, ctypes.c_longlong, ctypes.c_float, ctypes.c_uint64
 
@@ -43,6 +44,7 @@ _SIGS = {
     "cnb_reset_launch_count": (None, []),
     "cnb_has_tcgen05": (c_int, []),
     "cnb_conv2d": (c_int, [ctypes.POINTER(ConvParams), c_void_p]),
+    "cnb_conv2d_route": (c_int, [ctypes.POINTER(ConvParams), ctypes.POINTER(ctypes.c_int32)]),
     "cnb_pack_conv_weight": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "cnb_pack_convT_weight": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_void_p]),
     "cnb_cast_f16": (c_int, [c_void_p, c_void_p, c_ll, c_void_p]),

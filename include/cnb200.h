@@ -97,6 +97,30 @@ typedef struct cnb_conv_params {
 
 int cnb_conv2d(const cnb_conv_params* p, cnb_stream_t stream);
 
+/* The kernel route cnb_conv2d takes for `p` on the current device, without launching anything: route[] receives
+ * CNB_ROUTE_LEN values indexed by CNB_ROUTE_* (fields that do not apply to the path are 0).  Returns the error
+ * cnb_conv2d would return before its launch.  cnb_conv2d makes the same decision in the same code, so tests can name
+ * the variant a call site reaches and check that a replay of it reaches the same one. */
+#define CNB_ROUTE_LEN 16
+#define CNB_PATH_F32 0     /* CUDA-core fp32 implicit GEMM (conv_f32.cu)          */
+#define CNB_PATH_SMALL 1   /* direct kernels for Cin <= 4 or Cout <= 4 (conv_small.cu) */
+#define CNB_PATH_TMA 2     /* TMA-fed tcgen05 kernel (conv_tma.cu)                */
+#define CNB_ROUTE_PATH 0         /* CNB_PATH_*                                                   */
+#define CNB_ROUTE_RB 1           /* TMA: bytes of K per smem row (swizzle span 32 / 64 / 128)    */
+#define CNB_ROUTE_BN 2           /* TMA: N tile after N-split narrowing                           */
+#define CNB_ROUTE_EPI 3          /* TMA: epilogue variant 0..6 (conv_tma_impl.cuh)                */
+#define CNB_ROUTE_HALO 4         /* TMA: 1 = halo mode (3x3 bands loaded once per channel chunk)  */
+#define CNB_ROUTE_BRES 5         /* TMA: 1 = weights resident in shared memory                    */
+#define CNB_ROUTE_CTAS_PER_SM 6  /* TMA: 1 or 2                                                   */
+#define CNB_ROUTE_EPI_ALT 7      /* TMA: 1 = the epilogue warp groups alternate tiles             */
+#define CNB_ROUTE_EPI_NBUF 8     /* TMA, EPI 6: staging buffers per epilogue warp (2 or 3)        */
+#define CNB_ROUTE_GRID 9         /* TMA: CTAs launched (tile = blockIdx.x + k * grid)             */
+#define CNB_ROUTE_NTILES 10      /* TMA: tiles_m * tiles_n                                        */
+#define CNB_ROUTE_TILES_N 11     /* TMA: N tiles per M tile (tile = m_tile * tiles_n + n_tile)    */
+#define CNB_ROUTE_HALO_R 12      /* TMA, halo: image rows per band                                */
+#define CNB_ROUTE_TILES_Y 13     /* TMA, halo: bands per sample (sample = tile / tiles_y)         */
+int cnb_conv2d_route(const cnb_conv_params* p, int32_t* route);
+
 /* OIHW -> [O][KH*KW][I] (tap = ky*KW+kx).  round_tf32 != 0 rounds to nearest tf32 (for CNB_MODE_F16). */
 int cnb_pack_conv_weight(const float* w_oihw, float* dst, int O, int I, int KH, int KW, int round_tf32,
                          cnb_stream_t stream);
