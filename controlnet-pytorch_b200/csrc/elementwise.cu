@@ -274,6 +274,104 @@ __global__ void dpm_solver_step_kernel(const float* __restrict__ xt, const float
   }
 }
 
+// ------------------------------------------------------------------------------------------------
+// image-to-image start and inpainting (sampler.DDPMSampler.img2img): out = a * x_ref + s * z with the operation order
+// of LinearNoiseScheduler.add_noise (mul, mul, add), and the per-step blend that puts the known region back,
+// out = m == 1 ? x : (m == 0 ? known : m * x + (1 - m) * known); separate IEEE ops.  out may alias x_ref, so neither
+// is __restrict__.
+// ------------------------------------------------------------------------------------------------
+__device__ __forceinline__ float noised(float xr, float zv, float a, float s) {
+  return __fadd_rn(__fmul_rn(a, xr), __fmul_rn(s, zv));
+}
+
+__global__ void add_noise_kernel(const float* x_ref, const float* __restrict__ z, float* out, long long n, float a,
+                                 float s, uint64_t seed, uint64_t step, uint64_t elem_offset) {
+  const long long n4 = n >> 2;
+  const bool aligned4 = ((elem_offset & 3) == 0);
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
+    const float4 xr = reinterpret_cast<const float4*>(x_ref)[i];
+    const float4 zz = step_noise4(z, i, seed, step, elem_offset, aligned4);
+    reinterpret_cast<float4*>(out)[i] =
+        make_float4(noised(xr.x, zz.x, a, s), noised(xr.y, zz.y, a, s), noised(xr.z, zz.z, a, s),
+                    noised(xr.w, zz.w, a, s));
+  }
+  if (blockIdx.x == 0 && threadIdx.x < (n & 3)) {
+    long long i = (n4 << 2) + threadIdx.x;
+    out[i] = noised(x_ref[i], step_noise1(z, i, seed, step, elem_offset), a, s);
+  }
+}
+
+__device__ __forceinline__ float blend_one(float xv, float xr, float zv, float m, float a, float s) {
+  if (m == 1.0f) return xv;
+  const float known = noised(xr, zv, a, s);
+  if (m == 0.0f) return known;
+  return __fadd_rn(__fmul_rn(m, xv), __fmul_rn(__fsub_rn(1.0f, m), known));
+}
+
+// mask element of NCHW element e: [B, mask_c, H, W] with mask_c == C, or mask_c == 1 broadcast over the channels
+__device__ __forceinline__ long long mask_index(long long e, int C, long long HW, int mask_c) {
+  if (mask_c != 1) return e;
+  const long long row = e / HW;          // b * C + c
+  return (row / C) * HW + (e - row * HW);
+}
+
+__global__ void inpaint_blend_kernel(float* __restrict__ x, const float* __restrict__ x_ref,
+                                     const float* __restrict__ mask, const float* __restrict__ z, long long n, int C,
+                                     long long HW, int mask_c, const float* __restrict__ levels, long long step,
+                                     const int32_t* __restrict__ step_dev, uint64_t seed, uint64_t noise_step,
+                                     uint64_t elem_offset) {
+  const long long k = step_dev ? (long long)step_dev[0] : step;
+  const float a = levels[2 * k], s = levels[2 * k + 1];
+  const long long n4 = n >> 2;
+  const bool aligned4 = ((elem_offset & 3) == 0);
+  // four consecutive elements share one mask row (and a 16-byte aligned mask float4) unless a broadcast mask row
+  // length is not a multiple of 4
+  const bool mvec = mask_c != 1 || (HW & 3) == 0;
+  const long long stride = (long long)gridDim.x * blockDim.x;
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
+    const long long e = i << 2;
+    float4 m;
+    if (mvec) {
+      m = reinterpret_cast<const float4*>(mask)[mask_index(e, C, HW, mask_c) >> 2];
+    } else {
+      m = make_float4(mask[mask_index(e, C, HW, 1)], mask[mask_index(e + 1, C, HW, 1)],
+                      mask[mask_index(e + 2, C, HW, 1)], mask[mask_index(e + 3, C, HW, 1)]);
+    }
+    float4 xv = reinterpret_cast<const float4*>(x)[i];
+    if (m.x == 1.0f && m.y == 1.0f && m.z == 1.0f && m.w == 1.0f) continue;   // all generated: x stays as it is
+    const float4 xr = reinterpret_cast<const float4*>(x_ref)[i];
+    const float4 zz = step_noise4(z, i, seed, noise_step, elem_offset, aligned4);
+    xv.x = blend_one(xv.x, xr.x, zz.x, m.x, a, s);
+    xv.y = blend_one(xv.y, xr.y, zz.y, m.y, a, s);
+    xv.z = blend_one(xv.z, xr.z, zz.z, m.z, a, s);
+    xv.w = blend_one(xv.w, xr.w, zz.w, m.w, a, s);
+    reinterpret_cast<float4*>(x)[i] = xv;
+  }
+  if (blockIdx.x == 0 && threadIdx.x < (n & 3)) {
+    long long i = (n4 << 2) + threadIdx.x;
+    const float m = mask[mask_index(i, C, HW, mask_c)];
+    x[i] = blend_one(x[i], x_ref[i], m == 1.0f ? 0.f : step_noise1(z, i, seed, noise_step, elem_offset), m, a, s);
+  }
+}
+
+// out[p, oy, ox] = max of in[p, oy*f .. oy*f+f-1, ox*f .. ox*f+f-1] over the planes p of a [P, H, W] tensor
+__global__ void mask_max_pool_kernel(const float* __restrict__ in, float* __restrict__ out, long long total, int H,
+                                     int W, int f) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= total) return;
+  const int OW = W / f, OH = H / f;
+  const int ox = (int)(i % OW);
+  const long long r = i / OW;
+  const int oy = (int)(r % OH);
+  const long long p = r / OH;
+  const float* src = in + (p * H + (long long)oy * f) * W + (long long)ox * f;
+  float v = src[0];
+  for (int dy = 0; dy < f; ++dy)
+    for (int dx = 0; dx < f; ++dx) v = fmaxf(v, src[(long long)dy * W + dx]);
+  out[i] = v;
+}
+
 __global__ void gather_row_kernel(const float* __restrict__ table, const int32_t* __restrict__ row,
                                   float* __restrict__ dst, int ncols) {
   const size_t r = (size_t)row[0];
@@ -537,6 +635,55 @@ extern "C" int cnb_dpm_solver_step(const float* xt, const float* eps, const floa
   if (blocks > 148 * 16) blocks = 148 * 16;
   dpm_solver_step_kernel<<<blocks, 256, 0, (cudaStream_t)s>>>(xt, eps, z, hist, xt_prev, x0, n, coef, clip_sample,
                                                               seed, step, step_dev, elem_offset);
+  CNB_LAUNCH_CHECK();
+  return CNB_OK;
+}
+
+static unsigned elementwise4_blocks(long long n) {
+  long long blocks = ((n >> 2) + 255) / 256;
+  if (blocks < 1) blocks = 1;
+  if (blocks > 148 * 16) blocks = 148 * 16;
+  return (unsigned)blocks;
+}
+
+extern "C" int cnb_add_noise(const float* x_ref, const float* z, float* out, long long n, float sqrt_acp,
+                             float sqrt_one_minus, uint64_t seed, uint64_t step, uint64_t elem_offset,
+                             cnb_stream_t s) {
+  CNB_REQUIRE(n > 0 && x_ref && out, "add_noise: null pointer or n=%lld", n);
+  CNB_REQUIRE((((uintptr_t)x_ref | (uintptr_t)z | (uintptr_t)out) & 15) == 0,
+              "add_noise: pointers must be 16-byte aligned");
+  CNB_REQUIRE(x_ref == out || !cnb_overlaps(x_ref, out, n), "add_noise: out must be x_ref or not overlap it");
+  add_noise_kernel<<<elementwise4_blocks(n), 256, 0, (cudaStream_t)s>>>(x_ref, z, out, n, sqrt_acp, sqrt_one_minus,
+                                                                      seed, step, elem_offset);
+  CNB_LAUNCH_CHECK();
+  return CNB_OK;
+}
+
+extern "C" int cnb_inpaint_blend(float* x, const float* x_ref, const float* mask, const float* z, long long n, int C,
+                                 long long HW, int mask_c, const float* levels, long long step,
+                                 const int32_t* step_dev, uint64_t seed, uint64_t noise_step, uint64_t elem_offset,
+                                 cnb_stream_t s) {
+  CNB_REQUIRE(n > 0 && x && x_ref && mask && levels, "inpaint_blend: null pointer or n=%lld", n);
+  CNB_REQUIRE(C > 0 && HW > 0 && n % ((long long)C * HW) == 0 && (mask_c == 1 || mask_c == C) &&
+                  (step_dev || step >= 0),
+              "inpaint_blend: bad dims n=%lld C=%d HW=%lld mask_c=%d step=%lld", n, C, HW, mask_c, step);
+  const long long n_mask = n / C * mask_c;
+  CNB_REQUIRE(!cnb_overlaps(x, x_ref, n) && !(mask < x + n && x < mask + n_mask),
+              "inpaint_blend: x must not overlap x_ref or mask");
+  CNB_REQUIRE((((uintptr_t)x | (uintptr_t)x_ref | (uintptr_t)mask | (uintptr_t)z) & 15) == 0,
+              "inpaint_blend: pointers must be 16-byte aligned");
+  inpaint_blend_kernel<<<elementwise4_blocks(n), 256, 0, (cudaStream_t)s>>>(
+      x, x_ref, mask, z, n, C, HW, mask_c, levels, step, step_dev, seed, noise_step, elem_offset);
+  CNB_LAUNCH_CHECK();
+  return CNB_OK;
+}
+
+extern "C" int cnb_mask_max_pool(const float* in, float* out, int B, int H, int W, int f, cnb_stream_t s) {
+  CNB_REQUIRE(in && out && B > 0 && f > 0 && H > 0 && W > 0 && H % f == 0 && W % f == 0,
+              "mask_max_pool: bad args B=%d H=%d W=%d f=%d", B, H, W, f);
+  const long long total = (long long)B * (H / f) * (W / f);
+  CNB_REQUIRE(!cnb_overlaps(in, out, (long long)B * H * W), "mask_max_pool: out must not overlap in");
+  mask_max_pool_kernel<<<blocks_for(total, 256), 256, 0, (cudaStream_t)s>>>(in, out, total, H, W, f);
   CNB_LAUNCH_CHECK();
   return CNB_OK;
 }

@@ -291,6 +291,58 @@ def dpm_solver_step(xt, eps, coef, z=None, want_x0=True, clip_sample=False, seed
     return prev, x0
 
 
+def _f32(name, *tensors):
+    for t in tensors:
+        if t is not None and (t.dtype != torch.float32 or not t.is_contiguous()):
+            raise rt.CnbError(f"{name}: expected contiguous fp32 tensors")
+
+
+def add_noise(x_ref, sqrt_acp, sqrt_one_minus, z=None, seed=0, step=0, elem_offset=0, out=None):
+    """sqrt_acp * x_ref + sqrt_one_minus * z (cnb_add_noise): LinearNoiseScheduler.add_noise bit for bit with its fp32
+    table values at t.  z=None draws the Philox stream (seed, step, elem_offset + i); out may be x_ref."""
+    rt.require_cuda(x_ref, z, out)
+    out = torch.empty_like(x_ref) if out is None else out
+    _f32("add_noise", x_ref, z, out)
+    if (z is not None and z.numel() != x_ref.numel()) or out.numel() != x_ref.numel():
+        raise rt.CnbError("add_noise: z and out must have x_ref's number of elements")
+    rt.check(rt.lib().cnb_add_noise(x_ref.data_ptr(), rt.ptr(z), out.data_ptr(), x_ref.numel(), float(sqrt_acp),
+                                    float(sqrt_one_minus), seed, step, elem_offset, rt.stream()))
+    return out
+
+
+def inpaint_blend(x, x_ref, mask, levels, step=0, step_dev=None, z=None, seed=0, noise_step=0, elem_offset=0):
+    """In place on x (NCHW fp32): x = m * x + (1 - m) * (a * x_ref + s * z) with (a, s) = levels[k], k = step_dev[0]
+    or step (cnb_inpaint_blend; m == 1 keeps x, m == 0 writes the noised reference exactly).  mask is [B, 1, H, W] or
+    [B, C, H, W], 1 = generate, 0 = keep the reference.  z=None draws the Philox stream (seed, noise_step,
+    elem_offset + i).  Returns x."""
+    rt.require_cuda(x, x_ref, mask, levels, step_dev, z)
+    _f32("inpaint_blend", x, x_ref, mask, levels, z)
+    B, C, H, W = x.shape
+    if tuple(x_ref.shape) != tuple(x.shape) or (z is not None and tuple(z.shape) != tuple(x.shape)):
+        raise rt.CnbError("inpaint_blend: x_ref and z must have x's shape")
+    if mask.dim() != 4 or tuple(mask.shape) not in ((B, 1, H, W), (B, C, H, W)):
+        raise rt.CnbError(f"inpaint_blend: mask must be [{B}, 1 or {C}, {H}, {W}] (got {tuple(mask.shape)})")
+    if levels.dim() != 2 or levels.shape[1] != 2 or (step_dev is None and not 0 <= int(step) < levels.shape[0]):
+        raise rt.CnbError("inpaint_blend: levels must be [n_steps, 2] and step one of its rows")
+    rt.check(rt.lib().cnb_inpaint_blend(x.data_ptr(), x_ref.data_ptr(), mask.data_ptr(), rt.ptr(z), x.numel(), C,
+                                        H * W, mask.shape[1], levels.data_ptr(), int(step), rt.ptr(step_dev), seed,
+                                        noise_step, elem_offset, rt.stream()))
+    return x
+
+
+def mask_max_pool(mask, f):
+    """[B, C, H, W] -> [B, C, H / f, W / f], the maximum over each f x f window (cnb_mask_max_pool): an image-space
+    inpainting mask on the latent grid, where a latent cell touching any repainted pixel is repainted."""
+    rt.require_cuda(mask)
+    _f32("mask_max_pool", mask)
+    B, C, H, W = mask.shape
+    if f < 1 or H % f or W % f:
+        raise rt.CnbError(f"mask_max_pool: H={H} and W={W} must be divisible by f={f}")
+    out = torch.empty((B, C, H // f, W // f), device=mask.device, dtype=torch.float32)
+    rt.check(rt.lib().cnb_mask_max_pool(mask.data_ptr(), out.data_ptr(), B * C, H, W, f, rt.stream()))
+    return out
+
+
 def philox_normal(shape, device, seed, step, elem_offset=0):
     out = torch.empty(shape, device=device, dtype=torch.float32)
     rt.require_cuda(out)

@@ -66,6 +66,10 @@ _SIGS = {
                               c_void_p, c_u64, c_void_p]),
     "cnb_dpm_solver_step": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_ll, c_void_p, c_int,
                                     c_u64, c_u64, c_void_p, c_u64, c_void_p]),
+    "cnb_add_noise": (c_int, [c_void_p, c_void_p, c_void_p, c_ll, c_float, c_float, c_u64, c_u64, c_u64, c_void_p]),
+    "cnb_inpaint_blend": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_ll, c_int, c_ll, c_int, c_void_p, c_ll,
+                                  c_void_p, c_u64, c_u64, c_u64, c_void_p]),
+    "cnb_mask_max_pool": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "cnb_philox_normal": (c_int, [c_void_p, c_ll, c_u64, c_u64, c_u64, c_void_p]),
     "cnb_gather_row": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
     "cnb_sampler_prologue": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),

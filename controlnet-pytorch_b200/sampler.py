@@ -15,12 +15,19 @@ what a captured step depends on, and `new_state(x)`, the dict of per-run device 
 next (DPM-Solver++'s previous data prediction; empty for DDPM and DDIM) that the sampler allocates once per run, or
 once per captured graph, and passes to every `update`.  With steps=None the schedule is the scheduler's own (all T
 timesteps for DDPM, num_inference_steps for the strided schedulers).
+
+Image-to-image and inpainting (`img2img`) run the tail of the schedule, `timesteps(steps, skip)` with
+skip = strength_to_skip(S, strength), from the reference noised to its first timestep (cnb_add_noise, outside the
+graph).  With a mask the captured step gains one launch after the update, cnb_inpaint_blend, which puts the known
+region back at the noise level of the next timestep.  The noise z of the start and of every blend is the x_T stream
+(seed, _XT_STEP, global element): fixed over the run, like diffusers' legacy inpainting, and drawn in the kernels.
 """
 
 import torch
 
 from . import ops
 from . import runtime as rt
+from .scheduler.schedule import noise_levels, strength_to_skip
 
 _XT_STEP = (1 << 40)   # Philox "step" reserved for drawing x_T
 
@@ -35,15 +42,62 @@ class DDPMSampler:
     def draw_xT(self, shape, device, elem_offset=0):
         return ops.philox_normal(shape, device, self.seed, _XT_STEP, elem_offset)
 
+    # ---- image-to-image start ----------------------------------------------------------------------------
+    def _base(self):
+        """The LinearNoiseScheduler whose tables define the noise levels (a strided scheduler's `base`)."""
+        return getattr(self.scheduler, "base", self.scheduler)
+
+    def _img2img_args(self, x_ref, mask, strength, steps):
+        """(x_ref, mask, skip) checked: x_ref contiguous fp32, the mask fp32 (bool converted once), [B, 1 or C, H, W]
+        with values in [0, 1] (one check per call, outside the loop), skip from strength."""
+        rt.require_cuda(x_ref, mask)
+        if x_ref.dtype != torch.float32 or x_ref.dim() != 4:
+            raise rt.CnbError("img2img: the reference must be a fp32 NCHW tensor")
+        x_ref = x_ref.contiguous()
+        if mask is not None:
+            if mask.dtype == torch.bool:
+                mask = mask.float()
+            B, C, H, W = x_ref.shape
+            if mask.dtype != torch.float32 or mask.dim() != 4 or tuple(mask.shape) not in ((B, 1, H, W), (B, C, H, W)):
+                raise rt.CnbError(f"img2img: the mask must be fp32 or bool, shaped [{B}, 1 or {C}, {H}, {W}] "
+                                  f"(got {mask.dtype} {tuple(mask.shape)})")
+            mask = mask.contiguous()
+            if not bool(((mask >= 0) & (mask <= 1)).all()):
+                raise rt.CnbError("img2img: mask values must lie in [0, 1] (1 = generate, 0 = keep the reference)")
+        return x_ref, mask, strength_to_skip(len(self.scheduler.timesteps(steps)), strength)
+
+    def _noised_start(self, x_ref, t, z, elem_offset, out=None):
+        """add_noise(x_ref, z, t) with the base scheduler's fp32 values at t; z=None is the x_T stream."""
+        b = self._base()
+        return ops.add_noise(x_ref, float(b.sqrt_alpha_cum_prod[t]), float(b.sqrt_one_minus_alpha_cum_prod[t]), z=z,
+                             seed=self.seed, step=_XT_STEP, elem_offset=elem_offset, out=out)
+
     # ---- eager loop (injected z, parity tests, per-step callbacks) ----------------------------------------
     @torch.no_grad()
-    def sample_eager(self, x_T, hint, steps=None, zs=None, elem_offset=0, callback=None):
+    def sample_eager(self, x_T, hint, steps=None, zs=None, elem_offset=0, callback=None, x_ref=None, mask=None,
+                     strength=1.0):
+        """The loop without a graph; returns (x, x0).  With `x_ref` it is img2img's loop (see there): it starts from
+        add_noise(x_ref, z, tau_skip) and, with `mask`, blends after every step, where z is x_T when given (injected
+        noise) and otherwise the x_T stream."""
         sch = self.scheduler
-        ts = sch.timesteps(steps)
-        table = sch.coef_table(x_T.device, steps)
-        xt, x0 = x_T.contiguous(), None
+        skip, levels = 0, None
+        if x_ref is None and mask is not None:
+            raise rt.CnbError("sample_eager: a mask needs the reference x_ref")
+        if x_ref is not None:
+            x_ref, mask, skip = self._img2img_args(x_ref, mask, strength, steps)
+        ts = sch.timesteps(steps, skip)
+        dev = (x_T if x_ref is None else x_ref).device
+        table = sch.coef_table(dev, steps, skip)
+        if x_ref is None:
+            xt = x_T.contiguous()
+        else:
+            z0 = None if x_T is None else x_T.contiguous()
+            xt = self._noised_start(x_ref, ts[0], z0, elem_offset)
+            if mask is not None:
+                levels = noise_levels(self._base(), ts).to(dev)
+        x0 = None
         state = sch.new_state(xt)
-        t_dev = torch.empty((1,), device=x_T.device, dtype=torch.int64)
+        t_dev = torch.empty((1,), device=dev, dtype=torch.int64)
         for k, t in enumerate(ts):
             t_dev.fill_(t)
             eps = self.model(xt, t_dev, hint)
@@ -51,6 +105,9 @@ class DDPMSampler:
             z = zs[k].to(xt.device) if (zs is not None and k < len(ts) - 1) else None
             xt, x0 = sch.update(xt, eps, table[t], z=z, want_x0=True, seed=self.seed, step=k,
                                 elem_offset=elem_offset, **state)
+            if levels is not None:
+                ops.inpaint_blend(xt, x_ref, mask, levels, step=k, z=z0, seed=self.seed, noise_step=_XT_STEP,
+                                  elem_offset=elem_offset)
             if callback is not None:
                 callback(t, xt, x0)
         return xt, x0
@@ -69,7 +126,7 @@ class DDPMSampler:
             return
         fn(self._hint, rt.get_mode())
 
-    def _capture(self, x_T, hint, steps, elem_offset):
+    def _capture(self, x_T, hint, steps, elem_offset, skip=0, x_ref=None, mask=None):
         dev = x_T.device
         sch = self.scheduler
         self.xt = x_T.clone().contiguous()
@@ -77,15 +134,19 @@ class DDPMSampler:
         self._hint = hint.clone().contiguous()
         hint = self._hint
         self.x0 = torch.empty_like(self.xt)
-        ts = sch.timesteps(steps)
+        ts = sch.timesteps(steps, skip)
         self.t_seq = torch.tensor(ts, dtype=torch.int64).to(dev)
         self.step_idx = torch.zeros((1,), device=dev, dtype=torch.int32)
         self.t_out = torch.zeros((1,), device=dev, dtype=torch.int64)
         self.coef = torch.zeros((6,), device=dev, dtype=torch.float32)
-        table = sch.coef_table(dev, steps)
+        table = sch.coef_table(dev, steps, skip)
         self._table = table          # the graph reads it: kept alive, so no other table can take its address
         self._state = sch.new_state(self.xt)   # carried across replays: owned by the sampler, as long as the graph
         state = self._state
+        # inpainting: the reference, the mask and the noise-level table the blend reads, owned like the hint
+        self._xref = None if mask is None else x_ref.clone()
+        self._mask = None if mask is None else mask.clone()
+        self._levels = None if mask is None else noise_levels(self._base(), ts).to(dev)
         L = rt.lib()
 
         def one_step():
@@ -94,6 +155,9 @@ class DDPMSampler:
             eps = self.model(self.xt, self.t_out, hint)
             sch.update(self.xt, eps, self.coef, z=None, seed=self.seed, step_dev=self.step_idx,
                        elem_offset=elem_offset, out=self.xt, x0_out=self.x0, **state)
+            if mask is not None:
+                ops.inpaint_blend(self.xt, self._xref, self._mask, self._levels, step_dev=self.step_idx,
+                                  seed=self.seed, noise_step=_XT_STEP, elem_offset=elem_offset)
             rt.check(L.cnb_bump_index(self.step_idx.data_ptr(), 1, rt.stream()))
 
         # warm-up on a side stream: builds weight / hint caches and sets kernel attributes outside the capture
@@ -119,25 +183,59 @@ class DDPMSampler:
         """Run the scheduler's timesteps (DDPM: t = steps-1 .. 0, SURVEY.md 3.5 semantics) with fused on-device noise;
         returns (x after the last step, x0)."""
         rt.require_cuda(x_T, hint)
-        sch = self.scheduler
         if not self.use_graph:
             return self.sample_eager(x_T, hint, steps, None, elem_offset)
         if hint.shape[0] != x_T.shape[0]:
             raise rt.CnbError("sample: x_T and hint must have the same batch size")
-        # the table's address tells apart schedulers with equal graph keys but other beta schedules
-        key = (tuple(x_T.shape), tuple(hint.shape), sch.graph_key(steps), sch.coef_table(x_T.device, steps).data_ptr(),
-               elem_offset, rt.get_mode(), str(x_T.device), self._param_stamp())
+        self._prepare(x_T, hint, steps, elem_offset)
+        self.xt.copy_(x_T)
+        return self._run()
+
+    def _prepare(self, x_T, hint, steps, elem_offset, skip=0, x_ref=None, mask=None):
+        """Capture the step graph, or refresh the sampler-owned buffers of the one that fits."""
+        sch = self.scheduler
+        # the table's address tells apart schedulers with equal graph keys but other beta schedules; the noise-level
+        # table is sampler-owned and refreshed below, so its values need no key
+        key = (tuple(x_T.shape), tuple(hint.shape), sch.graph_key(steps, skip),
+               sch.coef_table(x_T.device, steps, skip).data_ptr(), elem_offset, rt.get_mode(), str(x_T.device),
+               self._param_stamp(), skip, None if mask is None else tuple(mask.shape))
         if self._graph is None or key != self._key:
-            self._capture(x_T, hint, steps, elem_offset)
+            self._capture(x_T, hint, steps, elem_offset, skip, x_ref, mask)
             self._key = key
         else:
             self._hint.copy_(hint)
             self._refresh_hint()
-        self.xt.copy_(x_T)
+            if mask is not None:
+                self._xref.copy_(x_ref)
+                self._mask.copy_(mask)
+                self._levels.copy_(noise_levels(self._base(), sch.timesteps(steps, skip)))
+
+    def _run(self):
         self.replay_steps(self._nsteps, reset=True)
         out = self.xt.clone(), self.x0.clone()
         check_device_errors()
         return out
+
+    @torch.no_grad()
+    def img2img(self, x_ref, hint, strength=1.0, mask=None, steps=None, elem_offset=0):
+        """Image-to-image (SDEdit) and inpainting under the hint; returns (x, x0).
+        The run keeps the last n = min(S, int(S * strength)) of the S timesteps of `timesteps(steps)`
+        (scheduler.schedule.strength_to_skip) and starts from add_noise(x_ref, z, tau_skip), z the x_T stream
+        (seed, _XT_STEP, global element index); step k of the tail draws its noise like step k of a plain run over the
+        same tail.  `mask` ([B, 1 or C, H, W], fp32 or bool; 1 = generate, 0 = keep the reference) adds one launch to
+        the captured step: after step k the elements with m = 0 are add_noise(x_ref, z, tau_{k+1}) with the same z,
+        x_ref exactly after the last step, and soft values blend m * x + (1 - m) * known.  The returned x is blended;
+        x0 is the update's own prediction of the last step, before the blend."""
+        rt.require_cuda(x_ref, hint)
+        if not self.use_graph:
+            return self.sample_eager(None, hint, steps, None, elem_offset, x_ref=x_ref, mask=mask, strength=strength)
+        x_ref, mask, skip = self._img2img_args(x_ref, mask, strength, steps)
+        if hint.shape[0] != x_ref.shape[0]:
+            raise rt.CnbError("img2img: x_ref and hint must have the same batch size")
+        ts = self.scheduler.timesteps(steps, skip)
+        self._prepare(x_ref, hint, steps, elem_offset, skip, x_ref, mask)
+        self._noised_start(x_ref, ts[0], None, elem_offset, out=self.xt)
+        return self._run()
 
     def replay_steps(self, n, reset=True):
         """bench.py hook: replay the captured step n times (state continues from wherever it is)."""
@@ -180,6 +278,37 @@ class LDMSampler(DDPMSampler):
             xt, _ = self.sample_eager(x_T, hint, steps, zs, elem_offset)
         else:
             xt, _ = self.sample(x_T, hint, steps=steps, elem_offset=elem_offset)
+        return self.decode(xt, to_unit_range), xt
+
+    @torch.no_grad()
+    def encode_mean(self, images):
+        """Latents of images in [-1, 1]: the VAE posterior mean, the first z_channels channels of the encoder output.
+        Deterministic, unlike the reference's `encode`, which samples the posterior with CPU noise."""
+        rt.require_cuda(images)
+        return self.vae._encode_out(images.contiguous(), rt.get_mode())[:, :self.vae.z_channels].contiguous()
+
+    def latent_mask(self, mask, latents):
+        """An image-space mask [B, 1, H, W] (fp32 or bool) on the latent grid of `latents`: the maximum over each
+        f x f window (cnb_mask_max_pool), so a latent cell touching any repainted pixel is repainted."""
+        rt.require_cuda(mask)
+        if mask.dtype == torch.bool:
+            mask = mask.float()
+        if mask.dim() != 4 or mask.shape[0] != latents.shape[0] or mask.shape[1] != 1:
+            raise rt.CnbError(f"img2img_images: the image-space mask must be [B, 1, H, W] (got {tuple(mask.shape)})")
+        f = mask.shape[2] // latents.shape[2]
+        if f < 1 or mask.shape[2] != f * latents.shape[2] or mask.shape[3] != f * latents.shape[3]:
+            raise rt.CnbError(f"img2img_images: mask {tuple(mask.shape[2:])} is not a multiple of the latent grid "
+                              f"{tuple(latents.shape[2:])}")
+        return ops.mask_max_pool(mask.contiguous(), f)
+
+    @torch.no_grad()
+    def img2img_images(self, images, hint, strength=1.0, mask=None, steps=None, elem_offset=0, to_unit_range=True):
+        """img2img on the latents of `images` ([-1, 1], encoded to the posterior mean) with an image-space `mask`
+        pooled to the latent grid; returns (decoded images, final latents).  The known LATENT region is exact; the
+        decoded pixels of the kept region are not (there is no paste-back after decode)."""
+        lat = self.encode_mean(images)
+        lmask = None if mask is None else self.latent_mask(mask, lat)
+        xt, _ = self.img2img(lat, hint, strength=strength, mask=lmask, steps=steps, elem_offset=elem_offset)
         return self.decode(xt, to_unit_range), xt
 
 
@@ -257,7 +386,7 @@ def shard_bounds(total, world, rank):
 
 @torch.no_grad()
 def sample_data_parallel(model, scheduler, shape, hint_fn, steps=None, seed=0, group=None, use_graph=True,
-                         gather=True, vae=None, sampler=None, x_T_fn=None):
+                         gather=True, vae=None, sampler=None, x_T_fn=None, x_ref_fn=None, mask_fn=None, strength=1.0):
     """One job over all ranks of `group` (tools/sample_ddpm_controlnet.py:21-51 sharded over the GPUs of a box): rank r
     draws (or receives) and denoises samples [lo, hi) of the global batch `shape[0]`, no collective inside the
     timestep loop, and the final samples are all-gathered ONCE (NCCL over NVLink).
@@ -265,7 +394,9 @@ def sample_data_parallel(model, scheduler, shape, hint_fn, steps=None, seed=0, g
     `x_T_fn(lo, hi)`, when given, supplies the shard's initial noise the same way (the reference draws x_T on the host,
     :26-29); otherwise x_T is Philox noise keyed by the GLOBAL element index, independent of the number of ranks.
     `sampler` re-uses a DDPMSampler / LDMSampler (and its captured step graph) across calls.  With `vae` the shard's
-    final latents are decoded locally (LDM path) and the images are what is gathered."""
+    final latents are decoded locally (LDM path) and the images are what is gathered.
+    `x_ref_fn(lo, hi)` (and `mask_fn(lo, hi)`), mirroring hint_fn, make the job img2img (inpainting) at `strength`:
+    they return the shard's references and masks, images and image-space masks with `vae` (encoded locally)."""
     import torch.distributed as dist
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     rank = dist.get_rank(group) if dist.is_initialized() else 0
@@ -279,13 +410,26 @@ def sample_data_parallel(model, scheduler, shape, hint_fn, steps=None, seed=0, g
     if smp is None:
         smp = (DDPMSampler(model, scheduler, seed=seed, use_graph=use_graph) if vae is None else
                LDMSampler(model, scheduler, vae, seed=seed, use_graph=use_graph))
-    if x_T_fn is not None:
-        x_T = x_T_fn(lo, hi)
+    if x_T_fn is not None and x_ref_fn is not None:
+        raise rt.CnbError("sample_data_parallel: x_T_fn and x_ref_fn exclude each other (img2img starts from x_ref)")
+    if mask_fn is not None and x_ref_fn is None:
+        raise rt.CnbError("sample_data_parallel: mask_fn needs x_ref_fn")
+    if x_ref_fn is not None:
+        mask = None if mask_fn is None else mask_fn(lo, hi)
+        if vae is not None:
+            xt, _ = smp.img2img_images(x_ref_fn(lo, hi), hint_fn(lo, hi), strength=strength, mask=mask, steps=steps,
+                                       elem_offset=lo * per)
+        else:
+            xt, _ = smp.img2img(x_ref_fn(lo, hi), hint_fn(lo, hi), strength=strength, mask=mask, steps=steps,
+                                elem_offset=lo * per)
     else:
-        x_T = smp.draw_xT((hi - lo,) + tuple(shape[1:]), dev, elem_offset=lo * per)
-    xt, x0 = smp.sample(x_T, hint_fn(lo, hi), steps=steps, elem_offset=lo * per)
-    if vae is not None:
-        xt = smp.decode(xt)
+        if x_T_fn is not None:
+            x_T = x_T_fn(lo, hi)
+        else:
+            x_T = smp.draw_xT((hi - lo,) + tuple(shape[1:]), dev, elem_offset=lo * per)
+        xt, x0 = smp.sample(x_T, hint_fn(lo, hi), steps=steps, elem_offset=lo * per)
+        if vae is not None:
+            xt = smp.decode(xt)
     if not gather or world == 1:
         return xt
     return gather_shards(xt, B, group)

@@ -19,7 +19,7 @@ import torch
 
 from .. import ops
 from .. import runtime as rt
-from .schedule import strided_timesteps
+from .schedule import strided_timesteps, tail
 
 
 class DDIMScheduler:
@@ -46,10 +46,11 @@ class DDIMScheduler:
             raise rt.CnbError(f"DDIMScheduler: eta must be a finite number >= 0 (got {self.eta!r})")
         return eta
 
-    def timesteps(self, steps=None):
-        """tau_0 > ... > tau_{S-1} as a tuple of ints; `steps` overrides num_inference_steps."""
-        return strided_timesteps("DDIMScheduler", self.num_timesteps, self.num_inference_steps, self.spacing,
-                                 self.explicit_timesteps, steps)
+    def timesteps(self, steps=None, skip=0):
+        """tau_0 > ... > tau_{S-1} as a tuple of ints; `steps` overrides num_inference_steps; the tail without the first
+        `skip` timesteps (0 <= skip < S) with skip > 0."""
+        return tail("DDIMScheduler", strided_timesteps("DDIMScheduler", self.num_timesteps, self.num_inference_steps,
+                                                       self.spacing, self.explicit_timesteps, steps), skip)
 
     def coef_table_host(self, steps=None):
         """fp32 [T, 6]: row tau_k is row_k of the module docstring; rows off the schedule are NaN, so that reading one
@@ -70,15 +71,18 @@ class DDIMScheduler:
             tab[t, 5] = 1.0 if sigma > 0.0 else 0.0
         return tab
 
-    def coef_table(self, device, steps=None):
+    def coef_table(self, device, steps=None, skip=0):
+        """The device copy of coef_table_host.  A row depends only on its own timestep and the next one, so the tail
+        of `skip` (validated) reads the same table at the same rows."""
+        self.timesteps(steps, skip)
         key = (str(device), self.timesteps(steps), self._eta())
         if key not in self._coef:
             self._coef[key] = self.coef_table_host(steps).to(device)
         return self._coef[key]
 
-    def graph_key(self, steps=None):
+    def graph_key(self, steps=None, skip=0):
         """Everything a captured sampling step depends on besides the model and the coefficient table."""
-        return ("ddim", self.timesteps(steps), self._eta(), bool(self.clip_sample))
+        return ("ddim", self.timesteps(steps, skip), self._eta(), bool(self.clip_sample))
 
     def new_state(self, x):
         """DDIM carries nothing from one step to the next."""

@@ -227,6 +227,33 @@ int cnb_ddim_step(const float* xt, const float* eps, const float* z, float* xt_p
 int cnb_dpm_solver_step(const float* xt, const float* eps, const float* z, float* hist, float* xt_prev, float* x0,
                         long long n, const float* coef, int clip_sample, uint64_t seed, uint64_t step,
                         const int32_t* step_dev, uint64_t elem_offset, cnb_stream_t stream);
+/*
+ * Image-to-image start (sampler.DDPMSampler.img2img; the forward diffusion of LinearNoiseScheduler.add_noise).  Per
+ * element, fp32, no FMA contraction, in add_noise's operation order (mul, mul, add):
+ *   out = sqrt_acp * x_ref + sqrt_one_minus * z
+ * so with the base scheduler's fp32 sqrt_alpha_cum_prod[t] / sqrt_one_minus_alpha_cum_prod[t] the result is
+ * add_noise(x_ref, z, t) bit for bit.  z == NULL draws the Philox stream of cnb_sched_step keyed by
+ * (seed, step, elem_offset + i).  out may alias x_ref (and must not overlap it otherwise).  16-byte aligned pointers.
+ */
+int cnb_add_noise(const float* x_ref, const float* z, float* out, long long n, float sqrt_acp, float sqrt_one_minus,
+                  uint64_t seed, uint64_t step, uint64_t elem_offset, cnb_stream_t stream);
+/*
+ * Inpainting blend (sampler.DDPMSampler.img2img with a mask), in place on x (NCHW fp32, n = B * C * HW elements).
+ * k = step_dev ? step_dev[0] : step selects row k of levels, a device fp32 [n_steps, 2] table, as (a, s).  Per element,
+ * fp32, separate IEEE operations:
+ *   known = a * x_ref + s * z                      (cnb_add_noise's operation order)
+ *   x     = m == 1 ? x : (m == 0 ? known : (m * x) + ((1 - m) * known))
+ * so m == 1 leaves x unchanged bit for bit and m == 0 writes known exactly.  m is mask[b, c, p] with mask shaped
+ * [B, mask_c, HW] and mask_c == C, or mask[b, 0, p] with mask_c == 1 (broadcast over the channels).  1 means
+ * "generate", 0 means "keep the reference".  z == NULL draws the Philox stream keyed by (seed, noise_step,
+ * elem_offset + i).  x must not overlap x_ref or mask; 16-byte aligned pointers.
+ */
+int cnb_inpaint_blend(float* x, const float* x_ref, const float* mask, const float* z, long long n, int C,
+                      long long HW, int mask_c, const float* levels, long long step, const int32_t* step_dev,
+                      uint64_t seed, uint64_t noise_step, uint64_t elem_offset, cnb_stream_t stream);
+/* out[p, oy, ox] = max over in[p, oy*f + dy, ox*f + dx], 0 <= dy, dx < f, for B planes of H x W (H and W divisible by
+ * f): an image-space inpainting mask on the latent grid, a latent cell touching any repainted pixel repainted. */
+int cnb_mask_max_pool(const float* in, float* out, int B, int H, int W, int f, cnb_stream_t stream);
 /* Fill out[i] with the same N(0,1) stream as cnb_sched_step (used for x_T and by tests). */
 int cnb_philox_normal(float* out, long long n, uint64_t seed, uint64_t step, uint64_t elem_offset,
                       cnb_stream_t stream);
