@@ -503,6 +503,24 @@ __global__ void edm_combine_to_nchw_kernel(const float* __restrict__ cskip, cons
   dst[i] = __fadd_rn(__fmul_rn(cskip[b], x[i]), __fmul_rn(cout[b], fv));
 }
 
+// Hint guidance (models/_controlnet_common.controlnet_forward with guidance=w): the two conv_out outputs leave the
+// channels-last workspace (fp32 or fp16, leading dimensions ldc / ldu) as eps = eu + w * (ec - eu) in NCHW fp32.  Sub,
+// mul, add as separate IEEE operations (no FMA contraction): bit-identical to that fp32 expression evaluated on the
+// two cnb_nhwc_to_nchw results.
+template <typename T>
+__global__ void guidance_combine_kernel(const T* __restrict__ hc, int ldc, const T* __restrict__ hu, int ldu,
+                                        float* __restrict__ dst, int C, int HW, float w, long long total) {
+  long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;   // index over (b, c, p): p fastest
+  if (i >= total) return;
+  int pix = (int)(i % HW);
+  long long bc = i / HW;
+  int c = (int)(bc % C);
+  long long q = (bc / C) * HW + pix;
+  const float ec = (float)hc[q * ldc + c];
+  const float eu = (float)hu[q * ldu + c];
+  dst[i] = __fadd_rn(eu, __fmul_rn(w, __fsub_rn(ec, eu)));
+}
+
 template <typename T>
 __global__ void copy_channels_kernel(const T* __restrict__ src, int lds, int s_coff, T* __restrict__ dst,
                                      int ldd, int d_coff, int C, long long total) {
@@ -781,6 +799,32 @@ extern "C" int cnb_edm_combine_to_nchw(const float* c_skip, const float* x, cons
   else
     edm_combine_to_nchw_kernel<float><<<blocks_for(total, 256), 256, 0, (cudaStream_t)s>>>(
         c_skip, x, c_out, reinterpret_cast<const float*>(f), ldi, in_coff, dst, C, HW, total);
+  CNB_LAUNCH_CHECK();
+  return CNB_OK;
+}
+
+extern "C" int cnb_guidance_combine(const void* h_c, int ldc, const void* h_u, int ldu, float* dst, int B, int C,
+                                    int HW, float w, int src_f16, cnb_stream_t s) {
+  const long long total = (long long)B * C * HW;
+  CNB_REQUIRE(h_c && h_u && dst && B > 0 && C > 0 && HW > 0 && ldc >= C && ldu >= C,
+              "guidance_combine: bad args B=%d C=%d HW=%d ldc=%d ldu=%d", B, C, HW, ldc, ldu);
+  const size_t elt = src_f16 ? 2 : 4;
+  CNB_REQUIRE((((uintptr_t)h_c | (uintptr_t)h_u) & (elt - 1)) == 0 && ((uintptr_t)dst & 3) == 0,
+              "guidance_combine: pointers must be aligned to their element size");
+  // byte ranges: the last element an input is read at is ((B * HW - 1) * ld + C - 1)
+  const char* o0 = reinterpret_cast<const char*>(dst);
+  const char* o1 = o0 + total * 4;
+  const char* c0 = reinterpret_cast<const char*>(h_c);
+  const char* c1 = c0 + ((long long)B * HW - 1) * ldc * elt + C * elt;
+  const char* u0 = reinterpret_cast<const char*>(h_u);
+  const char* u1 = u0 + ((long long)B * HW - 1) * ldu * elt + C * elt;
+  CNB_REQUIRE(!(o0 < c1 && c0 < o1) && !(o0 < u1 && u0 < o1), "guidance_combine: out must not overlap h_c or h_u");
+  if (src_f16)
+    guidance_combine_kernel<__half><<<blocks_for(total, 256), 256, 0, (cudaStream_t)s>>>(
+        reinterpret_cast<const __half*>(h_c), ldc, reinterpret_cast<const __half*>(h_u), ldu, dst, C, HW, w, total);
+  else
+    guidance_combine_kernel<float><<<blocks_for(total, 256), 256, 0, (cudaStream_t)s>>>(
+        reinterpret_cast<const float*>(h_c), ldc, reinterpret_cast<const float*>(h_u), ldu, dst, C, HW, w, total);
   CNB_LAUNCH_CHECK();
   return CNB_OK;
 }

@@ -77,7 +77,11 @@ class _Branches:
                 tns.record_stream(self.cur)
 
 
-def controlnet_forward(trained, control, down_zero, mid_zero, hint_feat_fn, x, t, hint):
+def controlnet_forward(trained, control, down_zero, mid_zero, hint_feat_fn, x, t, hint, scale=1.0, guidance=None):
+    """eps of the ControlNet.  `scale` multiplies the down and mid zero convolutions (conditioning scale): the result is
+    that of a copy of the model whose zero-conv weights and biases were multiplied by `scale` (E.scaled_conv).  With
+    `guidance` = w the frozen U-Net also runs without the control branch, sharing the encoder and mids[0], and
+    eps = eu + w * (ec - eu) (hint guidance, cnb_guidance_combine)."""
     x = E._check_x(x)
     hint = E._check_x(hint)
     mode = rt.get_mode()
@@ -87,22 +91,36 @@ def controlnet_forward(trained, control, down_zero, mid_zero, hint_feat_fn, x, t
     hf = hint_feat_fn(hint, mode)
     nmid = len(control.mids)
 
+    def zero_conv(zc, c, **kw):
+        if scale == 1.0:
+            return E.conv16(c, zc.weight, "1x1", zc.out_channels, mode, bias=E.raw(zc.bias), **kw)
+        packed, packed_lp, bias = E.scaled_conv(zc, scale, mode)
+        return E.conv16(c, zc.weight, "1x1", zc.out_channels, mode, packed=packed, packed_lp=packed_lp, bias=bias,
+                        **kw)
+
     def skip_sums(cs, t_skips):
         """zero_conv_i(control skip) + trained skip, written into the second half of the decoder's concat buffers
         (controlnet.py:190-192, 216-218)."""
         cats = []
         for i, c in enumerate(cs):
             B, H, W, C = c.shape
-            zc = down_zero[i]
             cat = ops.empty(B, H, W, 2 * C, device=dev, dtype=c.dtype)
-            E.conv16(c, zc.weight, "1x1", C, mode, bias=E.raw(zc.bias), residual=t_skips[i], out=cat, out_coff=C)
+            zero_conv(down_zero[i], c, residual=t_skips[i], out=cat, out_coff=C)
             cats.append(cat)
         return cats
 
     def inject(i, a, cm):
         """a + mid_zero_conv_i(control mid output): the sum rides in the zero conv's epilogue (:207)."""
-        zc = mid_zero[i]
-        return E.conv16(cm, zc.weight, "1x1", zc.out_channels, mode, bias=E.raw(zc.bias), residual=a)
+        return zero_conv(mid_zero[i], cm, residual=a)
+
+    def uncond(a):
+        """The frozen U-Net's own rest from the output of trained.mids[0]: the plain path of E.run_unet_body."""
+        skips = list(t_skips)
+        for m in trained.mids[1:]:
+            a = E.run_mid(m, a, plan_t[m], mode)
+        for u in trained.ups:
+            a = E.run_up(u, a, skips.pop(), plan_t[u], mode)
+        return E.conv_out(trained, a, mode)
 
     # The dependency graph of the reference's forward is wider than its statement order: the frozen encoder AND
     # trained.mids[0] never read a control tensor; trained.mids[i] needs control.mids[i-1] only through mid zero conv
@@ -114,6 +132,7 @@ def controlnet_forward(trained, control, down_zero, mid_zero, hint_feat_fn, x, t
     #     side      : control conv_in + hint feature -> downs -> mids[0] -> mids[1]
     #     skip      : trained t-embedding rows; later wait(both encoders) -> the skip sums
     #     aux       : control t-embedding rows
+    #     uncond    : with guidance, wait(trained mids[0]) -> the frozen U-Net's mids[1:] -> ups -> conv_out
     # The critical path loses one mid block per mid level, the skip sums and the t-embedding launches (measured, MNIST:
     # step at 128 samples 2.42 -> 2.24 ms, at 1024 samples 11.98 -> 11.80 ms; CelebHQ LDM at 256: 28.25 -> 27.7 ms; DESIGN.md 5);
     # the kernels of one branch fill the pipes the other leaves idle (MUFU-bound attention next to tensor- / HBM-bound
@@ -150,12 +169,20 @@ def controlnet_forward(trained, control, down_zero, mid_zero, hint_feat_fn, x, t
         br.wait(ev_tenc, *t_skips)
         br.wait(ev_cenc, *cs)
         cats = skip_sums(cs, t_skips)
+    h_u = None
     for i in range(nmid):
         a = E.run_mid(trained.mids[i], a, plan_t[trained.mids[i]], mode)
+        if i == 0 and guidance is not None:
+            ev_a = br.record()
+            with br.on("uncond"):
+                br.wait(ev_a, a, next(iter(plan_t.values())).table, *t_skips)
+                h_u = uncond(a)
         br.wait(ev_mid[i], cms[i])
         a = inject(i, a, cms[i])
-    br.join(*cats)
+    br.join(*cats, *([] if h_u is None else [h_u]))
 
     for u in trained.ups:
         a = E.run_up(u, a, None, plan_t[u], mode, cat=cats.pop())
-    return ops.nhwc_to_nchw(E.conv_out(trained, a, mode))
+    if h_u is None:
+        return ops.nhwc_to_nchw(E.conv_out(trained, a, mode))
+    return ops.guidance_combine(E.conv_out(trained, a, mode), h_u, guidance)

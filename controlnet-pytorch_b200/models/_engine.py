@@ -33,11 +33,11 @@ def zero_(module):
 # ----------------------------------------------------------------------------------------------------------
 # derived weight cache
 # ----------------------------------------------------------------------------------------------------------
-def _cached(params, key, builder):
+def _cached(params, key, builder, tag=None):
     """builder()'s result, kept on params[0] under `key` and rebuilt when any of `params` is changed in place (version
-    counter) or replaced (data_ptr)."""
+    counter) or replaced (data_ptr), or when `tag` (what else the result depends on) changes: one entry per key."""
     store = params[0].__dict__.setdefault("_cnb_pack", {})
-    stamp = tuple((p._version, p.data_ptr()) for p in params)
+    stamp = tuple((p._version, p.data_ptr()) for p in params) + (tag,)
     ent = store.get(key)
     if ent is None or ent[0] != stamp:
         with torch.no_grad():
@@ -59,6 +59,27 @@ def packed_conv(param, mode):
 def packed_conv_f16(param):
     """fp16 copy of the packed (unrounded) weights: B operand of the kind::f16 convolution."""
     return _cached((param,), ("conv_f16",), lambda: ops.cast_f16(ops.pack_conv_weight(param, False)))
+
+
+SCALED = ("scaled",)      # the _cnb_pack key of scaled_conv's entry
+
+
+def scaled_conv(conv, s, mode):
+    """(packed, packed fp16, bias) of `conv` with weight s * W and bias s * b, each product one fp32 rounding: what
+    packed_conv / packed_conv_f16 / raw give for a copy of the layer whose parameters were multiplied by s.  One entry
+    per layer, replaced when s or the mode changes; a captured graph that read an entry keeps it alive through
+    `pinned_scaled`."""
+    def build():
+        w = conv.weight.detach() * s
+        r = mode != rt.MODE_F32 and _tc_shape(w.shape[0], w.shape[1])
+        return ops.pack_conv_weight(w, r), ops.cast_f16(ops.pack_conv_weight(w, False)), conv.bias.detach() * s
+    return _cached((conv.weight, conv.bias), SCALED, build, tag=(float(s), mode))
+
+
+def pinned_scaled(module):
+    """The live scaled_conv entries of every parameter of `module`."""
+    return [p.__dict__["_cnb_pack"][SCALED] for p in module.parameters()
+            if SCALED in p.__dict__.get("_cnb_pack", {})]
 
 
 def use_f16(mode, cin, cout):

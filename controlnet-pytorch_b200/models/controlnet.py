@@ -80,3 +80,10 @@ class ControlNet(nn.Module):
         """eps = ControlNet(x_t, t, hint); x (B,C,H,W), hint (B,hint_channels,H,W) fp32 CUDA; t int (1,) or (B,)."""
         return controlnet_forward(self.trained_unet, self.control_copy_unet, self.control_copy_unet_down_zero_convs,
                                   self.control_copy_unet_mid_zero_convs, self._hint_feat, x, t, hint)
+
+    def _forward_controlled(self, x, t, hint, scale=1.0, guidance=None):
+        """forward with a conditioning scale on the down / mid zero convolutions and, with guidance = w, hint guidance
+        eps = eu + w * (ec - eu) against the frozen U-Net (_controlnet_common.controlnet_forward).  Device tensors."""
+        return controlnet_forward(self.trained_unet, self.control_copy_unet, self.control_copy_unet_down_zero_convs,
+                                  self.control_copy_unet_mid_zero_convs, self._hint_feat, x, t, hint, scale=scale,
+                                  guidance=guidance)

@@ -83,3 +83,10 @@ class ControlNet(nn.Module):
     def forward(self, x, t, hint):
         return controlnet_forward(self.trained_unet, self.control_unet, self.control_unet_down_zero_convs,
                                   self.control_unet_mid_zero_convs, self._hint_feat, x, t, hint)
+
+    def _forward_controlled(self, x, t, hint, scale=1.0, guidance=None):
+        """forward with a conditioning scale on the down / mid zero convolutions and, with guidance = w, hint guidance
+        eps = eu + w * (ec - eu) against the frozen U-Net (_controlnet_common.controlnet_forward).  Device tensors."""
+        return controlnet_forward(self.trained_unet, self.control_unet, self.control_unet_down_zero_convs,
+                                  self.control_unet_mid_zero_convs, self._hint_feat, x, t, hint, scale=scale,
+                                  guidance=guidance)

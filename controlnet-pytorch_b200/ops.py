@@ -199,9 +199,7 @@ def nhwc_to_nchw(x, in_coff=0, c=None, out=None):
     `out`: a contiguous fp32 (B, c, H, W) tensor (e.g. a batch slice of a larger one) to write into."""
     rt.require_cuda(x)
     B, H, W, cv = x.shape
-    ld = x.stride(2)
-    if x.stride(3) != 1 or x.stride(1) != W * ld or x.stride(0) != H * W * ld or ld < cv:
-        raise rt.CnbError("nhwc_to_nchw: expected a channels-last tensor or a channel slice of one")
+    ld = _nhwc_ld(x, "nhwc_to_nchw")
     c = cv - in_coff if c is None else c
     if out is None:
         if c == 1 and ld == 1 and x.dtype == torch.float32:
@@ -211,6 +209,36 @@ def nhwc_to_nchw(x, in_coff=0, c=None, out=None):
         raise rt.CnbError("nhwc_to_nchw: out must be a contiguous fp32 (B, c, H, W) tensor")
     rt.check(rt.lib().cnb_nhwc_to_nchw(x.data_ptr(), ld, in_coff, out.data_ptr(), B, c, H * W,
                                        1 if x.dtype == torch.float16 else 0, rt.stream()))
+    return out
+
+
+def _nhwc_ld(x, name):
+    """Leading dimension of a channels-last tensor or of a channel-narrowed view of one."""
+    B, H, W, cv = x.shape
+    ld = x.stride(2)
+    if x.stride(3) != 1 or x.stride(1) != W * ld or x.stride(0) != H * W * ld or ld < cv:
+        raise rt.CnbError(f"{name}: expected a channels-last tensor or a channel slice of one")
+    return ld
+
+
+def guidance_combine(h_c, h_u, w, out=None):
+    """eps = eu + w * (ec - eu) in NCHW fp32 (cnb_guidance_combine), ec / eu what nhwc_to_nchw returns for h_c / h_u:
+    the ControlNet's and the frozen U-Net's channels-last outputs, both fp32 or both fp16, each contiguous or a
+    channel-narrowed view of a wider buffer.  `out`: a contiguous fp32 (B, C, H, W) tensor overlapping neither input."""
+    rt.require_cuda(h_c, h_u, out)
+    if h_c.dtype != h_u.dtype or h_c.dtype not in (torch.float32, torch.float16):
+        raise rt.CnbError(f"guidance_combine: h_c and h_u must both be fp32 or both fp16 (got {h_c.dtype}, {h_u.dtype})")
+    if h_c.dim() != 4 or tuple(h_c.shape) != tuple(h_u.shape):
+        raise rt.CnbError(f"guidance_combine: h_c and h_u must share one (B, H, W, C) shape "
+                          f"(got {tuple(h_c.shape)}, {tuple(h_u.shape)})")
+    ldc, ldu = _nhwc_ld(h_c, "guidance_combine"), _nhwc_ld(h_u, "guidance_combine")
+    B, H, W, C = h_c.shape
+    if out is None:
+        out = torch.empty((B, C, H, W), device=h_c.device, dtype=torch.float32)
+    elif tuple(out.shape) != (B, C, H, W) or out.dtype != torch.float32 or not out.is_contiguous():
+        raise rt.CnbError("guidance_combine: out must be a contiguous fp32 (B, C, H, W) tensor")
+    rt.check(rt.lib().cnb_guidance_combine(h_c.data_ptr(), ldc, h_u.data_ptr(), ldu, out.data_ptr(), B, C, H * W,
+                                           float(w), 1 if h_c.dtype == torch.float16 else 0, rt.stream()))
     return out
 
 
@@ -377,9 +405,7 @@ def edm_combine_to_nchw(c_skip, x, c_out, f, in_coff=0, c=None):
     view): the student's output in NCHW fp32, one launch."""
     rt.require_cuda(c_skip, x, c_out, f)
     B, H, W, cv = f.shape
-    ld = f.stride(2)
-    if f.stride(3) != 1 or f.stride(1) != W * ld or f.stride(0) != H * W * ld or ld < cv:
-        raise rt.CnbError("edm_combine_to_nchw: expected a channels-last tensor or a channel slice of one")
+    ld = _nhwc_ld(f, "edm_combine_to_nchw")
     c = cv - in_coff if c is None else c
     if tuple(x.shape) != (B, c, H, W) or x.dtype != torch.float32 or not x.is_contiguous():
         raise rt.CnbError("edm_combine_to_nchw: x must be the contiguous fp32 NCHW tensor matching f")

@@ -83,6 +83,8 @@ _SIGS = {
                                         c_int, c_int, c_void_p]),
     "cnb_nchw_to_nhwc": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_int, c_void_p]),
     "cnb_nhwc_to_nchw": (c_int, [c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
+    "cnb_guidance_combine": (c_int, [c_void_p, c_int, c_void_p, c_int, c_void_p, c_int, c_int, c_int, c_float, c_int,
+                                     c_void_p]),
     "cnb_copy_channels": (c_int, [c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_ll, c_int, c_int, c_void_p]),
     "cnb_tc_error_flag": (c_int, []),
 }

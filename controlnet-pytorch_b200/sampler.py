@@ -21,15 +21,84 @@ skip = strength_to_skip(S, strength), from the reference noised to its first tim
 graph).  With a mask the captured step gains one launch after the update, cnb_inpaint_blend, which puts the known
 region back at the noise level of the next timestep.  The noise z of the start and of every blend is the x_T stream
 (seed, _XT_STEP, global element): fixed over the run, like diffusers' legacy inpainting, and drawn in the kernels.
+
+Control strength (`control=ControlOptions(...)`, a ControlNet only): a conditioning scale on the zero convolutions, a
+window [start, end) of the schedule outside which the step is the frozen U-Net alone, and hint guidance
+eps = eu + w * (ec - eu).  A non-default `control` captures up to two step graphs over the same sampler-owned buffers,
+the control graph (prologue -> model._forward_controlled -> update -> [blend] -> bump) and the plain graph (prologue ->
+model.trained_unet -> update -> [blend] -> bump), and picks one per step on the host from `ControlOptions.keep`.
 """
+
+import dataclasses
+import math
+import numbers
 
 import torch
 
 from . import ops
 from . import runtime as rt
+from .models import _engine as E
 from .scheduler.schedule import noise_levels, strength_to_skip
 
 _XT_STEP = (1 << 40)   # Philox "step" reserved for drawing x_T
+
+
+@dataclasses.dataclass(frozen=True)
+class ControlOptions:
+    """How strongly the hint steers a ControlNet sample (diffusers' names in brackets):
+      scale     multiplies every down and mid zero-convolution residual (controlnet_conditioning_scale); the hint
+                block's own zero convolution is not scaled;
+      start/end the control branch runs on the steps i of the n steps run with not (i / n < start or
+                (i + 1) / n > end) (control_guidance_start / _end); the other steps are the frozen U-Net alone;
+      guidance  w of eps = eu + w * (ec - eu), ec the ControlNet's and eu the frozen U-Net's prediction (guidance_scale
+                with guess_mode and no prompt); 1 is no guidance.
+    ControlOptions() is the plain ControlNet sampler."""
+    scale: float = 1.0
+    start: float = 0.0
+    end: float = 1.0
+    guidance: float = 1.0
+
+    def __post_init__(self):
+        for name in ("scale", "start", "end", "guidance"):
+            v = getattr(self, name)
+            if isinstance(v, bool) or not isinstance(v, numbers.Real) or not math.isfinite(v):
+                raise rt.CnbError(f"ControlOptions: {name} must be a finite number (got {v!r})")
+        for name in ("scale", "guidance"):
+            if getattr(self, name) < 0:
+                raise rt.CnbError(f"ControlOptions: {name} must be >= 0 (got {getattr(self, name)!r})")
+        if not 0 <= self.start < self.end <= 1:
+            raise rt.CnbError(f"ControlOptions: need 0 <= start < end <= 1 (got start={self.start!r}, "
+                              f"end={self.end!r})")
+
+    def keep(self, n):
+        """Per step of the n steps run (the tail for img2img): True where the control branch runs.  All False when
+        scale or guidance is 0: eps is then exactly the frozen U-Net's."""
+        if self.scale == 0 or self.guidance == 0:
+            return [False] * n
+        return [not (i / n < self.start or (i + 1) / n > self.end) for i in range(n)]
+
+
+def _control(model, control):
+    """None for the plain ControlNet step (control None or default), else the checked ControlOptions."""
+    if control is None:
+        return None
+    if not isinstance(control, ControlOptions):
+        raise rt.CnbError(f"control must be a sampler.ControlOptions (got {type(control).__name__})")
+    if control == ControlOptions():
+        return None
+    if not hasattr(model, "_forward_controlled"):
+        raise rt.CnbError(f"control options need a ControlNet; {type(model).__name__} has no control branch")
+    return control
+
+
+def _step_forward(model, ctl, controlled, hint):
+    """eps(xt, t) of one step: the model's forward, its controlled forward or the frozen U-Net alone."""
+    if ctl is None:
+        return lambda xt, t: model(xt, t, hint)
+    if not controlled:
+        return lambda xt, t: model.trained_unet(xt, t)
+    w = None if ctl.guidance == 1.0 else float(ctl.guidance)
+    return lambda xt, t: model._forward_controlled(xt, t, hint, ctl.scale, w)
 
 
 class DDPMSampler:
@@ -75,11 +144,12 @@ class DDPMSampler:
     # ---- eager loop (injected z, parity tests, per-step callbacks) ----------------------------------------
     @torch.no_grad()
     def sample_eager(self, x_T, hint, steps=None, zs=None, elem_offset=0, callback=None, x_ref=None, mask=None,
-                     strength=1.0):
+                     strength=1.0, control=None):
         """The loop without a graph; returns (x, x0).  With `x_ref` it is img2img's loop (see there): it starts from
         add_noise(x_ref, z, tau_skip) and, with `mask`, blends after every step, where z is x_T when given (injected
-        noise) and otherwise the x_T stream."""
+        noise) and otherwise the x_T stream.  `control`: ControlOptions (see there)."""
         sch = self.scheduler
+        ctl = _control(self.model, control)
         skip, levels = 0, None
         if x_ref is None and mask is not None:
             raise rt.CnbError("sample_eager: a mask needs the reference x_ref")
@@ -98,9 +168,11 @@ class DDPMSampler:
         x0 = None
         state = sch.new_state(xt)
         t_dev = torch.empty((1,), device=dev, dtype=torch.int64)
+        keep = [True] * len(ts) if ctl is None else ctl.keep(len(ts))
+        fwd = {c: _step_forward(self.model, ctl, c, hint) for c in set(keep)}
         for k, t in enumerate(ts):
             t_dev.fill_(t)
-            eps = self.model(xt, t_dev, hint)
+            eps = fwd[keep[k]](xt, t_dev)
             # the last step adds no noise in any scheduler, so zs may stop one short of the schedule
             z = zs[k].to(xt.device) if (zs is not None and k < len(ts) - 1) else None
             xt, x0 = sch.update(xt, eps, table[t], z=z, want_x0=True, seed=self.seed, step=k,
@@ -126,7 +198,7 @@ class DDPMSampler:
             return
         fn(self._hint, rt.get_mode())
 
-    def _capture(self, x_T, hint, steps, elem_offset, skip=0, x_ref=None, mask=None):
+    def _capture(self, x_T, hint, steps, elem_offset, skip=0, x_ref=None, mask=None, control=None):
         dev = x_T.device
         sch = self.scheduler
         self.xt = x_T.clone().contiguous()
@@ -148,11 +220,12 @@ class DDPMSampler:
         self._mask = None if mask is None else mask.clone()
         self._levels = None if mask is None else noise_levels(self._base(), ts).to(dev)
         L = rt.lib()
+        ctl = _control(self.model, control)
 
-        def one_step():
+        def one_step(forward):
             rt.check(L.cnb_sampler_prologue(self.step_idx.data_ptr(), self.t_seq.data_ptr(), self.t_out.data_ptr(),
                                             table.data_ptr(), self.coef.data_ptr(), rt.stream()))
-            eps = self.model(self.xt, self.t_out, hint)
+            eps = forward(self.xt, self.t_out)
             sch.update(self.xt, eps, self.coef, z=None, seed=self.seed, step_dev=self.step_idx,
                        elem_offset=elem_offset, out=self.xt, x0_out=self.x0, **state)
             if mask is not None:
@@ -160,47 +233,66 @@ class DDPMSampler:
                                   seed=self.seed, noise_step=_XT_STEP, elem_offset=elem_offset)
             rt.check(L.cnb_bump_index(self.step_idx.data_ptr(), 1, rt.stream()))
 
-        # warm-up on a side stream: builds weight / hint caches and sets kernel attributes outside the capture
-        s = torch.cuda.Stream(device=dev)
-        s.wait_stream(torch.cuda.current_stream())
-        with torch.cuda.stream(s):
-            one_step()
-        torch.cuda.current_stream().wait_stream(s)
-        torch.cuda.synchronize(dev)
-        c0 = rt.launch_count()
-        g = torch.cuda.CUDAGraph()
-        with torch.cuda.graph(g):
-            one_step()
-        self.launches_per_step = rt.launch_count() - c0
-        self._graph = g
+        def capture(forward):
+            # warm-up on a side stream: builds weight / hint caches and sets kernel attributes outside the capture
+            s = torch.cuda.Stream(device=dev)
+            s.wait_stream(torch.cuda.current_stream())
+            with torch.cuda.stream(s):
+                self.step_idx.zero_()
+                one_step(forward)
+            torch.cuda.current_stream().wait_stream(s)
+            torch.cuda.synchronize(dev)
+            c0 = rt.launch_count()
+            g = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(g):
+                one_step(forward)
+            return g, rt.launch_count() - c0
+
+        # with control options, the control graph and the plain graph share every buffer above and are captured only
+        # when some step uses them; replay_steps picks one per step from self._keep
+        self._keep = None if ctl is None else ctl.keep(len(ts))
+        self._graphs = {}
+        self.launches_per_step = self.plain_launches_per_step = None
+        for controlled in ((True,) if ctl is None else sorted(set(self._keep), reverse=True)):
+            g, n = capture(_step_forward(self.model, ctl, controlled, hint))
+            self._graphs[controlled] = g
+            if controlled:
+                self.launches_per_step = n
+            else:
+                self.plain_launches_per_step = n
+        self._graph = self._graphs[True] if self._keep is None else self._graphs[self._keep[0]]
         self._nsteps, self._pos = len(ts), 0
-        # keep every tensor the graph reads alive for as long as the graph: the hint features (HintCache may evict)
+        # keep every tensor the graphs read alive for as long as the graphs: the hint features (HintCache may evict)
+        # and the scaled zero-convolution weights (replaced when another scale is used)
         cache = getattr(self.model, "_hint_cache", None)
-        self._baked = cache.pinned() if cache is not None else []
+        self._baked = (cache.pinned() if cache is not None else []) + E.pinned_scaled(self.model)
 
     @torch.no_grad()
-    def sample(self, x_T, hint, steps=None, elem_offset=0):
+    def sample(self, x_T, hint, steps=None, elem_offset=0, control=None):
         """Run the scheduler's timesteps (DDPM: t = steps-1 .. 0, SURVEY.md 3.5 semantics) with fused on-device noise;
-        returns (x after the last step, x0)."""
+        returns (x after the last step, x0).  `control`: ControlOptions (see there)."""
         rt.require_cuda(x_T, hint)
         if not self.use_graph:
-            return self.sample_eager(x_T, hint, steps, None, elem_offset)
+            return self.sample_eager(x_T, hint, steps, None, elem_offset, control=control)
         if hint.shape[0] != x_T.shape[0]:
             raise rt.CnbError("sample: x_T and hint must have the same batch size")
-        self._prepare(x_T, hint, steps, elem_offset)
+        self._prepare(x_T, hint, steps, elem_offset, control=control)
         self.xt.copy_(x_T)
         return self._run()
 
-    def _prepare(self, x_T, hint, steps, elem_offset, skip=0, x_ref=None, mask=None):
-        """Capture the step graph, or refresh the sampler-owned buffers of the one that fits."""
+    def _prepare(self, x_T, hint, steps, elem_offset, skip=0, x_ref=None, mask=None, control=None):
+        """Capture the step graph(s), or refresh the sampler-owned buffers of the ones that fit."""
         sch = self.scheduler
         # the table's address tells apart schedulers with equal graph keys but other beta schedules; the noise-level
         # table is sampler-owned and refreshed below, so its values need no key
         key = (tuple(x_T.shape), tuple(hint.shape), sch.graph_key(steps, skip),
                sch.coef_table(x_T.device, steps, skip).data_ptr(), elem_offset, rt.get_mode(), str(x_T.device),
                self._param_stamp(), skip, None if mask is None else tuple(mask.shape))
+        ctl = _control(self.model, control)
+        if ctl is not None:
+            key += ((ctl.scale, ctl.guidance, tuple(ctl.keep(len(sch.timesteps(steps, skip))))),)
         if self._graph is None or key != self._key:
-            self._capture(x_T, hint, steps, elem_offset, skip, x_ref, mask)
+            self._capture(x_T, hint, steps, elem_offset, skip, x_ref, mask, ctl)
             self._key = key
         else:
             self._hint.copy_(hint)
@@ -217,7 +309,7 @@ class DDPMSampler:
         return out
 
     @torch.no_grad()
-    def img2img(self, x_ref, hint, strength=1.0, mask=None, steps=None, elem_offset=0):
+    def img2img(self, x_ref, hint, strength=1.0, mask=None, steps=None, elem_offset=0, control=None):
         """Image-to-image (SDEdit) and inpainting under the hint; returns (x, x0).
         The run keeps the last n = min(S, int(S * strength)) of the S timesteps of `timesteps(steps)`
         (scheduler.schedule.strength_to_skip) and starts from add_noise(x_ref, z, tau_skip), z the x_T stream
@@ -225,15 +317,17 @@ class DDPMSampler:
         same tail.  `mask` ([B, 1 or C, H, W], fp32 or bool; 1 = generate, 0 = keep the reference) adds one launch to
         the captured step: after step k the elements with m = 0 are add_noise(x_ref, z, tau_{k+1}) with the same z,
         x_ref exactly after the last step, and soft values blend m * x + (1 - m) * known.  The returned x is blended;
-        x0 is the update's own prediction of the last step, before the blend."""
+        x0 is the update's own prediction of the last step, before the blend.  `control`: ControlOptions, whose window
+        applies to the steps run."""
         rt.require_cuda(x_ref, hint)
         if not self.use_graph:
-            return self.sample_eager(None, hint, steps, None, elem_offset, x_ref=x_ref, mask=mask, strength=strength)
+            return self.sample_eager(None, hint, steps, None, elem_offset, x_ref=x_ref, mask=mask, strength=strength,
+                                     control=control)
         x_ref, mask, skip = self._img2img_args(x_ref, mask, strength, steps)
         if hint.shape[0] != x_ref.shape[0]:
             raise rt.CnbError("img2img: x_ref and hint must have the same batch size")
         ts = self.scheduler.timesteps(steps, skip)
-        self._prepare(x_ref, hint, steps, elem_offset, skip, x_ref, mask)
+        self._prepare(x_ref, hint, steps, elem_offset, skip, x_ref, mask, control)
         self._noised_start(x_ref, ts[0], None, elem_offset, out=self.xt)
         return self._run()
 
@@ -246,7 +340,7 @@ class DDPMSampler:
             if self._pos >= self._nsteps:      # wrap around the schedule instead of running off the t table
                 self.step_idx.zero_()
                 self._pos = 0
-            self._graph.replay()
+            (self._graph if self._keep is None else self._graphs[self._keep[self._pos]]).replay()
             self._pos += 1
 
 
@@ -272,12 +366,12 @@ class LDMSampler(DDPMSampler):
         return outs[0] if len(outs) == 1 else torch.cat(outs, dim=0)
 
     @torch.no_grad()
-    def sample_images(self, x_T, hint, steps=None, elem_offset=0, zs=None, to_unit_range=True):
+    def sample_images(self, x_T, hint, steps=None, elem_offset=0, zs=None, to_unit_range=True, control=None):
         """Returns (images, final latents).  zs: injected per-step noise (eager loop, parity tests)."""
         if zs is not None:
-            xt, _ = self.sample_eager(x_T, hint, steps, zs, elem_offset)
+            xt, _ = self.sample_eager(x_T, hint, steps, zs, elem_offset, control=control)
         else:
-            xt, _ = self.sample(x_T, hint, steps=steps, elem_offset=elem_offset)
+            xt, _ = self.sample(x_T, hint, steps=steps, elem_offset=elem_offset, control=control)
         return self.decode(xt, to_unit_range), xt
 
     @torch.no_grad()
@@ -302,13 +396,15 @@ class LDMSampler(DDPMSampler):
         return ops.mask_max_pool(mask.contiguous(), f)
 
     @torch.no_grad()
-    def img2img_images(self, images, hint, strength=1.0, mask=None, steps=None, elem_offset=0, to_unit_range=True):
+    def img2img_images(self, images, hint, strength=1.0, mask=None, steps=None, elem_offset=0, to_unit_range=True,
+                       control=None):
         """img2img on the latents of `images` ([-1, 1], encoded to the posterior mean) with an image-space `mask`
         pooled to the latent grid; returns (decoded images, final latents).  The known LATENT region is exact; the
         decoded pixels of the kept region are not (there is no paste-back after decode)."""
         lat = self.encode_mean(images)
         lmask = None if mask is None else self.latent_mask(mask, lat)
-        xt, _ = self.img2img(lat, hint, strength=strength, mask=lmask, steps=steps, elem_offset=elem_offset)
+        xt, _ = self.img2img(lat, hint, strength=strength, mask=lmask, steps=steps, elem_offset=elem_offset,
+                             control=control)
         return self.decode(xt, to_unit_range), xt
 
 
@@ -386,7 +482,8 @@ def shard_bounds(total, world, rank):
 
 @torch.no_grad()
 def sample_data_parallel(model, scheduler, shape, hint_fn, steps=None, seed=0, group=None, use_graph=True,
-                         gather=True, vae=None, sampler=None, x_T_fn=None, x_ref_fn=None, mask_fn=None, strength=1.0):
+                         gather=True, vae=None, sampler=None, x_T_fn=None, x_ref_fn=None, mask_fn=None, strength=1.0,
+                         control=None):
     """One job over all ranks of `group` (tools/sample_ddpm_controlnet.py:21-51 sharded over the GPUs of a box): rank r
     draws (or receives) and denoises samples [lo, hi) of the global batch `shape[0]`, no collective inside the
     timestep loop, and the final samples are all-gathered ONCE (NCCL over NVLink).
@@ -396,7 +493,8 @@ def sample_data_parallel(model, scheduler, shape, hint_fn, steps=None, seed=0, g
     `sampler` re-uses a DDPMSampler / LDMSampler (and its captured step graph) across calls.  With `vae` the shard's
     final latents are decoded locally (LDM path) and the images are what is gathered.
     `x_ref_fn(lo, hi)` (and `mask_fn(lo, hi)`), mirroring hint_fn, make the job img2img (inpainting) at `strength`:
-    they return the shard's references and masks, images and image-space masks with `vae` (encoded locally)."""
+    they return the shard's references and masks, images and image-space masks with `vae` (encoded locally).
+    `control`: ControlOptions (see there) for every shard."""
     import torch.distributed as dist
     world = dist.get_world_size(group) if dist.is_initialized() else 1
     rank = dist.get_rank(group) if dist.is_initialized() else 0
@@ -418,16 +516,16 @@ def sample_data_parallel(model, scheduler, shape, hint_fn, steps=None, seed=0, g
         mask = None if mask_fn is None else mask_fn(lo, hi)
         if vae is not None:
             xt, _ = smp.img2img_images(x_ref_fn(lo, hi), hint_fn(lo, hi), strength=strength, mask=mask, steps=steps,
-                                       elem_offset=lo * per)
+                                       elem_offset=lo * per, control=control)
         else:
             xt, _ = smp.img2img(x_ref_fn(lo, hi), hint_fn(lo, hi), strength=strength, mask=mask, steps=steps,
-                                elem_offset=lo * per)
+                                elem_offset=lo * per, control=control)
     else:
         if x_T_fn is not None:
             x_T = x_T_fn(lo, hi)
         else:
             x_T = smp.draw_xT((hi - lo,) + tuple(shape[1:]), dev, elem_offset=lo * per)
-        xt, x0 = smp.sample(x_T, hint_fn(lo, hi), steps=steps, elem_offset=lo * per)
+        xt, x0 = smp.sample(x_T, hint_fn(lo, hi), steps=steps, elem_offset=lo * per, control=control)
         if vae is not None:
             xt = smp.decode(xt)
     if not gather or world == 1:

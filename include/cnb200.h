@@ -294,7 +294,15 @@ int cnb_nchw_to_nhwc(const float* src, float* dst, int B, int C, int HW, int ldo
 /* src is fp32 (src_f16 == 0) or fp16; dst is always the fp32 NCHW tensor of the public API */
 int cnb_nhwc_to_nchw(const void* src, int ldi, int in_coff, float* dst, int B, int C, int HW, int src_f16,
                      cnb_stream_t stream);
-/* elt = bytes per element (4 or 2); offsets and leading dimensions in elements */
+/* Hint guidance (classifier-free guidance with the hint as the condition): h_c and h_u are the channels-last outputs
+ * of the ControlNet and of the frozen U-Net, both fp32 (src_f16 == 0) or both fp16, with leading dimensions ldc / ldu
+ * >= C (each pointer addresses channel 0 of its view).  Per element, in fp32, separate IEEE operations:
+ *   dst[b, c, p] = eu + w * (ec - eu)
+ * so the result equals that fp32 expression on the two cnb_nhwc_to_nchw results bit for bit (w == 0 gives eu).  dst is
+ * contiguous fp32 NCHW and must not overlap either input; pointers aligned to their element size. */
+int cnb_guidance_combine(const void* h_c, int ldc, const void* h_u, int ldu, float* dst, int B, int C, int HW, float w,
+                         int src_f16, cnb_stream_t stream);
+/* elt =bytes per element (4 or 2); offsets and leading dimensions in elements */
 int cnb_copy_channels(const void* src, int lds, int s_coff, void* dst, int ldd, int d_coff, long long npix,
                       int C, int elt, cnb_stream_t stream);
 
