@@ -655,11 +655,14 @@ conv_tma_kernel(const __grid_constant__ TmaArgs a) {
             const int rb = __shfl_sync(0xffffffffu, b, row);
             if (rp >= 0) {
               float4 o = *reinterpret_cast<const float4*>(slab + (size_t)row * SSTR + sub_c);
-              o.x += bv.x; o.y += bv.y; o.z += bv.z; o.w += bv.w;
+              float4 bt = bv;
               if (a.temb && a.temb_per_sample) {
+                // bias + row first, then the accumulator: the order of the shared-row epilogues, so a sample's bits do
+                // not depend on whether its time-embedding row is shared with the batch
                 const float4 t = __ldg(reinterpret_cast<const float4*>(a.temb + (size_t)rb * a.temb_ld + n));
-                o.x += t.x; o.y += t.y; o.z += t.z; o.w += t.w;
+                bt.x += t.x; bt.y += t.y; bt.z += t.z; bt.w += t.w;
               }
+              o.x += bt.x; o.y += bt.y; o.z += bt.z; o.w += bt.w;
               if (a.residual) {
                 const float4 t = a.res_f16
                     ? ld_half4(reinterpret_cast<const __half*>(a.residual) + rp * ldr + a.res_coff + n)

@@ -240,32 +240,33 @@ def _hint(B, s, seed):
     return (torch.rand(B, 1, s, s, generator=g, device="cuda") < 0.1).float().expand(B, 3, s, s).contiguous()
 
 
+_LATENT_PARAMS = dict(syn.CELEBHQ_LDM_PARAMS, im_channels=4, im_size=32)
+
+# The production workloads (bench.py configs 2-5): (tag, batch sizes in f16 mode, batch size in fp32 mode, builder,
+# call).  The largest f16 batch is the largest batch the workload runs in production.
+WORKLOADS = [
+    ("config2_mnist_controlnet", (1024, 128), 128, lambda: _mod("models.controlnet").ControlNet(syn.MNIST_PARAMS),
+     lambda m, B: m(torch.randn(B, 1, 28, 28, device="cuda"), torch.tensor([500], device="cuda"), _hint(B, 28, 1))),
+    ("config3_celebhq_ldm_controlnet", (256, 32), 32,
+     lambda: _mod("models.controlnet_ldm").ControlNet(4, syn.CELEBHQ_LDM_PARAMS, down_sample_factor=32),
+     lambda m, B: m(torch.randn(B, 4, 32, 32, device="cuda"), torch.tensor([500], device="cuda"), _hint(B, 1024, 2))),
+    ("config3_celebhq_vae_decode", (256, 32), 32, lambda: _mod("models.vae").VAE(3, syn.CELEBHQ_VAE_PARAMS),
+     lambda m, B: m.decode(torch.randn(B, 4, 32, 32, device="cuda"))),
+    ("config4_consistency_mnist", (4096,), 64,
+     lambda: _mod("models.consistency_controlnet_distilled").ConsistencyControlNet(syn.MNIST_PARAMS),
+     lambda m, B: m(torch.randn(B, 1, 28, 28, device="cuda"), torch.full((B,), 80.0, device="cuda"), _hint(B, 28, 3))),
+    ("config4_consistency_celebhq_latent", (4096,), 64,
+     lambda: _mod("models.consistency_controlnet_distilled").ConsistencyControlNet(_LATENT_PARAMS),
+     lambda m, B: m(torch.randn(B, 4, 32, 32, device="cuda"), torch.full((B,), 80.0, device="cuda"), _hint(B, 32, 4))),
+    ("config5_dm_cifar", (1, 7, 128, 1000, 8192), 7,
+     lambda: _mod("models.distribution_matching_controlnet").DistributionMatchingControlNet(syn.CIFAR_PARAMS),
+     lambda m, B: m(torch.randn(B, 3, 32, 32, device="cuda"), torch.full((B,), 999, device="cuda"), _hint(B, 32, 5))),
+]
+
+
 def _run_workloads(rec, rt):
-    """One eager no_grad forward of each production workload (bench.py configs 2-5)."""
-    cn, cnl, vae = _mod("models.controlnet"), _mod("models.controlnet_ldm"), _mod("models.vae")
-    cs, dm = _mod("models.consistency_controlnet_distilled"), _mod("models.distribution_matching_controlnet")
-    lat = dict(syn.CELEBHQ_LDM_PARAMS, im_channels=4, im_size=32)
-    runs = [
-        # (tag, batch sizes in f16 mode, batch size in fp32 mode, builder, call)
-        ("config2_mnist_controlnet", (1024, 128), 128, lambda: cn.ControlNet(syn.MNIST_PARAMS),
-         lambda m, B: m(torch.randn(B, 1, 28, 28, device="cuda"), torch.tensor([500], device="cuda"), _hint(B, 28, 1))),
-        ("config3_celebhq_ldm_controlnet", (256, 32), 32,
-         lambda: cnl.ControlNet(4, syn.CELEBHQ_LDM_PARAMS, down_sample_factor=32),
-         lambda m, B: m(torch.randn(B, 4, 32, 32, device="cuda"), torch.tensor([500], device="cuda"),
-                        _hint(B, 1024, 2))),
-        ("config3_celebhq_vae_decode", (256, 32), 32, lambda: vae.VAE(3, syn.CELEBHQ_VAE_PARAMS),
-         lambda m, B: m.decode(torch.randn(B, 4, 32, 32, device="cuda"))),
-        ("config4_consistency_mnist", (4096,), 64, lambda: cs.ConsistencyControlNet(syn.MNIST_PARAMS),
-         lambda m, B: m(torch.randn(B, 1, 28, 28, device="cuda"), torch.full((B,), 80.0, device="cuda"),
-                        _hint(B, 28, 3))),
-        ("config4_consistency_celebhq_latent", (4096,), 64, lambda: cs.ConsistencyControlNet(lat),
-         lambda m, B: m(torch.randn(B, 4, 32, 32, device="cuda"), torch.full((B,), 80.0, device="cuda"),
-                        _hint(B, 32, 4))),
-        ("config5_dm_cifar", (1, 7, 128, 1000, 8192), 7, lambda: dm.DistributionMatchingControlNet(syn.CIFAR_PARAMS),
-         lambda m, B: m(torch.randn(B, 3, 32, 32, device="cuda"), torch.full((B,), 999, device="cuda"),
-                        _hint(B, 32, 5))),
-    ]
-    for tag, f16_batches, f32_batch, build, call in runs:
+    """One eager no_grad forward of each production workload."""
+    for tag, f16_batches, f32_batch, build, call in WORKLOADS:
         m = _fill(build())
         for mode, batches in (("f16", f16_batches), ("fp32", (f32_batch,))):
             rt.set_mode(mode)
