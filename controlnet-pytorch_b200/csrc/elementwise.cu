@@ -85,7 +85,7 @@ __device__ __forceinline__ float philox_pick(float4 v, int k) {
 
 // One Philox4x32-10 block yields the four normals of global elements 4q .. 4q+3; a thread owns one such block and
 // stores it with one float4 when the output is 16-byte aligned with the global element grid (same element -> value
-// mapping as the fused draw inside sched_step_kernel).
+// mapping as the fused draw inside update_kernel).
 __global__ void philox_normal_kernel(float* __restrict__ out, long long n, uint64_t seed, uint64_t step,
                                      uint64_t elem_offset) {
   const uint64_t g0 = elem_offset & ~3ull;                       // first Philox block that overlaps the output
@@ -129,147 +129,107 @@ __device__ __forceinline__ float step_noise1(const float* __restrict__ z, long l
 }
 
 // ------------------------------------------------------------------------------------------------
-// sample_prev_timestep: separate IEEE ops in the reference's order (the *_rn intrinsics are never contracted)
+// The fused scheduler updates: one grid-stride kernel, one rule per scheduler.  Every rule evaluates its scheduler's
+// fp32 operation order with separate IEEE ops (the *_rn intrinsics are never contracted into an FMA) and starts from
+// the same data prediction, so x0 is bit-identical across the three.  A rule maps one element's (xt, eps, z, hist) to
+// (x_prev, its new hist value, x0); kHist marks the rule that carries a history buffer, which the kernel reads only
+// when the rule's `second` is set and writes every step.
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void sched_one(float xt, float e, float zv, const float s1, const float sq_acp,
-                                          const float beta, const float sq_alpha, const float sigma,
-                                          const bool noisy, float& prev, float& x0) {
-  float v = __fdiv_rn(__fsub_rn(xt, __fmul_rn(s1, e)), sq_acp);
-  x0 = fminf(fmaxf(v, -1.0f), 1.0f);
-  float mean = __fdiv_rn(__fsub_rn(xt, __fdiv_rn(__fmul_rn(beta, e), s1)), sq_alpha);
-  prev = noisy ? __fadd_rn(mean, __fmul_rn(sigma, zv)) : mean;
+// v = (xt - c0 * eps) / c1 with c0 = sqrt(1 - alpha_cum_prod[t]), c1 = sqrt(alpha_cum_prod[t]): x0 before its clamp
+__device__ __forceinline__ float data_prediction(float xt, float e, float c0, float c1) {
+  return __fdiv_rn(__fsub_rn(xt, __fmul_rn(c0, e)), c1);
 }
 
-__global__ void sched_step_kernel(const float* __restrict__ xt, const float* __restrict__ eps,
-                                  const float* __restrict__ z, float* __restrict__ prev, float* __restrict__ x0,
-                                  long long n, const float* __restrict__ coef, uint64_t seed, uint64_t step,
-                                  const int32_t* __restrict__ step_dev, uint64_t elem_offset) {
+__device__ __forceinline__ float clamp1(float v) { return fminf(fmaxf(v, -1.0f), 1.0f); }
+
+// DDPM (scheduler/linear_noise_scheduler.py, the reference's sample_prev_timestep):
+// x_prev = (xt - beta * eps / s1) / sqrt(alpha) (+ sigma * z)
+struct DdpmRule {
+  static constexpr bool kHist = false;
+  float s1, sq_acp, beta, sq_alpha, sigma;
+  bool noisy;
+  __device__ DdpmRule(const float* c, int)
+      : s1(c[0]), sq_acp(c[1]), beta(c[2]), sq_alpha(c[3]), sigma(c[4]), noisy(c[5] != 0.0f) {}
+  __device__ void operator()(float xt, float e, float zv, float, float& prev, float&, float& x0) const {
+    x0 = clamp1(data_prediction(xt, e, s1, sq_acp));
+    const float mean = __fdiv_rn(__fsub_rn(xt, __fdiv_rn(__fmul_rn(beta, e), s1)), sq_alpha);
+    prev = noisy ? __fadd_rn(mean, __fmul_rn(sigma, zv)) : mean;
+  }
+};
+
+// DDIM (scheduler/ddim_scheduler.py): x_prev = c2 * x0' + c3 * eps (+ c4 * z), x0' = clamp(v) with clip_sample, else v
+struct DdimRule {
+  static constexpr bool kHist = false;
+  float c0, c1, c2, c3, c4;
+  bool noisy, clip;
+  __device__ DdimRule(const float* c, int clip_sample)
+      : c0(c[0]), c1(c[1]), c2(c[2]), c3(c[3]), c4(c[4]), noisy(c[5] != 0.0f), clip(clip_sample != 0) {}
+  __device__ void operator()(float xt, float e, float zv, float, float& prev, float&, float& x0) const {
+    const float v = data_prediction(xt, e, c0, c1);
+    x0 = clamp1(v);
+    const float p = __fadd_rn(__fmul_rn(c2, clip ? x0 : v), __fmul_rn(c3, e));
+    prev = noisy ? __fadd_rn(p, __fmul_rn(c4, zv)) : p;
+  }
+};
+
+// DPM-Solver++ multistep (scheduler/dpm_solver_scheduler.py): D = clamp(v) with clip_sample, else v;
+// x_prev = A * xt + B0 * D (+ B1 * hist) (+ C * z), hist = D.  hist is read only when B1 != 0, so a first-order row
+// never touches the previous step's (possibly uninitialised) buffer.
+struct DpmSolverRule {
+  static constexpr bool kHist = true;
+  float c0, c1, A, B0, B1, C;
+  bool second, noisy, clip;
+  __device__ DpmSolverRule(const float* c, int clip_sample)
+      : c0(c[0]), c1(c[1]), A(c[2]), B0(c[3]), B1(c[4]), C(c[5]), second(c[4] != 0.0f), noisy(c[5] != 0.0f),
+        clip(clip_sample != 0) {}
+  __device__ void operator()(float xt, float e, float zv, float hv, float& prev, float& d, float& x0) const {
+    const float v = data_prediction(xt, e, c0, c1);
+    x0 = clamp1(v);
+    d = clip ? x0 : v;
+    float p = __fadd_rn(__fmul_rn(A, xt), __fmul_rn(B0, d));
+    if (second) p = __fadd_rn(p, __fmul_rn(B1, hv));
+    prev = noisy ? __fadd_rn(p, __fmul_rn(C, zv)) : p;
+  }
+};
+
+template <class Rule>
+__global__ void update_kernel(const float* __restrict__ xt, const float* __restrict__ eps, const float* __restrict__ z,
+                              float* __restrict__ hist, float* __restrict__ prev, float* __restrict__ x0, long long n,
+                              const float* __restrict__ coef, int clip_sample, uint64_t seed, uint64_t step,
+                              const int32_t* __restrict__ step_dev, uint64_t elem_offset) {
   if (step_dev) step = (uint64_t)step_dev[0];
-  const float s1 = coef[0], sq_acp = coef[1], beta = coef[2], sq_alpha = coef[3], sigma = coef[4];
-  const bool noisy = coef[5] != 0.0f;
+  const Rule rule(coef, clip_sample);
   const long long n4 = n >> 2;
   const bool aligned4 = ((elem_offset & 3) == 0);
   const long long stride = (long long)gridDim.x * blockDim.x;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
     float4 a = reinterpret_cast<const float4*>(xt)[i];
     float4 e = reinterpret_cast<const float4*>(eps)[i];
-    const float4 zz = noisy ? step_noise4(z, i, seed, step, elem_offset, aligned4) : make_float4(0.f, 0.f, 0.f, 0.f);
-    float4 p, o;
-    sched_one(a.x, e.x, zz.x, s1, sq_acp, beta, sq_alpha, sigma, noisy, p.x, o.x);
-    sched_one(a.y, e.y, zz.y, s1, sq_acp, beta, sq_alpha, sigma, noisy, p.y, o.y);
-    sched_one(a.z, e.z, zz.z, s1, sq_acp, beta, sq_alpha, sigma, noisy, p.z, o.z);
-    sched_one(a.w, e.w, zz.w, s1, sq_acp, beta, sq_alpha, sigma, noisy, p.w, o.w);
-    reinterpret_cast<float4*>(prev)[i] = p;
-    if (x0) reinterpret_cast<float4*>(x0)[i] = o;
-  }
-  // tail (n % 4 elements)
-  if (blockIdx.x == 0 && threadIdx.x < (n & 3)) {
-    long long i = (n4 << 2) + threadIdx.x;
-    const float zv = noisy ? step_noise1(z, i, seed, step, elem_offset) : 0.f;
-    float p, o;
-    sched_one(xt[i], eps[i], zv, s1, sq_acp, beta, sq_alpha, sigma, noisy, p, o);
-    prev[i] = p;
-    if (x0) x0[i] = o;
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// DDIM update (scheduler/ddim_scheduler.py): x0 exactly as sched_one computes it, then
-// x_prev = c2 * x0' + c3 * eps (+ c4 * z), x0' = clamp(x0) with clip_sample, else x0; separate IEEE ops
-// ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void ddim_one(float xt, float e, float zv, const float c0, const float c1, const float c2,
-                                         const float c3, const float c4, const bool noisy, const bool clip,
-                                         float& prev, float& x0) {
-  const float v = __fdiv_rn(__fsub_rn(xt, __fmul_rn(c0, e)), c1);
-  x0 = fminf(fmaxf(v, -1.0f), 1.0f);
-  const float p = __fadd_rn(__fmul_rn(c2, clip ? x0 : v), __fmul_rn(c3, e));
-  prev = noisy ? __fadd_rn(p, __fmul_rn(c4, zv)) : p;
-}
-
-__global__ void ddim_step_kernel(const float* __restrict__ xt, const float* __restrict__ eps,
-                                 const float* __restrict__ z, float* __restrict__ prev, float* __restrict__ x0,
-                                 long long n, const float* __restrict__ coef, int clip_sample, uint64_t seed,
-                                 uint64_t step, const int32_t* __restrict__ step_dev, uint64_t elem_offset) {
-  if (step_dev) step = (uint64_t)step_dev[0];
-  const float c0 = coef[0], c1 = coef[1], c2 = coef[2], c3 = coef[3], c4 = coef[4];
-  const bool noisy = coef[5] != 0.0f, clip = clip_sample != 0;
-  const long long n4 = n >> 2;
-  const bool aligned4 = ((elem_offset & 3) == 0);
-  const long long stride = (long long)gridDim.x * blockDim.x;
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
-    float4 a = reinterpret_cast<const float4*>(xt)[i];
-    float4 e = reinterpret_cast<const float4*>(eps)[i];
-    const float4 zz = noisy ? step_noise4(z, i, seed, step, elem_offset, aligned4) : make_float4(0.f, 0.f, 0.f, 0.f);
-    float4 p, o;
-    ddim_one(a.x, e.x, zz.x, c0, c1, c2, c3, c4, noisy, clip, p.x, o.x);
-    ddim_one(a.y, e.y, zz.y, c0, c1, c2, c3, c4, noisy, clip, p.y, o.y);
-    ddim_one(a.z, e.z, zz.z, c0, c1, c2, c3, c4, noisy, clip, p.z, o.z);
-    ddim_one(a.w, e.w, zz.w, c0, c1, c2, c3, c4, noisy, clip, p.w, o.w);
-    reinterpret_cast<float4*>(prev)[i] = p;
-    if (x0) reinterpret_cast<float4*>(x0)[i] = o;
-  }
-  // tail (n % 4 elements)
-  if (blockIdx.x == 0 && threadIdx.x < (n & 3)) {
-    long long i = (n4 << 2) + threadIdx.x;
-    const float zv = noisy ? step_noise1(z, i, seed, step, elem_offset) : 0.f;
-    float p, o;
-    ddim_one(xt[i], eps[i], zv, c0, c1, c2, c3, c4, noisy, clip, p, o);
-    prev[i] = p;
-    if (x0) x0[i] = o;
-  }
-}
-
-// ------------------------------------------------------------------------------------------------
-// DPM-Solver++ multistep update (scheduler/dpm_solver_scheduler.py): D = x0 as sched_one computes it (clamped with
-// clip_sample), x_prev = A * xt + B0 * D (+ B1 * hist) (+ C * z), hist = D; separate IEEE ops.  hist is read only
-// when B1 != 0, so a first-order row never touches the previous step's (possibly uninitialised) buffer.
-// ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void dpm_one(float xt, float e, float zv, float hv, const float c0, const float c1,
-                                        const float A, const float B0, const float B1, const float C,
-                                        const bool second, const bool noisy, const bool clip, float& prev,
-                                        float& d, float& x0) {
-  const float v = __fdiv_rn(__fsub_rn(xt, __fmul_rn(c0, e)), c1);
-  x0 = fminf(fmaxf(v, -1.0f), 1.0f);
-  d = clip ? x0 : v;
-  float p = __fadd_rn(__fmul_rn(A, xt), __fmul_rn(B0, d));
-  if (second) p = __fadd_rn(p, __fmul_rn(B1, hv));
-  prev = noisy ? __fadd_rn(p, __fmul_rn(C, zv)) : p;
-}
-
-__global__ void dpm_solver_step_kernel(const float* __restrict__ xt, const float* __restrict__ eps,
-                                       const float* __restrict__ z, float* __restrict__ hist,
-                                       float* __restrict__ prev, float* __restrict__ x0, long long n,
-                                       const float* __restrict__ coef, int clip_sample, uint64_t seed, uint64_t step,
-                                       const int32_t* __restrict__ step_dev, uint64_t elem_offset) {
-  if (step_dev) step = (uint64_t)step_dev[0];
-  const float c0 = coef[0], c1 = coef[1], A = coef[2], B0 = coef[3], B1 = coef[4], C = coef[5];
-  const bool second = B1 != 0.0f, noisy = C != 0.0f, clip = clip_sample != 0;
-  const long long n4 = n >> 2;
-  const bool aligned4 = ((elem_offset & 3) == 0);
-  const long long stride = (long long)gridDim.x * blockDim.x;
-  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += stride) {
-    float4 a = reinterpret_cast<const float4*>(xt)[i];
-    float4 e = reinterpret_cast<const float4*>(eps)[i];
-    const float4 zz = noisy ? step_noise4(z, i, seed, step, elem_offset, aligned4) : make_float4(0.f, 0.f, 0.f, 0.f);
-    const float4 h = second ? reinterpret_cast<const float4*>(hist)[i] : make_float4(0.f, 0.f, 0.f, 0.f);
+    const float4 zz =
+        rule.noisy ? step_noise4(z, i, seed, step, elem_offset, aligned4) : make_float4(0.f, 0.f, 0.f, 0.f);
+    float4 h = make_float4(0.f, 0.f, 0.f, 0.f);
+    if constexpr (Rule::kHist)
+      if (rule.second) h = reinterpret_cast<const float4*>(hist)[i];
     float4 p, d, o;
-    dpm_one(a.x, e.x, zz.x, h.x, c0, c1, A, B0, B1, C, second, noisy, clip, p.x, d.x, o.x);
-    dpm_one(a.y, e.y, zz.y, h.y, c0, c1, A, B0, B1, C, second, noisy, clip, p.y, d.y, o.y);
-    dpm_one(a.z, e.z, zz.z, h.z, c0, c1, A, B0, B1, C, second, noisy, clip, p.z, d.z, o.z);
-    dpm_one(a.w, e.w, zz.w, h.w, c0, c1, A, B0, B1, C, second, noisy, clip, p.w, d.w, o.w);
+    rule(a.x, e.x, zz.x, h.x, p.x, d.x, o.x);
+    rule(a.y, e.y, zz.y, h.y, p.y, d.y, o.y);
+    rule(a.z, e.z, zz.z, h.z, p.z, d.z, o.z);
+    rule(a.w, e.w, zz.w, h.w, p.w, d.w, o.w);
     reinterpret_cast<float4*>(prev)[i] = p;
-    reinterpret_cast<float4*>(hist)[i] = d;
+    if constexpr (Rule::kHist) reinterpret_cast<float4*>(hist)[i] = d;
     if (x0) reinterpret_cast<float4*>(x0)[i] = o;
   }
   // tail (n % 4 elements)
   if (blockIdx.x == 0 && threadIdx.x < (n & 3)) {
     long long i = (n4 << 2) + threadIdx.x;
-    const float zv = noisy ? step_noise1(z, i, seed, step, elem_offset) : 0.f;
-    const float hv = second ? hist[i] : 0.f;
+    const float zv = rule.noisy ? step_noise1(z, i, seed, step, elem_offset) : 0.f;
+    float hv = 0.f;
+    if constexpr (Rule::kHist)
+      if (rule.second) hv = hist[i];
     float p, d, o;
-    dpm_one(xt[i], eps[i], zv, hv, c0, c1, A, B0, B1, C, second, noisy, clip, p, d, o);
+    rule(xt[i], eps[i], zv, hv, p, d, o);
     prev[i] = p;
-    hist[i] = d;
+    if constexpr (Rule::kHist) hist[i] = d;
     if (x0) x0[i] = o;
   }
 }
@@ -372,13 +332,6 @@ __global__ void mask_max_pool_kernel(const float* __restrict__ in, float* __rest
   out[i] = v;
 }
 
-__global__ void gather_row_kernel(const float* __restrict__ table, const int32_t* __restrict__ row,
-                                  float* __restrict__ dst, int ncols) {
-  const size_t r = (size_t)row[0];
-  for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < ncols; i += gridDim.x * blockDim.x)
-    dst[i] = table[r * ncols + i];
-}
-
 __global__ void bump_index_kernel(int32_t* idx, int delta) { idx[0] += delta; }
 
 __global__ void sampler_prologue_kernel(const int32_t* __restrict__ step_idx, const int64_t* __restrict__ t_seq,
@@ -444,8 +397,7 @@ __global__ void x0_from_eps_kernel(const float* __restrict__ xt, const float* __
     out[i] = __int_as_float(0x7fc00000);
     return;
   }
-  const float v = __fdiv_rn(__fsub_rn(xt[i], __fmul_rn(sqrt_one_minus[tb], eps[i])), sqrt_alpha[tb]);
-  out[i] = fminf(fmaxf(v, -1.0f), 1.0f);
+  out[i] = clamp1(data_prediction(xt[i], eps[i], sqrt_one_minus[tb], sqrt_alpha[tb]));
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -602,59 +554,8 @@ extern "C" int cnb_linear_small(const float* x, const float* w, const float* b, 
   return CNB_OK;
 }
 
-extern "C" int cnb_sched_step(const float* xt, const float* eps, const float* z, float* xt_prev, float* x0,
-                              long long n, const float* coef, uint64_t seed, uint64_t step, const int32_t* step_dev,
-                              uint64_t elem_offset, cnb_stream_t s) {
-  CNB_REQUIRE(n > 0 && xt && eps && xt_prev && coef, "sched_step: null pointer or n=%lld", n);
-  CNB_REQUIRE((((uintptr_t)xt | (uintptr_t)eps | (uintptr_t)xt_prev | (uintptr_t)z | (uintptr_t)x0) & 15) == 0,
-              "sched_step: pointers must be 16-byte aligned");
-  long long n4 = n >> 2;
-  unsigned blocks = (unsigned)((n4 + 255) / 256);
-  if (blocks < 1) blocks = 1;
-  if (blocks > 148 * 16) blocks = 148 * 16;
-  sched_step_kernel<<<blocks, 256, 0, (cudaStream_t)s>>>(xt, eps, z, xt_prev, x0, n, coef, seed, step, step_dev,
-                                                         elem_offset);
-  CNB_LAUNCH_CHECK();
-  return CNB_OK;
-}
-
-extern "C" int cnb_ddim_step(const float* xt, const float* eps, const float* z, float* xt_prev, float* x0, long long n,
-                             const float* coef, int clip_sample, uint64_t seed, uint64_t step, const int32_t* step_dev,
-                             uint64_t elem_offset, cnb_stream_t s) {
-  CNB_REQUIRE(n > 0 && xt && eps && xt_prev && coef, "ddim_step: null pointer or n=%lld", n);
-  CNB_REQUIRE((((uintptr_t)xt | (uintptr_t)eps | (uintptr_t)xt_prev | (uintptr_t)z | (uintptr_t)x0) & 15) == 0,
-              "ddim_step: pointers must be 16-byte aligned");
-  long long n4 = n >> 2;
-  unsigned blocks = (unsigned)((n4 + 255) / 256);
-  if (blocks < 1) blocks = 1;
-  if (blocks > 148 * 16) blocks = 148 * 16;
-  ddim_step_kernel<<<blocks, 256, 0, (cudaStream_t)s>>>(xt, eps, z, xt_prev, x0, n, coef, clip_sample, seed, step,
-                                                        step_dev, elem_offset);
-  CNB_LAUNCH_CHECK();
-  return CNB_OK;
-}
-
 static bool cnb_overlaps(const float* a, const float* b, long long n) {
   return a && b && a < b + n && b < a + n;
-}
-
-extern "C" int cnb_dpm_solver_step(const float* xt, const float* eps, const float* z, float* hist, float* xt_prev,
-                                   float* x0, long long n, const float* coef, int clip_sample, uint64_t seed,
-                                   uint64_t step, const int32_t* step_dev, uint64_t elem_offset, cnb_stream_t s) {
-  CNB_REQUIRE(n > 0 && xt && eps && hist && xt_prev && coef, "dpm_solver_step: null pointer or n=%lld", n);
-  CNB_REQUIRE(!cnb_overlaps(hist, xt, n) && !cnb_overlaps(hist, xt_prev, n) && !cnb_overlaps(hist, x0, n),
-              "dpm_solver_step: hist must not overlap xt, xt_prev or x0");
-  CNB_REQUIRE((((uintptr_t)xt | (uintptr_t)eps | (uintptr_t)xt_prev | (uintptr_t)z | (uintptr_t)x0 |
-                (uintptr_t)hist) & 15) == 0,
-              "dpm_solver_step: pointers must be 16-byte aligned");
-  long long n4 = n >> 2;
-  unsigned blocks = (unsigned)((n4 + 255) / 256);
-  if (blocks < 1) blocks = 1;
-  if (blocks > 148 * 16) blocks = 148 * 16;
-  dpm_solver_step_kernel<<<blocks, 256, 0, (cudaStream_t)s>>>(xt, eps, z, hist, xt_prev, x0, n, coef, clip_sample,
-                                                              seed, step, step_dev, elem_offset);
-  CNB_LAUNCH_CHECK();
-  return CNB_OK;
 }
 
 static unsigned elementwise4_blocks(long long n) {
@@ -662,6 +563,45 @@ static unsigned elementwise4_blocks(long long n) {
   if (blocks < 1) blocks = 1;
   if (blocks > 148 * 16) blocks = 148 * 16;
   return (unsigned)blocks;
+}
+
+// The checks every scheduler update takes (hist is null for the rules without a history buffer), then one launch.
+template <class Rule>
+static int launch_update(const char* name, const float* xt, const float* eps, const float* z, float* hist,
+                         float* xt_prev, float* x0, long long n, const float* coef, int clip_sample, uint64_t seed,
+                         uint64_t step, const int32_t* step_dev, uint64_t elem_offset, cnb_stream_t s) {
+  CNB_REQUIRE(n > 0 && xt && eps && xt_prev && coef && (hist || !Rule::kHist), "%s: null pointer or n=%lld", name, n);
+  CNB_REQUIRE(!cnb_overlaps(hist, xt, n) && !cnb_overlaps(hist, xt_prev, n) && !cnb_overlaps(hist, x0, n),
+              "%s: hist must not overlap xt, xt_prev or x0", name);
+  CNB_REQUIRE((((uintptr_t)xt | (uintptr_t)eps | (uintptr_t)xt_prev | (uintptr_t)z | (uintptr_t)x0 |
+                (uintptr_t)hist) & 15) == 0,
+              "%s: pointers must be 16-byte aligned", name);
+  update_kernel<Rule><<<elementwise4_blocks(n), 256, 0, (cudaStream_t)s>>>(xt, eps, z, hist, xt_prev, x0, n, coef,
+                                                                           clip_sample, seed, step, step_dev,
+                                                                           elem_offset);
+  CNB_LAUNCH_CHECK();
+  return CNB_OK;
+}
+
+extern "C" int cnb_sched_step(const float* xt, const float* eps, const float* z, float* xt_prev, float* x0,
+                              long long n, const float* coef, uint64_t seed, uint64_t step, const int32_t* step_dev,
+                              uint64_t elem_offset, cnb_stream_t s) {
+  return launch_update<DdpmRule>("sched_step", xt, eps, z, nullptr, xt_prev, x0, n, coef, 0, seed, step, step_dev,
+                                 elem_offset, s);
+}
+
+extern "C" int cnb_ddim_step(const float* xt, const float* eps, const float* z, float* xt_prev, float* x0, long long n,
+                             const float* coef, int clip_sample, uint64_t seed, uint64_t step, const int32_t* step_dev,
+                             uint64_t elem_offset, cnb_stream_t s) {
+  return launch_update<DdimRule>("ddim_step", xt, eps, z, nullptr, xt_prev, x0, n, coef, clip_sample, seed, step,
+                                 step_dev, elem_offset, s);
+}
+
+extern "C" int cnb_dpm_solver_step(const float* xt, const float* eps, const float* z, float* hist, float* xt_prev,
+                                   float* x0, long long n, const float* coef, int clip_sample, uint64_t seed,
+                                   uint64_t step, const int32_t* step_dev, uint64_t elem_offset, cnb_stream_t s) {
+  return launch_update<DpmSolverRule>("dpm_solver_step", xt, eps, z, hist, xt_prev, x0, n, coef, clip_sample, seed,
+                                      step, step_dev, elem_offset, s);
 }
 
 extern "C" int cnb_add_noise(const float* x_ref, const float* z, float* out, long long n, float sqrt_acp,
@@ -714,14 +654,6 @@ extern "C" int cnb_philox_normal(float* out, long long n, uint64_t seed, uint64_
     if (blocks > 148 * 16) blocks = 148 * 16;
     philox_normal_kernel<<<(unsigned)blocks, 256, 0, (cudaStream_t)s>>>(out, n, seed, step, elem_offset);
   }
-  CNB_LAUNCH_CHECK();
-  return CNB_OK;
-}
-
-extern "C" int cnb_gather_row(const float* table, const int32_t* row_index, float* dst, int ncols, cnb_stream_t s) {
-  CNB_REQUIRE(ncols > 0, "gather_row: ncols=%d", ncols);
-  gather_row_kernel<<<blocks_for(ncols, 256) > 64 ? 64 : blocks_for(ncols, 256), 256, 0, (cudaStream_t)s>>>(
-      table, row_index, dst, ncols);
   CNB_LAUNCH_CHECK();
   return CNB_OK;
 }

@@ -279,12 +279,27 @@ def pack_convT_weight(w, round_tf32):
     return dst
 
 
-def sched_step(xt, eps, coef, z=None, want_x0=True, seed=0, step=0, step_dev=None, elem_offset=0, out=None,
-               x0_out=None):
-    """out may alias xt (every element is read before it is written by the same thread)."""
-    rt.require_cuda(xt, eps, coef, z, step_dev, out, x0_out)
+def _update_buffers(name, xt, eps, coef, z, step_dev, want_x0, out, x0_out, hist=None):
+    """(prev, x0) of a fused scheduler update, after the checks that keep its kernel inside its buffers: xt, eps and
+    the given z / out / x0_out / hist contiguous fp32 CUDA tensors with xt's number of elements, coef a contiguous fp32
+    CUDA tensor of at least 6 elements, step_dev an int32 CUDA tensor.  Attribute reads only: nothing synchronises."""
+    rt.require_cuda(xt, eps, coef, z, step_dev, out, x0_out, hist)
+    _f32(name, xt, eps, coef, z, out, x0_out, hist)
+    if any(t is not None and t.numel() != xt.numel() for t in (eps, z, out, x0_out, hist)) or coef.numel() < 6:
+        raise rt.CnbError(f"{name}: eps, z, out, x0_out and hist must have xt's {xt.numel()} elements and coef at "
+                          f"least 6")
+    if step_dev is not None and step_dev.dtype != torch.int32:
+        raise rt.CnbError(f"{name}: step_dev must be an int32 tensor (got {step_dev.dtype})")
     prev = torch.empty_like(xt) if out is None else out
     x0 = x0_out if x0_out is not None else (torch.empty_like(xt) if want_x0 else None)
+    return prev, x0
+
+
+def sched_step(xt, eps, coef, z=None, want_x0=True, seed=0, step=0, step_dev=None, elem_offset=0, out=None,
+               x0_out=None):
+    """One DDPM update (cnb_sched_step); coef is a row of LinearNoiseScheduler.coef_table.  out may alias xt (every
+    element is read before it is written by the same thread)."""
+    prev, x0 = _update_buffers("sched_step", xt, eps, coef, z, step_dev, want_x0, out, x0_out)
     rt.check(rt.lib().cnb_sched_step(xt.data_ptr(), eps.data_ptr(), rt.ptr(z), prev.data_ptr(), rt.ptr(x0),
                                      xt.numel(), coef.data_ptr(), seed, step, rt.ptr(step_dev), elem_offset,
                                      rt.stream()))
@@ -294,9 +309,7 @@ def sched_step(xt, eps, coef, z=None, want_x0=True, seed=0, step=0, step_dev=Non
 def ddim_step(xt, eps, coef, z=None, want_x0=True, clip_sample=False, seed=0, step=0, step_dev=None, elem_offset=0,
               out=None, x0_out=None):
     """One DDIM update (cnb_ddim_step); coef is a row of DDIMScheduler.coef_table.  Same conventions as sched_step."""
-    rt.require_cuda(xt, eps, coef, z, step_dev, out, x0_out)
-    prev = torch.empty_like(xt) if out is None else out
-    x0 = x0_out if x0_out is not None else (torch.empty_like(xt) if want_x0 else None)
+    prev, x0 = _update_buffers("ddim_step", xt, eps, coef, z, step_dev, want_x0, out, x0_out)
     rt.check(rt.lib().cnb_ddim_step(xt.data_ptr(), eps.data_ptr(), rt.ptr(z), prev.data_ptr(), rt.ptr(x0), xt.numel(),
                                     coef.data_ptr(), 1 if clip_sample else 0, seed, step, rt.ptr(step_dev),
                                     elem_offset, rt.stream()))
@@ -308,12 +321,8 @@ def dpm_solver_step(xt, eps, coef, z=None, want_x0=True, clip_sample=False, seed
     """One DPM-Solver++ update (cnb_dpm_solver_step); coef is a row of DPMSolverMultistepScheduler.coef_table.  hist
     (fp32, xt's size) holds the previous step's data prediction and receives this step's.  Same conventions as
     sched_step."""
-    rt.require_cuda(xt, eps, coef, z, step_dev, out, x0_out, hist)
-    if hist.dtype != torch.float32 or hist.numel() != xt.numel() or not hist.is_contiguous():
-        raise rt.CnbError("dpm_solver_step: hist must be a contiguous fp32 tensor with xt's number of elements")
-    prev = torch.empty_like(xt) if out is None else out
-    x0 = x0_out if x0_out is not None else (torch.empty_like(xt) if want_x0 else None)
-    rt.check(rt.lib().cnb_dpm_solver_step(xt.data_ptr(), eps.data_ptr(), rt.ptr(z), hist.data_ptr(), prev.data_ptr(),
+    prev, x0 = _update_buffers("dpm_solver_step", xt, eps, coef, z, step_dev, want_x0, out, x0_out, hist)
+    rt.check(rt.lib().cnb_dpm_solver_step(xt.data_ptr(), eps.data_ptr(), rt.ptr(z), rt.ptr(hist), prev.data_ptr(),
                                           rt.ptr(x0), xt.numel(), coef.data_ptr(), 1 if clip_sample else 0, seed,
                                           step, rt.ptr(step_dev), elem_offset, rt.stream()))
     return prev, x0

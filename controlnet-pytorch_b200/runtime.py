@@ -71,7 +71,6 @@ _SIGS = {
                                   c_void_p, c_u64, c_u64, c_u64, c_void_p]),
     "cnb_mask_max_pool": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int, c_int, c_void_p]),
     "cnb_philox_normal": (c_int, [c_void_p, c_ll, c_u64, c_u64, c_u64, c_void_p]),
-    "cnb_gather_row": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_void_p]),
     "cnb_sampler_prologue": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "cnb_bump_index": (c_int, [c_void_p, c_int, c_void_p]),
     "cnb_edm_coeffs": (c_int, [c_void_p, c_int, c_float, c_float, c_void_p, c_void_p, c_void_p, c_void_p]),

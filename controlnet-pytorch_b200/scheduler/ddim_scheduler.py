@@ -19,43 +19,31 @@ import torch
 
 from .. import ops
 from .. import runtime as rt
-from .schedule import strided_timesteps, tail
+from .schedule import StridedScheduler, step_inputs
 
 
-class DDIMScheduler:
+class DDIMScheduler(StridedScheduler):
     """`base` is a LinearNoiseScheduler (DDPM or LDM betas).  The schedule is `timesteps` when given (strictly
     decreasing, inside [0, T)), otherwise `num_inference_steps` timesteps with the given spacing:
       "trailing": round(T - k T / S) - 1, k = 0 .. S-1 (round half to even), starting at T-1 where x_T ~ N(0, I);
       "leading":  (S-1-k) * (T // S), ending at 0.
     Attributes may be changed after construction; every call re-validates them."""
+    TAG = "ddim"
 
     def __init__(self, base, num_inference_steps=50, eta=0.0, spacing="trailing", clip_sample=False, timesteps=None):
-        self.base = base
-        self.num_timesteps = base.num_timesteps
-        self.num_inference_steps, self.eta, self.spacing = num_inference_steps, eta, spacing
-        self.clip_sample = clip_sample
-        self.explicit_timesteps = None if timesteps is None else tuple(int(t) for t in timesteps)
-        self.seed = 0
-        self._coef = {}
-        self.timesteps()
-        self._eta()
+        self.eta = eta
+        super().__init__(base, num_inference_steps, spacing, clip_sample, timesteps)
 
-    def _eta(self):
+    def _params(self):
         eta = float(self.eta)
         if not (math.isfinite(eta) and eta >= 0.0):
             raise rt.CnbError(f"DDIMScheduler: eta must be a finite number >= 0 (got {self.eta!r})")
-        return eta
-
-    def timesteps(self, steps=None, skip=0):
-        """tau_0 > ... > tau_{S-1} as a tuple of ints; `steps` overrides num_inference_steps; the tail without the first
-        `skip` timesteps (0 <= skip < S) with skip > 0."""
-        return tail("DDIMScheduler", strided_timesteps("DDIMScheduler", self.num_timesteps, self.num_inference_steps,
-                                                       self.spacing, self.explicit_timesteps, steps), skip)
+        return (eta,)
 
     def coef_table_host(self, steps=None):
         """fp32 [T, 6]: row tau_k is row_k of the module docstring; rows off the schedule are NaN, so that reading one
         by mistake poisons the output instead of passing unnoticed."""
-        ts, eta, b = self.timesteps(steps), self._eta(), self.base
+        ts, (eta,), b = self.timesteps(steps), self._params(), self.base
         acp = b.alpha_cum_prod
         tab = torch.full((self.num_timesteps, 6), float("nan"), dtype=torch.float32)
         for k, t in enumerate(ts):
@@ -71,19 +59,6 @@ class DDIMScheduler:
             tab[t, 5] = 1.0 if sigma > 0.0 else 0.0
         return tab
 
-    def coef_table(self, device, steps=None, skip=0):
-        """The device copy of coef_table_host.  A row depends only on its own timestep and the next one, so the tail
-        of `skip` (validated) reads the same table at the same rows."""
-        self.timesteps(steps, skip)
-        key = (str(device), self.timesteps(steps), self._eta())
-        if key not in self._coef:
-            self._coef[key] = self.coef_table_host(steps).to(device)
-        return self._coef[key]
-
-    def graph_key(self, steps=None, skip=0):
-        """Everything a captured sampling step depends on besides the model and the coefficient table."""
-        return ("ddim", self.timesteps(steps, skip), self._eta(), bool(self.clip_sample))
-
     def new_state(self, x):
         """DDIM carries nothing from one step to the next."""
         return {}
@@ -97,16 +72,8 @@ class DDIMScheduler:
         LinearNoiseScheduler.sample_prev_timestep.  The noise is `z` when given, otherwise the fused Philox stream
         keyed by (self.seed, step, element); step defaults to t's position in timesteps(), the step index
         sampler.DDPMSampler uses, so a loop over timesteps() draws the sampler's noise."""
-        rt.require_cuda(xt, noise_pred)
-        if xt.dtype != torch.float32 or noise_pred.dtype != torch.float32:
-            raise rt.CnbError("sample_prev_timestep expects fp32 tensors")
-        ts, ti = self.timesteps(), int(t)
-        if ti not in ts:
-            raise rt.CnbError(f"DDIMScheduler: t={ti} is not one of the schedule's timesteps")
-        if z is not None:
-            rt.require_cuda(z)
-            z = z.contiguous()
-        step = ts.index(ti) if step_index is None else int(step_index)
-        coef = self.coef_table(xt.device)[ti]
-        return self.update(xt.contiguous(), noise_pred.contiguous(), coef, z=z, want_x0=True, seed=self.seed,
-                           step=step)
+        xt, noise_pred, z = step_inputs(xt, noise_pred, z)
+        ts, k = self._position(t)
+        coef = self.coef_table(xt.device)[ts[k]]
+        return self.update(xt, noise_pred, coef, z=z, want_x0=True, seed=self.seed,
+                           step=k if step_index is None else int(step_index))

@@ -9,8 +9,7 @@ default generator exactly like the reference (default), or from the fused Philox
 import torch
 
 from .. import ops
-from .. import runtime as rt
-from .schedule import tail
+from .schedule import step_inputs, tail
 
 
 class LinearNoiseScheduler:
@@ -81,16 +80,10 @@ class LinearNoiseScheduler:
 
     def sample_prev_timestep(self, xt, noise_pred, t, z=None, step_index=None):
         """(x_{t-1}, x0) from (x_t, eps, t); t is a 0-d / python int timestep shared by the batch (:49-77)."""
-        rt.require_cuda(xt, noise_pred)
-        if xt.dtype != torch.float32 or noise_pred.dtype != torch.float32:
-            raise rt.CnbError("sample_prev_timestep expects fp32 tensors")
+        xt, noise_pred, z = step_inputs(xt, noise_pred, z)
         ti = int(t)
-        xt, noise_pred = xt.contiguous(), noise_pred.contiguous()
         coef = self.coef_table(xt.device)[ti]
         if ti > 0 and z is None and self.rng == "torch_cpu":
             z = torch.randn(xt.shape).to(xt.device)          # CPU generator + H2D, as the reference does
-        if z is not None:
-            rt.require_cuda(z)
-            z = z.contiguous()
         step = ti if step_index is None else int(step_index)
         return ops.sched_step(xt, noise_pred, coef, z=z, want_x0=True, seed=self.seed, step=step)

@@ -1,5 +1,6 @@
-"""The strided timestep schedules the few-step samplers (ddim_scheduler.py, dpm_solver_scheduler.py) share, and the
-truncated ("tail") schedules of image-to-image sampling that every scheduler shares."""
+"""The strided timestep schedules and the scheduler base the few-step samplers (ddim_scheduler.py,
+dpm_solver_scheduler.py) share, and what every scheduler shares: the truncated ("tail") schedules of image-to-image
+sampling and the input checks of sample_prev_timestep."""
 import math
 import numbers
 from fractions import Fraction
@@ -42,6 +43,62 @@ def tail(owner, ts, skip):
         raise rt.CnbError(f"{owner}: skip must be an int in [0, {len(ts)}) for a schedule of {len(ts)} steps "
                           f"(got {skip!r})")
     return ts[int(skip):]
+
+
+def step_inputs(xt, noise_pred, z):
+    """The input checks of sample_prev_timestep: xt and noise_pred fp32 CUDA tensors, z a CUDA tensor when given.
+    Returns the three made contiguous."""
+    rt.require_cuda(xt, noise_pred, z)
+    if xt.dtype != torch.float32 or noise_pred.dtype != torch.float32:
+        raise rt.CnbError("sample_prev_timestep expects fp32 tensors")
+    return xt.contiguous(), noise_pred.contiguous(), None if z is None else z.contiguous()
+
+
+class StridedScheduler:
+    """What DDIMScheduler and DPMSolverMultistepScheduler share: a strided schedule (strided_timesteps) over the
+    tables of `base`, a LinearNoiseScheduler; a fp32 [T, 6] coefficient table per schedule, built by the subclass's
+    coef_table_host and cached per device; and the graph key.  A subclass sets TAG (the graph key's first element)
+    and TAIL_TABLE, and defines _params(): its validated solver parameters, part of both keys."""
+    TAG = None
+    TAIL_TABLE = False      # True: a tail's rows differ from the full schedule's (coef_table_host takes `skip`)
+
+    def __init__(self, base, num_inference_steps, spacing, clip_sample, timesteps):
+        self.base = base
+        self.num_timesteps = base.num_timesteps
+        self.num_inference_steps, self.spacing, self.clip_sample = num_inference_steps, spacing, clip_sample
+        self.explicit_timesteps = None if timesteps is None else tuple(int(t) for t in timesteps)
+        self.seed = 0
+        self._coef = {}
+        self.timesteps()
+        self._params()
+
+    def timesteps(self, steps=None, skip=0):
+        """tau_0 > ... > tau_{S-1} as a tuple of ints; `steps` overrides num_inference_steps; the tail without the first
+        `skip` timesteps (0 <= skip < S) with skip > 0."""
+        owner = type(self).__name__
+        return tail(owner, strided_timesteps(owner, self.num_timesteps, self.num_inference_steps, self.spacing,
+                                             self.explicit_timesteps, steps), skip)
+
+    def coef_table(self, device, steps=None, skip=0):
+        """The device copy of coef_table_host.  Without TAIL_TABLE a row depends only on its own timestep and the next
+        one, so the tail of `skip` (validated) reads the full schedule's table at the same rows."""
+        self.timesteps(steps, skip)
+        args = (steps, skip) if self.TAIL_TABLE else (steps,)
+        key = (str(device), self.timesteps(*args)) + self._params()
+        if key not in self._coef:
+            self._coef[key] = self.coef_table_host(*args).to(device)
+        return self._coef[key]
+
+    def graph_key(self, steps=None, skip=0):
+        """Everything a captured sampling step depends on besides the model and the coefficient table."""
+        return (self.TAG, self.timesteps(steps, skip)) + self._params() + (bool(self.clip_sample),)
+
+    def _position(self, t):
+        """(timesteps(), k) for the k-th timestep t of the schedule; CnbError for a t off the schedule."""
+        ts, ti = self.timesteps(), int(t)
+        if ti not in ts:
+            raise rt.CnbError(f"{type(self).__name__}: t={ti} is not one of the schedule's timesteps")
+        return ts, ts.index(ti)
 
 
 def strength_to_skip(S, strength):

@@ -257,9 +257,6 @@ int cnb_mask_max_pool(const float* in, float* out, int B, int H, int W, int f, c
 /* Fill out[i] with the same N(0,1) stream as cnb_sched_step (used for x_T and by tests). */
 int cnb_philox_normal(float* out, long long n, uint64_t seed, uint64_t step, uint64_t elem_offset,
                       cnb_stream_t stream);
-/* dst[0..ncols) = table[row_index[0] * ncols ..]; row_index lives on the device so a captured graph can be
- * replayed for every timestep (used for the per-t scheduler coefficients and t-embedding bias rows). */
-int cnb_gather_row(const float* table, const int32_t* row_index, float* dst, int ncols, cnb_stream_t stream);
 /* Start of a replayed denoising step: k = step_idx[0]; t_out[0] = t_seq[k] (int64, what the model's
  * time-embedding reads); coef_out[0..6) = coef_table[t_seq[k]][0..6) (what cnb_sched_step reads). */
 int cnb_sampler_prologue(const int32_t* step_idx, const int64_t* t_seq, int64_t* t_out, const float* coef_table,

@@ -388,6 +388,32 @@ def test_philox_properties(pk):
     assert torch.allclose(prev, 0.3 * a[:4096], rtol=0, atol=1e-7)
 
 
+@pytest.mark.parametrize("name", ["sched_step", "ddim_step", "dpm_solver_step"])
+def test_update_ops_reject_what_the_kernel_would_overrun(pk, name):
+    """The fused updates index every per-element buffer by xt's element count: a shorter, non-contiguous or non-fp32
+    buffer, a short coef row or a non-int32 step counter is refused before anything is launched."""
+    ops, rt = pk
+    op = getattr(ops, name)
+    n = 4 * 1024 + 3
+    good = dict(xt=torch.zeros(n, device="cuda"), eps=torch.zeros(n, device="cuda"),
+                coef=torch.tensor([0.5, 0.8, 0.01, 0.99, 0.3, 1.0], device="cuda"))
+    if name == "dpm_solver_step":
+        good["hist"] = torch.zeros(n, device="cuda")
+    short = torch.zeros(n - 1, device="cuda")
+    bad = [dict(eps=short), dict(z=short), dict(out=short), dict(x0_out=short),
+           dict(xt=torch.zeros(2 * n, device="cuda")[::2]), dict(xt=good["xt"].half()), dict(coef=good["coef"][:5]),
+           dict(step_dev=torch.zeros(1, device="cuda", dtype=torch.int64))]
+    if name == "dpm_solver_step":
+        bad.append(dict(hist=short))
+    c0 = rt.launch_count()
+    op(**good)
+    assert rt.launch_count() == c0 + 1
+    for b in bad:
+        with pytest.raises(rt.CnbError):
+            op(**{**good, **b})
+        assert rt.launch_count() == c0 + 1, b
+
+
 def test_layout_and_scale(pk):
     ops, rt = pk
     x = rnd(3, 5, 6, 7, seed=1)
