@@ -27,8 +27,13 @@ window [start, end) of the schedule outside which the step is the frozen U-Net a
 eps = eu + w * (ec - eu).  A non-default `control` captures up to two step graphs over the same sampler-owned buffers,
 the control graph (prologue -> model._forward_controlled -> update -> [blend] -> bump) and the plain graph (prologue ->
 model.trained_unet -> update -> [blend] -> bump), and picks one per step on the host from `ControlOptions.keep`.
+
+Each call is checked and set up once, by `DDPMSampler._plan`, whichever loop runs it.  Both loops run one step body,
+`DDPMSampler._step` (forward -> update -> [blend]): the eager loop with host values, the captured step between the
+prologue and the bump with the device step counter and the sampler-owned buffers.
 """
 
+import collections
 import dataclasses
 import math
 import numbers
@@ -78,27 +83,11 @@ class ControlOptions:
         return [not (i / n < self.start or (i + 1) / n > self.end) for i in range(n)]
 
 
-def _control(model, control):
-    """None for the plain ControlNet step (control None or default), else the checked ControlOptions."""
-    if control is None:
-        return None
-    if not isinstance(control, ControlOptions):
-        raise rt.CnbError(f"control must be a sampler.ControlOptions (got {type(control).__name__})")
-    if control == ControlOptions():
-        return None
-    if not hasattr(model, "_forward_controlled"):
-        raise rt.CnbError(f"control options need a ControlNet; {type(model).__name__} has no control branch")
-    return control
-
-
-def _step_forward(model, ctl, controlled, hint):
-    """eps(xt, t) of one step: the model's forward, its controlled forward or the frozen U-Net alone."""
-    if ctl is None:
-        return lambda xt, t: model(xt, t, hint)
-    if not controlled:
-        return lambda xt, t: model.trained_unet(xt, t)
-    w = None if ctl.guidance == 1.0 else float(ctl.guidance)
-    return lambda xt, t: model._forward_controlled(xt, t, hint, ctl.scale, w)
+# One sampling call, checked and derived once by DDPMSampler._plan: the timesteps run (img2img's tail), the scheduler's
+# [T, 6] coefficient table on x's device, the checked ControlOptions and its window keep(len(ts)) (both None for the
+# plain ControlNet step), img2img's checked reference and mask and the blend's noise-level table (None without a mask),
+# and the key of everything a captured step depends on: an equal key reuses the captured graph(s).
+_Plan = collections.namedtuple("_Plan", "ts table ctl keep x_ref mask levels key")
 
 
 class DDPMSampler:
@@ -111,19 +100,32 @@ class DDPMSampler:
     def draw_xT(self, shape, device, elem_offset=0):
         return ops.philox_normal(shape, device, self.seed, _XT_STEP, elem_offset)
 
-    # ---- image-to-image start ----------------------------------------------------------------------------
+    # ---- what both loops share: the checked run of one call, the image-to-image start, the step body --------
     def _base(self):
         """The LinearNoiseScheduler whose tables define the noise levels (a strided scheduler's `base`)."""
         return getattr(self.scheduler, "base", self.scheduler)
 
-    def _img2img_args(self, x_ref, mask, strength, steps):
-        """(x_ref, mask, skip) checked: x_ref contiguous fp32, the mask fp32 (bool converted once), [B, 1 or C, H, W]
-        with values in [0, 1] (one check per call, outside the loop), skip from strength."""
-        rt.require_cuda(x_ref, mask)
-        if x_ref.dtype != torch.float32 or x_ref.dim() != 4:
-            raise rt.CnbError("img2img: the reference must be a fp32 NCHW tensor")
-        x_ref = x_ref.contiguous()
+    def _noised_start(self, x_ref, t, z, elem_offset, out=None):
+        """add_noise(x_ref, z, t) with the base scheduler's fp32 values at t; z=None is the x_T stream."""
+        b = self._base()
+        return ops.add_noise(x_ref, float(b.sqrt_alpha_cum_prod[t]), float(b.sqrt_one_minus_alpha_cum_prod[t]), z=z,
+                             seed=self.seed, step=_XT_STEP, elem_offset=elem_offset, out=out)
+
+    def _plan(self, x_T, hint, steps, elem_offset, x_ref=None, mask=None, strength=1.0, control=None):
+        """Every check of a sampling call and what it runs (_Plan).  With x_ref the run is img2img and x_T, when given,
+        the eager loop's injected noise: x_ref contiguous fp32 NCHW, the mask fp32 (bool converted once),
+        [B, 1 or C, H, W] with values in [0, 1] (one check per call, outside the loop), skip from strength.  The hint
+        must have the batch size of the x the model reads: the forward's convolutions index the hint by sample."""
+        rt.require_cuda(x_T, hint, x_ref, mask)
+        sch, skip = self.scheduler, 0
+        if x_ref is not None:
+            if x_ref.dtype != torch.float32 or x_ref.dim() != 4:
+                raise rt.CnbError("img2img: the reference must be a fp32 NCHW tensor")
+            x_ref = x_ref.contiguous()
+            skip = strength_to_skip(len(sch.timesteps(steps)), strength)
         if mask is not None:
+            if x_ref is None:
+                raise rt.CnbError("a mask needs the reference x_ref")
             if mask.dtype == torch.bool:
                 mask = mask.float()
             B, C, H, W = x_ref.shape
@@ -133,13 +135,46 @@ class DDPMSampler:
             mask = mask.contiguous()
             if not bool(((mask >= 0) & (mask <= 1)).all()):
                 raise rt.CnbError("img2img: mask values must lie in [0, 1] (1 = generate, 0 = keep the reference)")
-        return x_ref, mask, strength_to_skip(len(self.scheduler.timesteps(steps)), strength)
+        x = x_T if x_ref is None else x_ref
+        if hint.shape[0] != x.shape[0]:
+            raise rt.CnbError(f"the hint's batch size {hint.shape[0]} differs from the {x.shape[0]} samples of "
+                              f"{'x_T' if x_ref is None else 'x_ref'}")
+        if control is not None and not isinstance(control, ControlOptions):
+            raise rt.CnbError(f"control must be a sampler.ControlOptions (got {type(control).__name__})")
+        ctl = None if control is None or control == ControlOptions() else control     # None: the plain step
+        if ctl is not None and not hasattr(self.model, "_forward_controlled"):
+            raise rt.CnbError(f"control options need a ControlNet; {type(self.model).__name__} has no control branch")
+        ts = sch.timesteps(steps, skip)
+        table = sch.coef_table(x.device, steps, skip)
+        keep = None if ctl is None else ctl.keep(len(ts))
+        levels = None if mask is None else noise_levels(self._base(), ts).to(x.device)
+        # the table's address tells apart schedulers with equal graph keys but other beta schedules; the noise-level
+        # table is sampler-owned and refreshed on reuse, so its values need no key
+        key = (tuple(x.shape), tuple(hint.shape), sch.graph_key(steps, skip), table.data_ptr(), elem_offset,
+               rt.get_mode(), str(x.device), self._param_stamp(), skip, None if mask is None else tuple(mask.shape))
+        if ctl is not None:
+            key += ((ctl.scale, ctl.guidance, tuple(keep)),)
+        return _Plan(ts, table, ctl, keep, x_ref, mask, levels, key)
 
-    def _noised_start(self, x_ref, t, z, elem_offset, out=None):
-        """add_noise(x_ref, z, t) with the base scheduler's fp32 values at t; z=None is the x_T stream."""
-        b = self._base()
-        return ops.add_noise(x_ref, float(b.sqrt_alpha_cum_prod[t]), float(b.sqrt_one_minus_alpha_cum_prod[t]), z=z,
-                             seed=self.seed, step=_XT_STEP, elem_offset=elem_offset, out=out)
+    def _step(self, ctl, controlled, hint, xt, t, coef, state, blend, elem_offset, step=0, step_dev=None, z=None,
+              z0=None, out=None, x0_out=None):
+        """One denoising step, the body of both loops; returns (x, x0).  eps is the model's forward (ctl None), its
+        controlled forward or, outside the control window, the frozen U-Net alone; then the scheduler's fused update
+        and, with blend = (x_ref, mask, levels), the inpainting blend.  The eager loop passes host values (step=k,
+        injected z and z0), the captured step the device step counter and the sampler-owned buffers."""
+        if ctl is None:
+            eps = self.model(xt, t, hint)
+        elif controlled:
+            eps = self.model._forward_controlled(xt, t, hint, ctl.scale,
+                                                 None if ctl.guidance == 1.0 else float(ctl.guidance))
+        else:
+            eps = self.model.trained_unet(xt, t)
+        xt, x0 = self.scheduler.update(xt, eps, coef, z=z, seed=self.seed, step=step, step_dev=step_dev,
+                                       elem_offset=elem_offset, out=out, x0_out=x0_out, **state)
+        if blend is not None:
+            ops.inpaint_blend(xt, *blend, step=step, step_dev=step_dev, z=z0, seed=self.seed, noise_step=_XT_STEP,
+                              elem_offset=elem_offset)
+        return xt, x0
 
     # ---- eager loop (injected z, parity tests, per-step callbacks) ----------------------------------------
     @torch.no_grad()
@@ -148,38 +183,19 @@ class DDPMSampler:
         """The loop without a graph; returns (x, x0).  With `x_ref` it is img2img's loop (see there): it starts from
         add_noise(x_ref, z, tau_skip) and, with `mask`, blends after every step, where z is x_T when given (injected
         noise) and otherwise the x_T stream.  `control`: ControlOptions (see there)."""
-        sch = self.scheduler
-        ctl = _control(self.model, control)
-        skip, levels = 0, None
-        if x_ref is None and mask is not None:
-            raise rt.CnbError("sample_eager: a mask needs the reference x_ref")
-        if x_ref is not None:
-            x_ref, mask, skip = self._img2img_args(x_ref, mask, strength, steps)
-        ts = sch.timesteps(steps, skip)
-        dev = (x_T if x_ref is None else x_ref).device
-        table = sch.coef_table(dev, steps, skip)
-        if x_ref is None:
-            xt = x_T.contiguous()
-        else:
-            z0 = None if x_T is None else x_T.contiguous()
-            xt = self._noised_start(x_ref, ts[0], z0, elem_offset)
-            if mask is not None:
-                levels = noise_levels(self._base(), ts).to(dev)
+        p = self._plan(x_T, hint, steps, elem_offset, x_ref, mask, strength, control)
+        z0 = None if x_ref is None or x_T is None else x_T.contiguous()
+        xt = x_T.contiguous() if x_ref is None else self._noised_start(p.x_ref, p.ts[0], z0, elem_offset)
+        blend = None if p.mask is None else (p.x_ref, p.mask, p.levels)
         x0 = None
-        state = sch.new_state(xt)
-        t_dev = torch.empty((1,), device=dev, dtype=torch.int64)
-        keep = [True] * len(ts) if ctl is None else ctl.keep(len(ts))
-        fwd = {c: _step_forward(self.model, ctl, c, hint) for c in set(keep)}
-        for k, t in enumerate(ts):
+        state = self.scheduler.new_state(xt)
+        t_dev = torch.empty((1,), device=xt.device, dtype=torch.int64)
+        for k, t in enumerate(p.ts):
             t_dev.fill_(t)
-            eps = fwd[keep[k]](xt, t_dev)
             # the last step adds no noise in any scheduler, so zs may stop one short of the schedule
-            z = zs[k].to(xt.device) if (zs is not None and k < len(ts) - 1) else None
-            xt, x0 = sch.update(xt, eps, table[t], z=z, want_x0=True, seed=self.seed, step=k,
-                                elem_offset=elem_offset, **state)
-            if levels is not None:
-                ops.inpaint_blend(xt, x_ref, mask, levels, step=k, z=z0, seed=self.seed, noise_step=_XT_STEP,
-                                  elem_offset=elem_offset)
+            z = zs[k].to(xt.device) if (zs is not None and k < len(p.ts) - 1) else None
+            xt, x0 = self._step(p.ctl, p.keep is None or p.keep[k], hint, xt, t_dev, p.table[t], state, blend,
+                                elem_offset, step=k, z=z, z0=z0)
             if callback is not None:
                 callback(t, xt, x0)
         return xt, x0
@@ -198,70 +214,62 @@ class DDPMSampler:
             return
         fn(self._hint, rt.get_mode())
 
-    def _capture(self, x_T, hint, steps, elem_offset, skip=0, x_ref=None, mask=None, control=None):
+    def _capture(self, x_T, hint, steps, elem_offset, plan=None):
+        """Capture the step graph(s) of `plan` (by default the plain run of x_T, hint and steps) over buffers the
+        sampler owns, x_T's copy the start of the run."""
+        p = self._plan(x_T, hint, steps, elem_offset) if plan is None else plan
         dev = x_T.device
-        sch = self.scheduler
         self.xt = x_T.clone().contiguous()
         # the graph reads a hint buffer OWNED by the sampler: callers may free or overwrite theirs
         self._hint = hint.clone().contiguous()
         hint = self._hint
         self.x0 = torch.empty_like(self.xt)
-        ts = sch.timesteps(steps, skip)
-        self.t_seq = torch.tensor(ts, dtype=torch.int64).to(dev)
+        self.t_seq = torch.tensor(p.ts, dtype=torch.int64).to(dev)
         self.step_idx = torch.zeros((1,), device=dev, dtype=torch.int32)
         self.t_out = torch.zeros((1,), device=dev, dtype=torch.int64)
         self.coef = torch.zeros((6,), device=dev, dtype=torch.float32)
-        table = sch.coef_table(dev, steps, skip)
-        self._table = table          # the graph reads it: kept alive, so no other table can take its address
-        self._state = sch.new_state(self.xt)   # carried across replays: owned by the sampler, as long as the graph
-        state = self._state
-        # inpainting: the reference, the mask and the noise-level table the blend reads, owned like the hint
-        self._xref = None if mask is None else x_ref.clone()
-        self._mask = None if mask is None else mask.clone()
-        self._levels = None if mask is None else noise_levels(self._base(), ts).to(dev)
+        self._table = p.table        # the graph reads it: kept alive, so no other table can take its address
+        self._state = self.scheduler.new_state(self.xt)   # carried across replays: owned by the sampler, as the graph
+        # inpainting: the reference and the mask the blend reads, owned like the hint, and the plan's own level table
+        self._blend = None if p.mask is None else (p.x_ref.clone(), p.mask.clone(), p.levels)
         L = rt.lib()
-        ctl = _control(self.model, control)
 
-        def one_step(forward):
+        def one_step(controlled):
             rt.check(L.cnb_sampler_prologue(self.step_idx.data_ptr(), self.t_seq.data_ptr(), self.t_out.data_ptr(),
-                                            table.data_ptr(), self.coef.data_ptr(), rt.stream()))
-            eps = forward(self.xt, self.t_out)
-            sch.update(self.xt, eps, self.coef, z=None, seed=self.seed, step_dev=self.step_idx,
-                       elem_offset=elem_offset, out=self.xt, x0_out=self.x0, **state)
-            if mask is not None:
-                ops.inpaint_blend(self.xt, self._xref, self._mask, self._levels, step_dev=self.step_idx,
-                                  seed=self.seed, noise_step=_XT_STEP, elem_offset=elem_offset)
+                                            p.table.data_ptr(), self.coef.data_ptr(), rt.stream()))
+            self._step(p.ctl, controlled, hint, self.xt, self.t_out, self.coef, self._state, self._blend, elem_offset,
+                       step_dev=self.step_idx, out=self.xt, x0_out=self.x0)
             rt.check(L.cnb_bump_index(self.step_idx.data_ptr(), 1, rt.stream()))
 
-        def capture(forward):
+        def capture(controlled):
             # warm-up on a side stream: builds weight / hint caches and sets kernel attributes outside the capture
             s = torch.cuda.Stream(device=dev)
             s.wait_stream(torch.cuda.current_stream())
             with torch.cuda.stream(s):
                 self.step_idx.zero_()
-                one_step(forward)
+                one_step(controlled)
             torch.cuda.current_stream().wait_stream(s)
             torch.cuda.synchronize(dev)
             c0 = rt.launch_count()
             g = torch.cuda.CUDAGraph()
             with torch.cuda.graph(g):
-                one_step(forward)
+                one_step(controlled)
             return g, rt.launch_count() - c0
 
         # with control options, the control graph and the plain graph share every buffer above and are captured only
         # when some step uses them; replay_steps picks one per step from self._keep
-        self._keep = None if ctl is None else ctl.keep(len(ts))
+        self._keep = p.keep
         self._graphs = {}
         self.launches_per_step = self.plain_launches_per_step = None
-        for controlled in ((True,) if ctl is None else sorted(set(self._keep), reverse=True)):
-            g, n = capture(_step_forward(self.model, ctl, controlled, hint))
+        for controlled in ((True,) if p.keep is None else sorted(set(p.keep), reverse=True)):
+            g, n = capture(controlled)
             self._graphs[controlled] = g
             if controlled:
                 self.launches_per_step = n
             else:
                 self.plain_launches_per_step = n
         self._graph = self._graphs[True] if self._keep is None else self._graphs[self._keep[0]]
-        self._nsteps, self._pos = len(ts), 0
+        self._nsteps, self._pos = len(p.ts), 0
         # keep every tensor the graphs read alive for as long as the graphs: the hint features (HintCache may evict)
         # and the scaled zero-convolution weights (replaced when another scale is used)
         cache = getattr(self.model, "_hint_cache", None)
@@ -271,36 +279,24 @@ class DDPMSampler:
     def sample(self, x_T, hint, steps=None, elem_offset=0, control=None):
         """Run the scheduler's timesteps (DDPM: t = steps-1 .. 0, SURVEY.md 3.5 semantics) with fused on-device noise;
         returns (x after the last step, x0).  `control`: ControlOptions (see there)."""
-        rt.require_cuda(x_T, hint)
         if not self.use_graph:
             return self.sample_eager(x_T, hint, steps, None, elem_offset, control=control)
-        if hint.shape[0] != x_T.shape[0]:
-            raise rt.CnbError("sample: x_T and hint must have the same batch size")
-        self._prepare(x_T, hint, steps, elem_offset, control=control)
+        plan = self._plan(x_T, hint, steps, elem_offset, control=control)
+        self._prepare(x_T, hint, elem_offset, plan)
         self.xt.copy_(x_T)
         return self._run()
 
-    def _prepare(self, x_T, hint, steps, elem_offset, skip=0, x_ref=None, mask=None, control=None):
-        """Capture the step graph(s), or refresh the sampler-owned buffers of the ones that fit."""
-        sch = self.scheduler
-        # the table's address tells apart schedulers with equal graph keys but other beta schedules; the noise-level
-        # table is sampler-owned and refreshed below, so its values need no key
-        key = (tuple(x_T.shape), tuple(hint.shape), sch.graph_key(steps, skip),
-               sch.coef_table(x_T.device, steps, skip).data_ptr(), elem_offset, rt.get_mode(), str(x_T.device),
-               self._param_stamp(), skip, None if mask is None else tuple(mask.shape))
-        ctl = _control(self.model, control)
-        if ctl is not None:
-            key += ((ctl.scale, ctl.guidance, tuple(ctl.keep(len(sch.timesteps(steps, skip))))),)
-        if self._graph is None or key != self._key:
-            self._capture(x_T, hint, steps, elem_offset, skip, x_ref, mask, ctl)
-            self._key = key
+    def _prepare(self, x_T, hint, elem_offset, plan):
+        """Capture the step graph(s) of `plan`, or refresh the sampler-owned buffers of the ones whose key it has."""
+        if self._graph is None or plan.key != self._key:
+            self._capture(x_T, hint, None, elem_offset, plan)
+            self._key = plan.key
         else:
             self._hint.copy_(hint)
             self._refresh_hint()
-            if mask is not None:
-                self._xref.copy_(x_ref)
-                self._mask.copy_(mask)
-                self._levels.copy_(noise_levels(self._base(), sch.timesteps(steps, skip)))
+            if plan.mask is not None:
+                for buf, new in zip(self._blend, (plan.x_ref, plan.mask, plan.levels)):
+                    buf.copy_(new)
 
     def _run(self):
         self.replay_steps(self._nsteps, reset=True)
@@ -319,16 +315,12 @@ class DDPMSampler:
         x_ref exactly after the last step, and soft values blend m * x + (1 - m) * known.  The returned x is blended;
         x0 is the update's own prediction of the last step, before the blend.  `control`: ControlOptions, whose window
         applies to the steps run."""
-        rt.require_cuda(x_ref, hint)
         if not self.use_graph:
             return self.sample_eager(None, hint, steps, None, elem_offset, x_ref=x_ref, mask=mask, strength=strength,
                                      control=control)
-        x_ref, mask, skip = self._img2img_args(x_ref, mask, strength, steps)
-        if hint.shape[0] != x_ref.shape[0]:
-            raise rt.CnbError("img2img: x_ref and hint must have the same batch size")
-        ts = self.scheduler.timesteps(steps, skip)
-        self._prepare(x_ref, hint, steps, elem_offset, skip, x_ref, mask, control)
-        self._noised_start(x_ref, ts[0], None, elem_offset, out=self.xt)
+        plan = self._plan(None, hint, steps, elem_offset, x_ref, mask, strength, control)
+        self._prepare(plan.x_ref, hint, elem_offset, plan)
+        self._noised_start(plan.x_ref, plan.ts[0], None, elem_offset, out=self.xt)
         return self._run()
 
     def replay_steps(self, n, reset=True):
@@ -512,22 +504,15 @@ def sample_data_parallel(model, scheduler, shape, hint_fn, steps=None, seed=0, g
         raise rt.CnbError("sample_data_parallel: x_T_fn and x_ref_fn exclude each other (img2img starts from x_ref)")
     if mask_fn is not None and x_ref_fn is None:
         raise rt.CnbError("sample_data_parallel: mask_fn needs x_ref_fn")
-    if x_ref_fn is not None:
+    kw = dict(steps=steps, elem_offset=lo * per, control=control)
+    if x_ref_fn is not None:                   # xt: with vae the shard's decoded images
         mask = None if mask_fn is None else mask_fn(lo, hi)
-        if vae is not None:
-            xt, _ = smp.img2img_images(x_ref_fn(lo, hi), hint_fn(lo, hi), strength=strength, mask=mask, steps=steps,
-                                       elem_offset=lo * per, control=control)
-        else:
-            xt, _ = smp.img2img(x_ref_fn(lo, hi), hint_fn(lo, hi), strength=strength, mask=mask, steps=steps,
-                                elem_offset=lo * per, control=control)
+        run = smp.img2img if vae is None else smp.img2img_images
+        xt, _ = run(x_ref_fn(lo, hi), hint_fn(lo, hi), strength=strength, mask=mask, **kw)
     else:
-        if x_T_fn is not None:
-            x_T = x_T_fn(lo, hi)
-        else:
-            x_T = smp.draw_xT((hi - lo,) + tuple(shape[1:]), dev, elem_offset=lo * per)
-        xt, x0 = smp.sample(x_T, hint_fn(lo, hi), steps=steps, elem_offset=lo * per, control=control)
-        if vae is not None:
-            xt = smp.decode(xt)
+        x_T = x_T_fn(lo, hi) if x_T_fn is not None else smp.draw_xT((hi - lo,) + tuple(shape[1:]), dev, lo * per)
+        run = smp.sample if vae is None else smp.sample_images
+        xt, _ = run(x_T, hint_fn(lo, hi), **kw)
     if not gather or world == 1:
         return xt
     return gather_shards(xt, B, group)

@@ -77,11 +77,10 @@ def main():
         mask = torch.zeros((B, 1, 28, 28), device=dev)
         mask[:, :, 7:21, 7:21] = 1.0
         sch = DDIM(ddpm, 50)
-        skip = 25                                         # strength 0.5 of S = 50
         smps = {"no_mask": S.DDPMSampler(model, sch, seed=5), "mask": S.DDPMSampler(model, sch, seed=5)}
         with torch.no_grad():
-            smps["no_mask"]._prepare(x_ref, hint, None, 0, skip)
-            smps["mask"]._prepare(x_ref, hint, None, 0, skip, x_ref, mask)
+            smps["no_mask"].img2img(x_ref, hint, strength=0.5)
+            smps["mask"].img2img(x_ref, hint, strength=0.5, mask=mask)
             times = step_times(torch, smps, args.replays, args.rounds)
         rec = {"batch": B, "step_ms": {k: [round(v, 4) for v in ts] for k, ts in times.items()},
                "step_ms_median": {k: round(statistics.median(ts), 4) for k, ts in times.items()},

@@ -9,39 +9,20 @@ re-capture and two samplers on one model; oracle parity for the DDPM and the LDM
 """
 import copy
 import ctypes
-import importlib
 import os
 import sys
 
 import pytest
 import torch
 
-from helpers import inputs, rel_l2, syn, ROOT
+from helpers import (inputs, rel_l2, syn, ROOT, TRAJ_TOL, _base, _ddim, _dpm, _fill, _hang_guard, _mod, _modes,
+                     rt)  # noqa: F401 (fixtures)
 
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
-
-TRAJ_TOL = {"fp32": 5e-4, "f16": 3e-2}     # test_img2img.py's trajectory tolerances
-
-
-def _mod(name):
-    return importlib.import_module("controlnet-pytorch_b200." + name)
 
 
 def _opts(**kw):
     return _mod("sampler").ControlOptions(**kw)
-
-
-def _base(ldm=False):
-    L = _mod("scheduler.linear_noise_scheduler").LinearNoiseScheduler
-    return L(ldm_scheduler=True, **syn.CELEBHQ_DIFFUSION) if ldm else L(**syn.MNIST_DIFFUSION)
-
-
-def _ddim(base=None, **kw):
-    return _mod("scheduler.ddim_scheduler").DDIMScheduler(_base() if base is None else base, **kw)
-
-
-def _dpm(base=None, **kw):
-    return _mod("scheduler.dpm_solver_scheduler").DPMSolverMultistepScheduler(_base() if base is None else base, **kw)
 
 
 # ---- CPU ---------------------------------------------------------------------------------------------------
@@ -78,29 +59,6 @@ def test_keep_is_the_diffusers_window_rule():
 
 
 # ---- GPU ---------------------------------------------------------------------------------------------------
-@pytest.fixture(scope="module")
-def rt():
-    r = _mod("runtime")
-    r.lib()
-    return r
-
-
-@pytest.fixture(autouse=True)
-def _hang_guard(request):
-    yield
-    if request.node.get_closest_marker("gpu") is not None:
-        assert _mod("runtime").lib().cnb_tc_error_flag() == 0
-
-
-def _modes(rt):
-    return ["fp32", "f16"] if rt.lib().cnb_has_tcgen05() else ["fp32"]
-
-
-def _fill(model, seed=0):
-    model.load_state_dict(syn.det_state_dict(model.state_dict(), seed))
-    return model.cuda().eval()
-
-
 def _combine(ec, eu, w):
     """cnb_guidance_combine restated in torch-CPU fp32, one rounding per operation."""
     return eu + torch.tensor(w, dtype=torch.float32) * (ec - eu)

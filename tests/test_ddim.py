@@ -4,49 +4,22 @@ CPU: the timestep schedules, the rejection of bad schedules and the [T, 6] coeff
 float64 restatement.  GPU: the fused kernel against a torch-CPU fp32 restatement of its operation order (bit for bit),
 its Philox noise and x0 against the DDPM kernel, the DDPM limit (eta = 1, every timestep), parity of the sampled
 trajectory with the oracle for the DDPM and the LDM ControlNet, graph replay against the eager loop, sharding,
-re-capture and the launch count of the captured step.
+re-capture and the launch count of the captured step.  The oracle parity and MNIST-size tests also run DPM-Solver++.
 """
-import importlib
 import os
 import sys
 
-import numpy as np
 import pytest
 import torch
 
-from helpers import inputs, max_abs, rel_l2, syn, ROOT
+from helpers import (inputs, max_abs, rel_l2, syn, ROOT, TRAJ_TOL, _base, _ddim, _ddim_oracle_loop, _ddim_rows, _dpm,
+                     _dpm_oracle_loop, _fill, _hang_guard, _mod, _modes, rt)  # noqa: F401 (fixtures)
 
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
 
-TRAJ_TOL = {"fp32": 5e-4, "f16": 3e-2}     # test_models_gpu.py's trajectory tolerances
-
-
-def _mod(name):
-    return importlib.import_module("controlnet-pytorch_b200." + name)
-
-
-def _base(ldm=False):
-    L = _mod("scheduler.linear_noise_scheduler").LinearNoiseScheduler
-    return L(ldm_scheduler=True, **syn.CELEBHQ_DIFFUSION) if ldm else L(**syn.MNIST_DIFFUSION)
-
-
-def _ddim(base=None, **kw):
-    return _mod("scheduler.ddim_scheduler").DDIMScheduler(_base() if base is None else base, **kw)
-
-
-def _rows(base, ts, eta):
-    """row_k of the DDIM update, restated: {tau_k: [c0 .. c5]} as float64 values of the fp32 base tables."""
-    acp = base.alpha_cum_prod.double().numpy()
-    s1m = base.sqrt_one_minus_alpha_cum_prod.double().numpy()
-    sa = base.sqrt_alpha_cum_prod.double().numpy()
-    out = {}
-    for k, t in enumerate(ts):
-        nxt = ts[k + 1] if k + 1 < len(ts) else None
-        a_t, a_p = acp[t], (1.0 if nxt is None else acp[nxt])
-        sig = eta * np.sqrt((1 - a_p) / (1 - a_t)) * np.sqrt(1 - a_t / a_p)
-        out[t] = [s1m[t], sa[t], 1.0 if nxt is None else sa[nxt], np.sqrt(max(1 - a_p - sig * sig, 0.0)), sig,
-                  1.0 if sig > 0 else 0.0]
-    return out
+# the oracle parity cases: (the scheduler over a base scheduler, its host oracle loop); the name seeds the inputs
+ORACLE_CASES = {"ddim": (lambda base: _ddim(base, num_inference_steps=4, eta=0.0), _ddim_oracle_loop),
+                "dpm": (lambda base: _dpm(base, num_inference_steps=4), _dpm_oracle_loop)}
 
 
 # ---- CPU ---------------------------------------------------------------------------------------------------
@@ -92,7 +65,7 @@ def test_coef_table_matches_the_restated_contract(ldm, S, eta, spacing):
     ts = s.timesteps()
     tab = s.coef_table_host()
     assert tab.shape == (1000, 6) and tab.dtype == torch.float32
-    want = _rows(base, ts, eta)
+    want = _ddim_rows(base, ts, eta)
     ddpm = base.coef_table_host()
     on = torch.zeros(1000, dtype=torch.bool)
     on[list(ts)] = True
@@ -117,29 +90,6 @@ def test_eta1_at_every_timestep_has_the_ddpm_posterior_sigma(ldm):
 
 
 # ---- GPU ---------------------------------------------------------------------------------------------------
-@pytest.fixture(scope="module")
-def rt():
-    r = _mod("runtime")
-    r.lib()
-    return r
-
-
-@pytest.fixture(autouse=True)
-def _hang_guard(request):
-    yield
-    if request.node.get_closest_marker("gpu") is not None:
-        assert _mod("runtime").lib().cnb_tc_error_flag() == 0
-
-
-def _fill(model, seed=0):
-    model.load_state_dict(syn.det_state_dict(model.state_dict(), seed))
-    return model.cuda().eval()
-
-
-def _modes(rt):
-    return ["fp32", "f16"] if rt.lib().cnb_has_tcgen05() else ["fp32"]
-
-
 def _host_ddim(xt, eps, z, row, clip):
     """The kernel's operation order in torch-CPU fp32, one rounding per operation."""
     c = row.float()
@@ -216,29 +166,20 @@ def test_whole_loop_with_every_timestep_and_eta1_is_the_ddpm_loop(rt):
     assert rel_l2(got.cpu(), want.cpu()) < 1e-4 and rel_l2(got0.cpu(), want0.cpu()) < 1e-4
 
 
-def _oracle_loop(forward, base, ts, x):
-    """eta = 0: x_prev = sqrt(a_p) x0 + sqrt(1 - a_p) eps, with the restated coefficients, on the host."""
-    rows = _rows(base, ts, 0.0)
-    xt = x.double()
-    for t in ts:
-        c = [float(v) for v in rows[t]]
-        eps = forward(xt.float(), torch.as_tensor(t).unsqueeze(0)).double()
-        xt = c[2] * (xt - c[0] * eps) / c[1] + c[3] * eps
-    return xt.float()
-
-
 @pytest.mark.gpu
-def test_ddpm_controlnet_parity_with_the_oracle(rt):
+@pytest.mark.parametrize("case", list(ORACLE_CASES))
+def test_ddpm_controlnet_parity_with_the_oracle(rt, case):
     import cn_oracle as O
     S = _mod("sampler")
+    sched, oracle_loop = ORACLE_CASES[case]
     cfg = syn.TINY_PARAMS
     m = _fill(_mod("models.controlnet").ControlNet(cfg))
     sd = {k: v.cpu() for k, v in m.state_dict().items()}
-    x, hint = inputs("ddim_tiny", 2, 1, 16)
+    x, hint = inputs(case + "_tiny", 2, 1, 16)
     base = _base()
-    s = _ddim(base, num_inference_steps=4, eta=0.0)
+    s = sched(base)
     with torch.no_grad():
-        want = _oracle_loop(lambda a, t: O.controlnet_ddpm_forward(sd, cfg, a, t, hint), base, s.timesteps(), x)
+        want = oracle_loop(lambda a, t: O.controlnet_ddpm_forward(sd, cfg, a, t, hint), base, s.timesteps(), x)
     for mode in _modes(rt):
         rt.set_mode(mode)
         got, _ = S.DDPMSampler(m, s, use_graph=True).sample(x.cuda(), hint.cuda())
@@ -246,19 +187,21 @@ def test_ddpm_controlnet_parity_with_the_oracle(rt):
 
 
 @pytest.mark.gpu
-def test_ldm_controlnet_with_vae_decode_parity_with_the_oracle(rt):
+@pytest.mark.parametrize("case", list(ORACLE_CASES))
+def test_ldm_controlnet_with_vae_decode_parity_with_the_oracle(rt, case):
     import cn_oracle as O
     S = _mod("sampler")
+    sched, oracle_loop = ORACLE_CASES[case]
     cfg, vcfg = syn.TINY_LDM_PARAMS, syn.TINY_VAE_PARAMS
     m = _fill(_mod("models.controlnet_ldm").ControlNet(4, cfg, down_sample_factor=8))
     vae = _fill(_mod("models.vae").VAE(3, vcfg), seed=1)
     sd = {k: v.cpu() for k, v in m.state_dict().items()}
     vsd = {k: v.cpu() for k, v in vae.state_dict().items()}
-    x, hint = inputs("ddim_ldm", 2, 4, 8, hint_size=64, p=0.05)
+    x, hint = inputs(case + "_ldm", 2, 4, 8, hint_size=64, p=0.05)
     base = _base(ldm=True)
-    s = _ddim(base, num_inference_steps=4, eta=0.0)
+    s = sched(base)
     with torch.no_grad():
-        lat_ref = _oracle_loop(lambda a, t: O.controlnet_ldm_forward(sd, cfg, a, t, hint), base, s.timesteps(), x)
+        lat_ref = oracle_loop(lambda a, t: O.controlnet_ldm_forward(sd, cfg, a, t, hint), base, s.timesteps(), x)
         want = (torch.clamp(O.vae_decode(vsd, vcfg, lat_ref), -1., 1.) + 1) / 2
     for mode in _modes(rt):
         rt.set_mode(mode)
@@ -345,12 +288,13 @@ def test_one_sampler_recaptures_on_every_change(rt):
 
 
 @pytest.mark.gpu
-def test_mnist_size_run_and_launch_count(rt):
+@pytest.mark.parametrize("case", ["ddim", "dpm"])
+def test_mnist_size_run_and_launch_count(rt, case):
     S = _mod("sampler")
     rt.set_mode("f16" if rt.lib().cnb_has_tcgen05() else "fp32")
     m = _fill(_mod("models.controlnet").ControlNet(syn.MNIST_PARAMS))
     hint = syn.det_hint(64, 28).cuda()
-    s = _ddim(num_inference_steps=50, eta=1.0)
+    s = _ddim(num_inference_steps=50, eta=1.0) if case == "ddim" else _dpm(num_inference_steps=20, variant="sde")
     g = S.DDPMSampler(m, s, seed=3)
     xT = g.draw_xT((64, 1, 28, 28), "cuda")
     a, a0 = g.sample(xT, hint)

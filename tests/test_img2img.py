@@ -6,7 +6,6 @@ kernels against torch-CPU restatements bit for bit; img2img without a mask again
 (bit for bit); the mask identities; graph replay against the eager loop, sharding and sample_data_parallel;
 re-capture; oracle parity for the DDPM and the LDM ControlNet; an MNIST-size run and the launch count.
 """
-import importlib
 import os
 import sys
 
@@ -14,28 +13,10 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from helpers import inputs, rel_l2, syn, ROOT
+from helpers import (inputs, rel_l2, syn, ROOT, TRAJ_TOL, _base, _ddim, _dpm, _fill, _hang_guard, _mod, _modes,
+                     rt)  # noqa: F401 (fixtures)
 
 sys.path.insert(0, os.path.join(ROOT, "oracle"))
-
-TRAJ_TOL = {"fp32": 5e-4, "f16": 3e-2}     # test_models_gpu.py's trajectory tolerances
-
-
-def _mod(name):
-    return importlib.import_module("controlnet-pytorch_b200." + name)
-
-
-def _base(ldm=False):
-    L = _mod("scheduler.linear_noise_scheduler").LinearNoiseScheduler
-    return L(ldm_scheduler=True, **syn.CELEBHQ_DIFFUSION) if ldm else L(**syn.MNIST_DIFFUSION)
-
-
-def _ddim(base=None, **kw):
-    return _mod("scheduler.ddim_scheduler").DDIMScheduler(_base() if base is None else base, **kw)
-
-
-def _dpm(base=None, **kw):
-    return _mod("scheduler.dpm_solver_scheduler").DPMSolverMultistepScheduler(_base() if base is None else base, **kw)
 
 
 def _sched():
@@ -110,29 +91,6 @@ def test_noise_levels(ldm):
 
 
 # ---- GPU ---------------------------------------------------------------------------------------------------
-@pytest.fixture(scope="module")
-def rt():
-    r = _mod("runtime")
-    r.lib()
-    return r
-
-
-@pytest.fixture(autouse=True)
-def _hang_guard(request):
-    yield
-    if request.node.get_closest_marker("gpu") is not None:
-        assert _mod("runtime").lib().cnb_tc_error_flag() == 0
-
-
-def _fill(model, seed=0):
-    model.load_state_dict(syn.det_state_dict(model.state_dict(), seed))
-    return model.cuda().eval()
-
-
-def _modes(rt):
-    return ["fp32", "f16"] if rt.lib().cnb_has_tcgen05() else ["fp32"]
-
-
 def _xt_noise(shape, seed, elem_offset=0):
     """The x_T stream the start and the blend draw from, on the host."""
     S = _mod("sampler")
@@ -337,6 +295,29 @@ def test_graph_equals_eager_shards_and_data_parallel(rt):
             g.img2img(x_ref, hint, strength=0.7, mask=bad)
     with pytest.raises(rt.CnbError):
         g.img2img(x_ref, hint, strength=0.01)                                # keeps no step of 8
+
+
+@pytest.mark.gpu
+def test_every_path_rejects_a_hint_of_another_batch_size_before_launching(rt):
+    """The ControlNet forward reads the hint by sample, so a hint with fewer samples than x would be read past its end:
+    the eager paths check it as the graph paths do, before the first launch."""
+    S = _mod("sampler")
+    m, hint, x_ref = _tiny(rt)
+    s = _ddim(num_inference_steps=4)
+    e, g = S.DDPMSampler(m, s, seed=1, use_graph=False), S.DDPMSampler(m, s, seed=1)
+    x_T = e.draw_xT(tuple(x_ref.shape), "cuda")
+    zs = [torch.zeros(tuple(x_ref.shape)) for _ in range(4)]
+    mask = torch.ones((4, 1, 16, 16), device="cuda")
+    for h in (hint[:3], torch.cat([hint, hint[:1]])):
+        calls = [lambda: e.sample(x_T, h), lambda: e.sample_eager(x_T, h, zs=zs),
+                 lambda: e.img2img(x_ref, h, strength=0.5), lambda: e.img2img(x_ref, h, strength=0.5, mask=mask),
+                 lambda: e.sample_eager(x_T, h, x_ref=x_ref, mask=mask, strength=0.5),
+                 lambda: g.sample(x_T, h), lambda: g.img2img(x_ref, h, strength=0.5, mask=mask)]
+        for i, fn in enumerate(calls):
+            c0 = rt.launch_count()
+            with pytest.raises(rt.CnbError, match="batch size"):
+                fn()
+            assert rt.launch_count() == c0, (h.shape[0], i)
 
 
 @pytest.mark.gpu
